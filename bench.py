@@ -42,7 +42,9 @@ RRF_K0 = 60.0
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="timed steps of the headline region (one user query each); the e2e and the "
+                         "two-users regions time as many steps")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", type=int, default=10_000_000)
@@ -52,9 +54,6 @@ def parse():
                          "batch's merges / exchange / fusion run under the next one's scans")
     ap.add_argument("--k", type=int, default=10,
                     help="result depth (10 = the headline metric; 100 with --rows 100000000 --gpus 8 = config C5)")
-    ap.add_argument("--min-time", type=float, default=0.25,
-                    help="the timed region repeats the K-step block until it lasts this long (seconds); "
-                         "`steps` stays K, `timed_steps` says how many were timed")
     ap.add_argument("--parity-queries", type=int, default=8,
                     help="pool queries checked against the on-device float64 brute force (0 = skip)")
     ap.add_argument("--kernel-events", default="on", choices=["on", "off"],
@@ -66,7 +65,16 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-stages", action="store_true", help="skip the K1 / K2a / K2b stage measurements")
     ap.add_argument("--cpu-sample-rows", type=int, default=1_000_000)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed region, write the results of its last step (ids, score, semantic, "
+                         "keyword, status of every sub-query, as float64) to DIR/<name>.npy, so that two "
+                         "builds can be compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the CUDA path (--impl ours)")
+    return args
 
 
 # ------------------------------------------------------------------ clocks
@@ -838,19 +846,20 @@ def run_ours(args):
         return float(t.item()), t_h
 
     clocks.start()
-    ms, t_host = timed_block(args.steps, warm)                  # exactly K steps
-    timed_steps, blocks = args.steps, 1
-    if ms * 1e-3 < args.min_time:
-        # K steps are too short a region to measure (pipeline fill / drain, rank skew): time R more
-        # blocks of K steps as ONE region and report that; every rank computes the same R
-        blocks = int(math.ceil(args.min_time / max(ms * 1e-3, 1e-6)))
-        blocks = max(2, min(blocks, 2000))
-        ms, t_host = timed_block(args.steps * blocks, warm + args.steps)
-        timed_steps = args.steps * blocks
+    ms, t_host = timed_block(args.steps, warm)
+    timed_steps = args.steps
     clk = clocks.stop()
     launches = sum(d.launches for d in devs) - launches0
     for o in all_outs:
         assert int(o[4].sum().item()) == 0, "status words set in the timed region"
+    if args.dump_outputs and rank == 0:
+        # the last timed step ran on handle (warm + steps - 1) % n_fly; the results are replicated
+        # on every rank.  Copied now: the passes below reuse the handles' output buffers.
+        last_outs = all_outs[(warm + args.steps - 1) % n_fly]
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        for name, t in zip(("ids", "score", "semantic", "keyword", "status"), last_outs):
+            np.save(out_dir / f"{name}.npy", t.cpu().numpy().astype(np.float64))
 
     # ---- roofline pass: the same chain, the same queries, ONE batch in flight, with CUDA event
     #      nodes around the two streaming kernels inside the captured chains.  With two batches in
@@ -900,7 +909,7 @@ def run_ours(args):
 
     e2e_run(max(6, 3 * n_fly))
     barrier()
-    e2e_steps = max(args.steps, int(timed_steps // 4), 10)
+    e2e_steps = args.steps
     ev0.record()
     last = e2e_run(e2e_steps)
     ev1.record()
@@ -931,7 +940,7 @@ def run_ours(args):
                 devs[i % n_fly].search_host_end()
         two_run(max(6, 3 * n_fly))
         barrier()
-        two_steps = max(e2e_steps // 2, 10)
+        two_steps = args.steps
         ev0.record()
         two_run(two_steps)
         ev1.record()
@@ -987,7 +996,7 @@ def run_ours(args):
             "metric": metric_name(args),
             "value": qps, "unit": "queries/s", "n_gpus": world, "steps": args.steps,
             "warmup": warm, "ms_per_step": step_ms,
-            "timed_steps": timed_steps, "timed_blocks": blocks, "timed_region_ms": ms,
+            "timed_steps": timed_steps, "timed_region_ms": ms,
             "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
             "dtype": ("f16 matrix + its int8 shadow: s8 x s8 -> s32 scan of the shadow, exact f64 re-score "
                       "of the fp16 rows; f64 BM25" if q8 else

@@ -1,18 +1,21 @@
-"""The drop-in boundary, end to end on the host side: the reference's UNMODIFIED
-``src/retrieval/orchestrator.py`` (read from /root/reference at run time -- never copied into the
-repo; the test is skipped where the reference tree is absent, e.g. on the GPU box) runs over the
-shim ``src/retrieval/retrieval_engine.py`` and this package's ``RetrievalEngine``.
+"""The drop-in boundary, end to end on the host side: the shim ``src/retrieval/retrieval_engine.py``
+and this package's ``RetrievalEngine``, called as the reference's ``src/retrieval/orchestrator.py``
+calls them (``RetrievalEngine(store_dir)``, ``engine.search(q, k=k, hybrid_weight=w)``,
+``engine.chunks``).  With ``LRX_REFERENCE_DIR`` pointing at a checkout of the reference project, its
+UNMODIFIED ``orchestrator.py`` also runs over the shim (that file is not part of this repository, so
+the test is skipped without it).
 
 No GPU here, so the device boundary is replaced by an oracle-backed double (test infrastructure):
 ``DeviceIndex`` -> the CPU oracle of K2..K4, ``lrx_encode_host`` -> the fp32 oracle encoder.
 Everything above it is the product's host code: the checkpoint loader (a synthetic
 ``model.safetensors`` + ``vocab.txt`` written here, found through EMBEDDING_MODEL_DIR), the
 WordPiece tokenizer, the store reader, ``query.lower().split()`` -> term ids, the result dicts.
-``orchestrate()``'s output is compared with the oracle path restated call by call
+The results are compared with the oracle path restated call by call
 (oracle/search.py fan-out + oracle/postprocess.py)."""
 import copy
 import importlib
 import json
+import os
 import shutil
 import sys
 from collections import Counter
@@ -24,7 +27,8 @@ import torch
 
 from conftest import ROOT
 
-REF_ORCH = Path("/root/reference/src/retrieval/orchestrator.py")
+REF_ORCH = (Path(os.environ["LRX_REFERENCE_DIR"]) / "src" / "retrieval" / "orchestrator.py"
+            if os.environ.get("LRX_REFERENCE_DIR") else None)
 
 STUB_CLASSIFIER = '''
 from typing import List, Optional
@@ -96,9 +100,8 @@ class OracleDevice:
 
 
 @pytest.fixture(scope="module")
-def deployment(tmp_path_factory, legal_chunks):
-    if not REF_ORCH.exists():
-        pytest.skip("the reference tree is not on this machine")
+def store_deployment(tmp_path_factory, legal_chunks):
+    """A checkpoint directory and a vector store built from the reference's corpus."""
     from safetensors.numpy import save_file
     from legal_rag_engine_b200 import synth, store
     from legal_rag_engine_b200.bm25_index import BM25Index
@@ -139,7 +142,15 @@ def deployment(tmp_path_factory, legal_chunks):
         x[idx] = oenc.encode_ids(sd, ids, lens)
     vs = root / "data" / "vector_store"
     store.save_store(vs, chunks, x, BM25Index.from_texts(texts))
-    # ---- the reference tree's package with ONE file replaced
+    return root, vs, model_dir, sd, chunks
+
+
+@pytest.fixture(scope="module")
+def deployment(store_deployment):
+    """`store_deployment` + the reference tree's package with ONE file replaced."""
+    if REF_ORCH is None or not REF_ORCH.exists():
+        pytest.skip("set LRX_REFERENCE_DIR to a checkout of the reference project")
+    root, vs, model_dir, sd, chunks = store_deployment
     pkg = root / "src" / "retrieval"
     pkg.mkdir(parents=True)
     (root / "src" / "__init__.py").write_text("")
@@ -150,13 +161,11 @@ def deployment(tmp_path_factory, legal_chunks):
     return root, vs, model_dir, sd, chunks
 
 
-def test_reference_orchestrator_runs_unchanged_over_the_engine(deployment, monkeypatch):
-    root, vs, model_dir, sd, chunks = deployment
+def _oracle_device(monkeypatch, model_dir):
+    """The device boundary -> the oracle double; the checkpoint is found through EMBEDDING_MODEL_DIR."""
     from legal_rag_engine_b200 import encoder as lenc
     from legal_rag_engine_b200 import engine as leng
     from oracle import encoder as oenc
-    from oracle import postprocess as opost
-    from oracle import search as osearch
 
     def fake_upload(dev, state_dict):
         dev.sd = {k: np.asarray(v) for k, v in lenc._strip(state_dict).items()}
@@ -166,6 +175,49 @@ def test_reference_orchestrator_runs_unchanged_over_the_engine(deployment, monke
     monkeypatch.setattr(lenc.SentenceEncoder, "encode_ids",
                         lambda self, ids, lens: oenc.encode_ids(self.dev.sd, np.asarray(ids), np.asarray(lens)))
     monkeypatch.setenv("EMBEDDING_MODEL_DIR", str(model_dir))
+
+
+def test_shim_engine_answers_the_orchestrator_calls_as_the_oracle(store_deployment, monkeypatch):
+    """What orchestrator.py:10,57 asks of the engine, through the shim: ``RetrievalEngine(store_dir)``
+    (positional), then ``search(q, k=5, hybrid_weight=w)`` for every fan-out string; the result
+    dicts carry the engine's own ``chunks`` objects and the oracle's scores."""
+    root, vs, model_dir, sd, chunks = store_deployment
+    from oracle import search as osearch
+    _oracle_device(monkeypatch, model_dir)
+    shim = importlib.import_module("src.retrieval.retrieval_engine")
+    assert Path(shim.__file__).resolve() == ROOT / "src" / "retrieval" / "retrieval_engine.py"
+    eng = shim.RetrievalEngine(str(vs))
+    try:
+        assert type(eng).__module__ == "legal_rag_engine_b200.engine" and len(eng.chunks) == len(chunks)
+        assert type(eng.model.tokenizer).__name__ == "WordPieceTokenizer"     # the checkpoint's vocab.txt
+        np.testing.assert_array_equal(
+            eng.dev.sd["encoder.layer.3.output.dense.weight"], sd["encoder.layer.3.output.dense.weight"])
+        csr, x = eng.dev.csr, eng.dev.x
+        csr.vocab = eng.bm25.vocab
+        oidx = osearch.OracleIndex(x, csr)
+        n_sub = 0
+        for query, intent in INTENTS.items():
+            qs, ws = osearch.fanout_queries(query, intent["user_context"], intent["key_entities"],
+                                            intent["category"])
+            for q, w in zip(qs, ws):
+                got = eng.search(q, k=5, hybrid_weight=w)
+                qh = eng.encode([q]).astype(np.float16)[0]
+                want = oidx.search_vec(qh, csr.term_ids(q.lower().split()), 5, w, "linear")
+                assert 1 <= len(got) <= 5 and len(got) == len(want), q
+                for r, (i, s, sem, kw) in zip(got, want):
+                    assert r["chunk"] is eng.chunks[i], q
+                    assert (r["score"], r["semantic"], r["keyword"]) == (s, sem, kw), q
+                n_sub += 1
+        assert n_sub == 9                                 # two fan-outs of 4 strings and one single query
+    finally:
+        eng.close()
+
+
+def test_reference_orchestrator_runs_unchanged_over_the_engine(deployment, monkeypatch):
+    root, vs, model_dir, sd, chunks = deployment
+    from oracle import postprocess as opost
+    from oracle import search as osearch
+    _oracle_device(monkeypatch, model_dir)
     saved = {k: v for k, v in sys.modules.items() if k == "src" or k.startswith("src.")}
     for k in saved:
         del sys.modules[k]
