@@ -117,6 +117,22 @@ int lrx_set_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const void* de
  * dev_postings_out (nnz x 8 bytes).  LRX_E_ARG if a tf or a length exceeds 65535. */
 int lrx_bm25_build_postings(lrx_handle* h, const uint32_t* dev_doc_tf, int64_t nnz,
                             const uint32_t* dev_doc_len, void* dev_postings_out);
+/* Index append (the reference has none: it rebuilds, create_vector_store.py:14-83).  Current index:
+ * dev_term_ptr [n_terms+1] + dev_postings (nnz 8-byte entries, as lrx_set_postings takes them) over
+ * local documents [0, n_docs_old).  Appended documents: dev_add_ptr [n_terms_out+1] +
+ * dev_add_doc_tf {u32 doc_local, u32 tf}[nnz_add], their own term-major CSR (n_terms_out >= n_terms,
+ * ids >= n_terms are new terms), doc_local in [n_docs_old, n_docs_out).  dev_doc_len [n_docs_out].
+ * Writes dev_term_ptr_out [n_terms_out+1] and dev_postings_out (nnz + nnz_add entries, rounded up to
+ * an even count, 16-byte aligned, pad zeroed): term t's current postings, then its appended ones --
+ * byte for byte what lrx_bm25_build_postings makes of the whole corpus's CSR.  The outputs must not
+ * overlap the inputs.  The handle's index is not touched: pass the outputs to lrx_set_postings with
+ * the new idf / avgdl.  Synchronous.  LRX_E_ARG when a tf or a document length exceeds 65535, an
+ * appended doc id is out of range, or term_ptr[n_terms] != nnz / add_ptr[n_terms_out] != nnz_add. */
+int lrx_bm25_append_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const void* dev_postings,
+                             int64_t n_terms, int64_t nnz, int64_t n_docs_old,
+                             const uint64_t* dev_add_ptr, const uint32_t* dev_add_doc_tf,
+                             int64_t n_terms_out, int64_t nnz_add, const uint32_t* dev_doc_len,
+                             int64_t n_docs_out, uint64_t* dev_term_ptr_out, void* dev_postings_out);
 
 /* ---- K1: encoder (replaces SentenceTransformer("all-MiniLM-L6-v2").encode followed by
  *      faiss.normalize_L2; retrieval_engine.py:28,61-62, create_vector_store.py:33-34,45,51) --

@@ -80,6 +80,8 @@ _SIGNATURES = {
     "lrx_set_dense_prefilter": (C.c_int, [_vp, _vp, _i64, C.POINTER(C.c_double)]),
     "lrx_set_postings": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _f64, _f64, _f64, _i32]),
     "lrx_bm25_build_postings": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
+    "lrx_bm25_append_postings": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _i64, _i64, _vp,
+                                           _i64, _vp, _vp]),
     "lrx_set_encoder_weights": (C.c_int, [_vp, C.POINTER(lrx_bert_weights)]),
     "lrx_encode": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _vp, _vp]),
     "lrx_encode_host": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _vp]),

@@ -39,6 +39,88 @@ def okapi_idf(df: np.ndarray, n_docs: int, epsilon: float = EPSILON):
 
 
 @dataclass
+class BM25Append:
+    """Documents appended to an index: their own term-major CSR over the extended vocabulary, and
+    the whole corpus's statistics after the append."""
+    new_words: List[str]         # vocabulary extension, first-appearance order: ids n_terms, n_terms + 1, ...
+    term_ptr: np.ndarray         # int64 [V_out+1]
+    postings: np.ndarray         # uint32 [nnz_add, 2] = (doc id, tf), doc ids >= the old n_docs
+    doc_len: np.ndarray          # uint32 [m]
+    df: np.ndarray               # int64 [V_out] document frequencies, old + appended documents
+    n_docs: int                  # after the append
+    total_len: int               # tokens after the append
+    idf: np.ndarray              # float64 [V_out]
+    avgdl: float
+
+    @property
+    def n_terms(self) -> int:
+        return len(self.term_ptr) - 1
+
+    @property
+    def nnz(self) -> int:
+        return int(self.term_ptr[-1])
+
+
+def csr_append(vocab: Dict[str, int], df: np.ndarray, n_docs: int, total_len: int,
+               token_lists: Sequence[Sequence[str]], epsilon: float = EPSILON) -> BM25Append:
+    """The appended documents' CSR and the updated statistics, in O(new tokens + V): no pass over
+    the existing postings.  ``vocab`` is read, not changed.  A rebuild numbers terms in first
+    appearance order over all documents in order; the old documents come first, so it keeps every
+    old id and numbers the new terms in first-appearance order over the appended documents -- the
+    order used here -- and okapi_idf's sequential mean, hence every idf bit, comes out the same."""
+    new: Dict[str, int] = {}
+    n_old = len(vocab)
+    t_l, d_l, f_l, lens = [], [], [], []
+    for d, document in enumerate(token_lists, start=n_docs):
+        lens.append(len(document))
+        freqs: Dict[str, int] = {}
+        for word in document:
+            freqs[word] = freqs.get(word, 0) + 1
+        for word, f in freqs.items():
+            t = vocab.get(word)
+            if t is None:
+                t = new.get(word)
+                if t is None:
+                    t = new[word] = n_old + len(new)
+            t_l.append(t); d_l.append(d); f_l.append(f)
+    n_out = n_old + len(new)
+    t = np.asarray(t_l, dtype=np.int64)
+    d = np.asarray(d_l, dtype=np.int64)
+    f = np.asarray(f_l, dtype=np.int64)
+    order = np.lexsort((d, t))
+    t, d, f = t[order], d[order], f[order]
+    count = np.bincount(t, minlength=n_out)
+    term_ptr = np.zeros(n_out + 1, dtype=np.int64)
+    np.cumsum(count, out=term_ptr[1:])
+    postings = np.empty((len(d), 2), dtype=np.uint32)
+    postings[:, 0] = d
+    postings[:, 1] = f
+    df_out = np.zeros(n_out, dtype=np.int64)
+    df_out[:n_old] = df
+    df_out += count
+    n_all = int(n_docs) + len(lens)
+    len_all = int(total_len) + sum(lens)
+    idf, _ = okapi_idf(df_out, n_all, epsilon)
+    return BM25Append(list(new), term_ptr, postings, np.asarray(lens, dtype=np.uint32), df_out, n_all,
+                      len_all, idf, len_all / n_all)
+
+
+def merge_csr(term_ptr: np.ndarray, postings: np.ndarray, app: BM25Append):
+    """Host merge (the device does the same in lrx_bm25_append_postings): term t's old postings,
+    then its appended ones.  Returns (term_ptr uint64 [V_out+1], postings uint32 [nnz + nnz_add, 2])."""
+    old_ptr = np.asarray(term_ptr, dtype=np.int64)
+    n_old = len(old_ptr) - 1
+    add_ptr = app.term_ptr
+    old_at = old_ptr[np.minimum(np.arange(app.n_terms + 1), n_old)]
+    out = np.empty((len(postings) + len(app.postings), 2), dtype=np.uint32)
+    shift = np.repeat(add_ptr[:n_old], np.diff(old_ptr))                   # old posting i of t -> i + add_ptr[t]
+    out[np.arange(len(postings), dtype=np.int64) + shift] = postings
+    ends = old_at[1:]                                                      # appended j of t -> old_end(t) + j
+    out[np.repeat(ends, np.diff(add_ptr)) + np.arange(len(app.postings), dtype=np.int64)] = app.postings
+    return (old_at + add_ptr).astype(np.uint64), out
+
+
+@dataclass
 class BM25Index:
     n_docs: int
     doc_len: np.ndarray          # uint32 [n_docs]
@@ -121,6 +203,20 @@ class BM25Index:
         np.add.at(term_ptr, t + 1, 1)
         term_ptr = np.cumsum(term_ptr)
         return cls.from_postings(n_docs, doc_len, term_ptr, d, tf, **kw)
+
+    # ------------------------------------------------------------------ append
+    def append(self, token_lists: Sequence[Sequence[str]]) -> "BM25Index":
+        """This index with the tokenised documents appended (ids n_docs, n_docs + 1, ...): equal,
+        field by field and bit for bit, to ``from_token_lists(old documents + token_lists)``."""
+        if self.vocab is None:
+            raise ValueError("index has no string vocabulary")
+        app = csr_append(self.vocab, np.diff(self.term_ptr.astype(np.int64)), self.n_docs,
+                         int(self.doc_len.astype(np.int64).sum()), token_lists, self.epsilon)
+        term_ptr, postings = merge_csr(self.term_ptr, self.postings, app)
+        vocab = dict(self.vocab)
+        vocab.update((w, len(self.vocab) + i) for i, w in enumerate(app.new_words))
+        return BM25Index(app.n_docs, np.concatenate([self.doc_len, app.doc_len]), term_ptr, postings,
+                         app.idf, app.avgdl, vocab, self.k1, self.b, self.epsilon)
 
     # ------------------------------------------------------------------ query
     def term_ids(self, tokens: Sequence[str]) -> List[int]:

@@ -355,6 +355,40 @@ int lrx_bm25_build_postings(lrx_handle* h, const uint32_t* dev_doc_tf, int64_t n
     return LRX_OK;
 }
 
+int lrx_bm25_append_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const void* dev_postings,
+                             int64_t n_terms, int64_t nnz, int64_t n_docs_old,
+                             const uint64_t* dev_add_ptr, const uint32_t* dev_add_doc_tf,
+                             int64_t n_terms_out, int64_t nnz_add, const uint32_t* dev_doc_len,
+                             int64_t n_docs_out, uint64_t* dev_term_ptr_out, void* dev_postings_out) {
+    if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_bm25_append_postings: null handle");
+    std::lock_guard<std::mutex> g(h->mu);
+    if (n_terms < 0 || nnz < 0 || n_docs_old < 0 || nnz_add < 0 || n_terms_out < n_terms ||
+        n_docs_out < n_docs_old || n_docs_out >= (1ll << 32))
+        return fail(h, LRX_E_ARG, "lrx_bm25_append_postings: bad size");
+    if (dev_term_ptr == nullptr || dev_add_ptr == nullptr || dev_term_ptr_out == nullptr ||
+        (nnz > 0 && dev_postings == nullptr) ||
+        (nnz_add > 0 && (dev_add_doc_tf == nullptr || dev_doc_len == nullptr)) ||
+        (nnz + nnz_add > 0 && dev_postings_out == nullptr))
+        return fail(h, LRX_E_ARG, "lrx_bm25_append_postings: null pointer");
+    if ((((uintptr_t)dev_postings | (uintptr_t)dev_postings_out) & 15) != 0 ||
+        (((uintptr_t)dev_add_doc_tf | (uintptr_t)dev_term_ptr | (uintptr_t)dev_add_ptr |
+          (uintptr_t)dev_term_ptr_out) & 7) != 0)
+        return fail(h, LRX_E_ARG, "lrx_bm25_append_postings: postings must be 16-byte aligned, "
+                                  "pointer tables and (doc, tf) pairs 8-byte aligned");
+    LRX_CUDA(h, cudaSetDevice(h->device));
+    int bad = 0;
+    LRX_CUDA(h, launch_bm25_append(h, dev_term_ptr, dev_postings, n_terms, nnz, n_docs_old, dev_add_ptr,
+                                   dev_add_doc_tf, n_terms_out, nnz_add, dev_doc_len, n_docs_out,
+                                   dev_term_ptr_out, dev_postings_out, &bad));
+    if (bad == 2)
+        return fail(h, LRX_E_ARG, "lrx_bm25_append_postings: term_ptr[n_terms] != nnz or "
+                                  "add_ptr[n_terms_out] != nnz_add");
+    if (bad)
+        return fail(h, LRX_E_ARG, "lrx_bm25_append_postings: a term frequency or document length "
+                                  "exceeds 65535, or an appended doc id is outside [n_docs_old, n_docs_out)");
+    return LRX_OK;
+}
+
 int lrx_set_encoder_weights(lrx_handle* h, const lrx_bert_weights* w) {
     if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_set_encoder_weights: null handle");
     std::lock_guard<std::mutex> g(h->mu);

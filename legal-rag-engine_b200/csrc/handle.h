@@ -146,6 +146,12 @@ cudaError_t launch_bm25_at(lrx_handle* h, const int32_t* q_terms, const int32_t*
                            const int64_t* ids, int n, double* out, cudaStream_t st);
 cudaError_t launch_bm25_pack(lrx_handle* h, const uint32_t* doc_tf, int64_t nnz, const uint32_t* doc_len,
                              void* out, int* host_overflow);
+// host_bad: 1 = a tf / length over 16 bits or an appended doc id out of range, 2 = a CSR end does
+// not match nnz / nnz_add (nothing launched)
+cudaError_t launch_bm25_append(lrx_handle* h, const uint64_t* old_ptr, const void* old_post, int64_t n_terms,
+                               int64_t nnz, int64_t n_docs_old, const uint64_t* add_ptr, const uint32_t* add,
+                               int64_t n_terms_out, int64_t nnz_add, const uint32_t* doc_len,
+                               int64_t n_docs_out, uint64_t* ptr_out, void* post_out, int* host_bad);
 cudaError_t launch_bm25_lut(lrx_handle* h, double avgdl, double k1, double b, int max_len);
 cudaError_t launch_bm25_divcheck(lrx_handle* h, double avgdl, double k1, double b, int n_tf, int n_len,
                                  unsigned long long* host_mismatches);

@@ -31,7 +31,9 @@ class DeviceIndex:
         _lib.check(self.lib.lrx_open(C.byref(cfg), C.byref(h)))
         self.h = h
         self.x = None
+        self._xbuf = None
         self._q8 = None
+        self._prefilter_on = False
         self.n_local = 0
         self.id_base = 0
         self._post = None
@@ -66,12 +68,41 @@ class DeviceIndex:
         assert x.dtype == torch.float16 and x.is_cuda and x.is_contiguous()
         assert x.dim() == 2 and x.shape[1] == LRX_DIM
         self.x, self.n_local, self.id_base = x, int(x.shape[0]), int(id_base)
+        self._xbuf = x                                      # the rows append_rows can fill: x is its prefix
         self._ck(self.lib.lrx_set_corpus(self.h, _ptr(x), self.n_local, self.id_base, LRX_DIM))
         self._q8 = None
         if prefilter is None:
             prefilter = os.environ.get("LRX_DENSE_PREFILTER", "1") not in ("0", "", "off")
+        self._prefilter_on = False
         if prefilter and self.n_local > 0:
             self.build_prefilter()
+
+    def append_rows(self, x_new: torch.Tensor):
+        """Append fp16 rows (local ids n_local, n_local + 1, ...).  The matrix is the prefix of a
+        capacity buffer; a buffer too small is replaced by one 1/16 larger than needed (the old rows
+        are copied on the device, the old buffer freed).  An index whose pre-filter is on gets its
+        int8 shadow rebuilt (its row scales sit after the padded rows, so it cannot grow in place)."""
+        assert x_new.dtype == torch.float16 and x_new.is_cuda and x_new.dim() == 2
+        assert x_new.shape[1] == LRX_DIM
+        n, m = self.n_local, int(x_new.shape[0])
+        if m == 0:
+            return
+        buf = self._xbuf
+        if buf is None or buf.shape[0] < n + m:
+            grown = torch.empty((n + m + (n + m) // 16, LRX_DIM), dtype=torch.float16, device=self.device)
+            if n:
+                grown[:n].copy_(self.x)
+            buf = grown
+        buf[n:n + m].copy_(x_new)
+        prefilter = self._prefilter_on
+        self._q8 = None                                     # the shadow of the old matrix
+        self.set_corpus(buf[:n + m], self.id_base, prefilter=prefilter)
+        self._xbuf = buf
+
+    @property
+    def capacity(self) -> int:
+        """Rows the matrix buffer holds before append_rows has to grow it."""
+        return int(self._xbuf.shape[0]) if self._xbuf is not None else 0
 
     def build_prefilter(self):
         nbytes = int(self.lib.lrx_dense_prefilter_bytes(self.n_local))
@@ -79,6 +110,7 @@ class DeviceIndex:
         bounds = (C.c_double * 2)()
         self._ck(self.lib.lrx_build_dense_prefilter(self.h, _ptr(buf), nbytes, bounds))
         self._q8 = (buf, nbytes, (float(bounds[0]), float(bounds[1])))
+        self._prefilter_on = True
 
     def set_prefilter(self, on: bool):
         """Switch the int8 pre-filter of an index that has a shadow (A/B runs, tests)."""
@@ -90,6 +122,7 @@ class DeviceIndex:
             self._ck(self.lib.lrx_set_dense_prefilter(self.h, _ptr(buf), nbytes, (C.c_double * 2)(*b)))
         else:
             self._ck(self.lib.lrx_set_dense_prefilter(self.h, C.c_void_p(0), 0, None))
+        self._prefilter_on = bool(on)
 
     @property
     def prefilter_bounds(self):
@@ -116,6 +149,7 @@ class DeviceIndex:
         idf_t = dev(idf, torch.float64)
         nnz = int(tp[-1].item())
         assert po.shape[0] == nnz, (po.shape, nnz)
+        self.n_docs = int(dl.numel())
         if dl.numel() == 0:
             dl = torch.zeros(1, dtype=torch.int32, device=self.device)
         max_len = int(dl.max().item())
@@ -128,6 +162,36 @@ class DeviceIndex:
         self.n_terms = int(tp.numel() - 1)
         self._ck(self.lib.lrx_set_postings(self.h, _ptr(tp), _ptr(p8), _ptr(idf_t), self.n_terms, nnz,
                                            float(avgdl), float(k1), float(b), max_len))
+
+    def append_postings(self, add_ptr, add_postings, add_doc_len, idf, avgdl: float):
+        """Append documents n_docs, n_docs + 1, ... to the resident postings: their own term-major
+        CSR (add_ptr int64 [V_out+1], add_postings uint32 [nnz_add, 2] = (local doc, tf)), their
+        lengths, and the whole corpus's new idf float64 [V_out] / avgdl.  The merge runs on the
+        device into new buffers (lrx_bm25_append_postings); the old ones are dropped only after
+        lrx_set_postings has taken the new ones, so a failure leaves the index as it was."""
+        tp, p8, _ = self._post
+        nnz, _, k1, b, max_len = self._post_args
+        up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a).view(dt)).to(self.device)
+        add_ptr = np.ascontiguousarray(add_ptr, dtype=np.int64)
+        add_len = np.ascontiguousarray(add_doc_len, dtype=np.uint32)
+        ap = up(add_ptr, np.int64)
+        ad = up(np.ascontiguousarray(add_postings, dtype=np.uint32).reshape(-1, 2), np.int32)
+        n_old, m = self.n_docs, len(add_len)
+        dl = torch.cat([self.doc_len[:n_old], up(add_len, np.int32)])
+        n_terms_out, nnz_add = len(add_ptr) - 1, int(add_ptr[-1])
+        tp_out = torch.empty(n_terms_out + 1, dtype=torch.int64, device=self.device)
+        p8_out = torch.empty((nnz + nnz_add + 2, 2), dtype=torch.int32, device=self.device)
+        self._ck(self.lib.lrx_bm25_append_postings(
+            self.h, _ptr(tp), _ptr(p8), self.n_terms, nnz, n_old, _ptr(ap), _ptr(ad), n_terms_out, nnz_add,
+            _ptr(dl), n_old + m, _ptr(tp_out), _ptr(p8_out)))
+        idf_t = torch.from_numpy(np.ascontiguousarray(idf, dtype=np.float64)).to(self.device)
+        max_len = max(max_len, int(add_len.max()) if m else 0)
+        self._ck(self.lib.lrx_set_postings(self.h, _ptr(tp_out), _ptr(p8_out), _ptr(idf_t), n_terms_out,
+                                           nnz + nnz_add, float(avgdl), k1, b, max_len))
+        self._post = (tp_out, p8_out, idf_t)
+        self._post_args = (nnz + nnz_add, float(avgdl), k1, b, max_len)
+        self.doc_len = dl if dl.numel() else self.doc_len
+        self.n_terms, self.n_docs = n_terms_out, n_old + m
 
     def clone_view(self) -> "DeviceIndex":
         """A second handle (own stream binding, workspaces, exchange region) over the SAME resident

@@ -6,7 +6,8 @@ store directory; everything numeric runs in the CUDA library behind include/lrx.
 
 Additive surface only: ``search_batch`` (the orchestrator's concept-expansion fan-out in one
 launch chain, orchestrator.py:38-62), ``fusion="linear"|"rrf"`` (default "linear" = the
-reference's behaviour, retrieval_engine.py:71-96), ``encode``.
+reference's behaviour, retrieval_engine.py:71-96), ``encode``, ``add_chunks`` / ``save`` (grow a
+loaded index without a rebuild; results stay bit-identical to a rebuild).
 
 There is no CPU fallback: without a CUDA device or the built library the constructor raises.
 """
@@ -16,6 +17,9 @@ import ctypes as C
 import json
 import logging
 import os
+import shutil
+import tempfile
+import threading
 from pathlib import Path
 from typing import Dict, List, Optional, Sequence
 
@@ -24,7 +28,7 @@ import torch
 
 from . import store as _store
 from ._lib import LRX_MAX_BATCH, LRX_MAX_DEPTH
-from .bm25_index import BM25Index, tokenize
+from .bm25_index import BM25Index, csr_append, merge_csr, tokenize
 from .device_index import FUSION, DeviceIndex
 from .encoder import SentenceEncoder
 from .sharding import shard_range
@@ -94,7 +98,11 @@ class RetrievalEngine:
         self.chunks, xh, bm25 = _store.load_store(self.store_dir, mmap=self.world > 1)
         self.n_total = len(self.chunks)
         self.lo, self.hi = shard_range(self.n_total, self.rank, self.world)
-        self.bm25 = bm25                                   # whole-corpus statistics + vocabulary
+        self._lock = threading.Lock()                      # searches see the index before or after an add
+        self._bm25 = bm25                                  # whole-corpus statistics + vocabulary
+        self._bm25_pending = []                            # appended CSRs not yet merged into _bm25's postings
+        self._df = np.diff(bm25.term_ptr.astype(np.int64))
+        self._total_len = int(bm25.doc_len.astype(np.int64).sum())
         local = bm25 if self.world == 1 else bm25.shard(self.lo, self.hi)
         self._x = torch.from_numpy(np.ascontiguousarray(xh[self.lo:self.hi])).to(self.dev.device)
         self.dev.set_corpus(self._x, self.lo)
@@ -154,6 +162,10 @@ class RetrievalEngine:
         ones go in separate blocks: the short ones take the encoder's query path, whose result for a
         query does not depend on what it is batched with (csrc/encoder.cu, small_path), so a query
         returns the same scores however a serving front coalesced it."""
+        with self._lock:
+            return self._search_all_locked(queries, k, weights, mode)
+
+    def _search_all_locked(self, queries, k, weights, mode):
         tok = self.model.tokenizer
         enc = [tok.encode(q, self.model.MAX_SEQ) for q in queries]
         out: List[Optional[List[dict]]] = [None] * len(queries)
@@ -181,7 +193,7 @@ class RetrievalEngine:
         # BM25 side: query.lower().split() -> term ids (retrieval_engine.py:67).  EVERY token is
         # scored, in order, repeats included, as rank_bm25 does; out-of-vocabulary tokens are
         # dropped here because `idf.get(q) or 0` makes them add exactly 0.0.
-        term_lists = [[t for t in self.bm25.term_ids(tokenize(q)) if t >= 0] for q in queries]
+        term_lists = [[t for t in self._bm25.term_ids(tokenize(q)) if t >= 0] for q in queries]
         o_ids, o_score, o_sem, o_kw = self.dev.search_text_host(ids, lens, term_lists, k, weights, mode)
         results = []
         for b in range(B):
@@ -194,6 +206,89 @@ class RetrievalEngine:
                              "semantic": float(o_sem[b, j]), "keyword": float(o_kw[b, j])})
             results.append(rows)
         return results
+
+    # ------------------------------------------------------------------ growth
+    @property
+    def bm25(self) -> BM25Index:
+        """The BM25 index of the whole current corpus (host postings of added chunks are merged in
+        when this is read)."""
+        with self._lock:
+            return self._bm25_current()
+
+    def _bm25_current(self) -> BM25Index:
+        b = self._bm25
+        for app in self._bm25_pending:
+            b.term_ptr, b.postings = merge_csr(b.term_ptr, b.postings, app)
+            b.doc_len = np.concatenate([b.doc_len, app.doc_len])
+        self._bm25_pending = []
+        return b
+
+    def add_chunks(self, chunks: Sequence[dict]) -> range:
+        """Append chunks to the loaded index; returns their ids (positions in ``self.chunks``).
+        Searches afterwards return exactly what an engine over a store rebuilt from all chunks (with
+        these rows as their embeddings) returns.  Each chunk is a dict with a str ``"text"``, embedded
+        with the encoder ``create_vector_store`` uses and stored as float16.  Input is validated
+        before anything changes; a rejected call leaves the engine as it was.  Not supported on a
+        sharded engine (world > 1)."""
+        if self.world > 1:
+            raise NotImplementedError("add_chunks on a sharded engine: rebuild the store instead")
+        chunks = list(chunks)
+        tokens = []
+        for i, c in enumerate(chunks):
+            if not isinstance(c, dict) or not isinstance(c.get("text"), str):
+                raise ValueError(f"chunk {i}: expected a dict with a str 'text'")
+            tokens.append(tokenize(c["text"]))
+            if len(tokens[-1]) > 65535:
+                raise ValueError(f"chunk {i}: {len(tokens[-1])} tokens; a BM25 document holds at most 65535")
+        with self._lock:
+            n = self.n_total
+            if n + len(chunks) >= 1 << 32:
+                raise ValueError("chunk ids must stay below 2^32")
+            if not chunks:
+                return range(n, n)
+            x16 = self.model.encode([c["text"] for c in chunks]).astype(np.float16)
+            b = self._bm25
+            app = csr_append(b.vocab, self._df, b.n_docs, self._total_len, tokens, b.epsilon)
+            self.dev.append_postings(app.term_ptr, app.postings, app.doc_len, app.idf, app.avgdl)
+            self.dev.append_rows(torch.from_numpy(x16).to(self.dev.device))
+            base = len(b.vocab)
+            b.vocab.update((w, base + i) for i, w in enumerate(app.new_words))
+            b.n_docs, b.idf, b.avgdl = app.n_docs, app.idf, app.avgdl
+            self._bm25_pending.append(app)
+            self._df, self._total_len = app.df, app.total_len
+            self.chunks.extend(chunks)
+            self.n_total = self.hi = len(self.chunks)
+            self._x = self.dev.x
+            return range(n, self.n_total)
+
+    def save(self, store_dir: Optional[str] = None) -> Path:
+        """Write the current index (added chunks included) as a store that ``RetrievalEngine`` and
+        the reference load: to ``store_dir`` or the directory this engine was loaded from.  The
+        files are written into a temporary sibling directory that replaces the target only when
+        every file is complete."""
+        if self.world > 1:
+            raise NotImplementedError("save on a sharded engine: each rank holds only its rows")
+        target = Path(store_dir) if store_dir is not None else self.store_dir
+        target.parent.mkdir(parents=True, exist_ok=True)
+        with self._lock:
+            tmp = Path(tempfile.mkdtemp(prefix=f".{target.name}.", dir=target.parent))
+            os.chmod(tmp, 0o755)                          # mkdtemp's 0700 would follow the store
+            old = None
+            try:
+                x = self._x.cpu().numpy().astype(np.float32)
+                _store.save_store(tmp, self.chunks, x, self._bm25_current())
+                if target.exists():
+                    old = Path(tempfile.mkdtemp(prefix=f".{target.name}.old.", dir=target.parent))
+                    os.rename(target, old / target.name)
+                os.rename(tmp, target)
+            except BaseException:
+                if old is not None and (old / target.name).exists() and not target.exists():
+                    os.rename(old / target.name, target)  # put the previous store back
+                shutil.rmtree(tmp, ignore_errors=True)
+                raise
+            if old is not None:
+                shutil.rmtree(old, ignore_errors=True)
+        return target
 
     def close(self):
         if getattr(self, "world", 1) > 1 and self.rank == 0 and self.dev.h:
