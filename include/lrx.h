@@ -133,6 +133,27 @@ int lrx_bm25_append_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const 
                              const uint64_t* dev_add_ptr, const uint32_t* dev_add_doc_tf,
                              int64_t n_terms_out, int64_t nnz_add, const uint32_t* dev_doc_len,
                              int64_t n_docs_out, uint64_t* dev_term_ptr_out, void* dev_postings_out);
+/* Index removal (the reference has none: it rebuilds the store).  Current index: dev_term_ptr
+ * [n_terms+1] + dev_postings (nnz 8-byte entries) over local documents [0, n_docs_old).  Removed:
+ * dev_removed_docs [n_removed], strictly ascending; per old term t its removed documents
+ * dev_rem_doc[dev_rem_ptr[t] .. dev_rem_ptr[t+1]), ascending (nnz_rem = rem_ptr[n_terms]);
+ * dev_term_map [n_terms]: t's new id, -1 for a term left without postings; dev_term_ptr_out
+ * [n_terms_out+1]: the new CSR's pointers (from the surviving document frequencies).  Writes
+ * dev_postings_out (nnz - nnz_rem entries, rounded up to an even count, 16-byte aligned, pad
+ * zeroed): every surviving posting under its term's new id, its document renumbered to
+ * d - |{r in removed : r < d}|, tf and length copied -- byte for byte what lrx_bm25_build_postings
+ * makes of the rebuilt CSR.  The outputs must not overlap the inputs.  The handle's index is not
+ * touched: pass the outputs to lrx_set_postings with the new idf / avgdl.  Synchronous.  LRX_E_ARG,
+ * with nothing else changed, when the CSR ends do not match the counts, a removed list is not
+ * strictly ascending or holds a document that is not a removed posting of its term, a posting of a
+ * removed document is missing from its term's list, term_map is not a bijection from the terms
+ * with survivors onto [0, n_terms_out), or a term's survivors do not fill its output range. */
+int lrx_bm25_remove_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const void* dev_postings,
+                             int64_t n_terms, int64_t nnz, int64_t n_docs_old,
+                             const uint32_t* dev_removed_docs, int64_t n_removed,
+                             const uint64_t* dev_rem_ptr, const uint32_t* dev_rem_doc,
+                             const int32_t* dev_term_map, const uint64_t* dev_term_ptr_out,
+                             int64_t n_terms_out, void* dev_postings_out);
 
 /* ---- K1: encoder (replaces SentenceTransformer("all-MiniLM-L6-v2").encode followed by
  *      faiss.normalize_L2; retrieval_engine.py:28,61-62, create_vector_store.py:33-34,45,51) --

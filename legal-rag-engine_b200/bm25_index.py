@@ -11,7 +11,7 @@ from __future__ import annotations
 
 import math
 from dataclasses import dataclass
-from typing import Dict, List, Optional, Sequence
+from typing import Callable, Dict, List, Optional, Sequence
 
 import numpy as np
 
@@ -120,6 +120,170 @@ def merge_csr(term_ptr: np.ndarray, postings: np.ndarray, app: BM25Append):
     return (old_at + add_ptr).astype(np.uint64), out
 
 
+def _ranges(starts: np.ndarray, counts: np.ndarray) -> np.ndarray:
+    """Concatenated ``arange(s, s + c)`` for each (s, c)."""
+    starts = np.asarray(starts, dtype=np.int64)
+    counts = np.asarray(counts, dtype=np.int64)
+    excl = np.cumsum(counts) - counts
+    return np.repeat(starts - excl, counts) + np.arange(int(counts.sum()), dtype=np.int64)
+
+
+@dataclass
+class BM25Remove:
+    """Documents removed from an index: their per-term lists, the surviving terms in the order a
+    rebuild numbers them, and the statistics after the removal."""
+    removed: np.ndarray          # int64 [m] removed document ids, ascending
+    rem_ptr: np.ndarray          # int64 [V+1] per old term, its removed documents ...
+    rem_doc: np.ndarray          # uint32 [nnz_rem] ... ascending
+    term_map: np.ndarray         # int32 [V] old term id -> new id, -1 = no surviving posting
+    term_ptr: np.ndarray         # int64 [V_out+1] the compacted CSR's pointers
+    words: List[str]             # the new vocabulary, new id order
+    first_doc: np.ndarray        # int64 [V_out] each term's first document (new ids)
+    df: np.ndarray               # int64 [V_out]
+    n_docs: int                  # after the removal
+    total_len: int               # tokens after the removal
+    idf: np.ndarray              # float64 [V_out]
+    avgdl: float
+
+    @property
+    def n_terms(self) -> int:
+        return len(self.term_ptr) - 1
+
+    @property
+    def nnz(self) -> int:
+        return int(self.term_ptr[-1])
+
+    @property
+    def nnz_rem(self) -> int:
+        return int(self.rem_ptr[-1])
+
+
+def csr_remove(vocab: Dict[str, int], df: np.ndarray, first_doc: np.ndarray, n_docs: int, total_len: int,
+               ids: Sequence[int], doc_tokens: Callable[[int], Sequence[str]],
+               first_postings: Callable[[np.ndarray, np.ndarray], np.ndarray],
+               epsilon: float = EPSILON) -> BM25Remove:
+    """The plan of removing documents ``ids`` from an index, equal to what a rebuild over the
+    remaining documents computes.  ``vocab`` (insertion order = id order) and ``df`` describe the
+    index, ``first_doc[t]`` is the first document of term t (``postings[term_ptr[t]]``);
+    ``doc_tokens(d)`` tokenises document d; ``first_postings(terms, counts)`` returns the documents of
+    the first ``counts[i]`` postings of each ``terms[i]``, concatenated.
+
+    A rebuild numbers terms in first-appearance order over the remaining documents, i.e. by the key
+    (first surviving document, position of the term's first occurrence among that document's
+    distinct tokens).  Old ids already follow that key, so a term whose first document survives
+    keeps its place relative to the other such terms.  Only an *affected* term (its first document
+    removed) moves: its new first document is among its first ``r_t + 1`` postings (r_t = its removed
+    count), and the position comes from tokenising that one document.  The affected terms, sorted by
+    key, are merged into the others; okapi_idf over the document frequencies in that order gives
+    every idf bit of the rebuild.  Work: O(removed tokens + affected terms + tokens of their new first
+    documents + V); no pass over the postings, no other document read."""
+    V = len(vocab)
+    ids = np.asarray(ids, dtype=np.int64).reshape(-1)
+    removed = np.unique(ids)
+    if len(removed) != len(ids):
+        raise ValueError("duplicate ids")
+    if len(removed) and (removed[0] < 0 or removed[-1] >= n_docs):
+        raise ValueError(f"ids must lie in [0, {n_docs})")
+    n_out = int(n_docs) - len(removed)
+    if n_out <= 0:
+        raise ValueError("removing every document: the BM25 statistics of an empty corpus are undefined")
+    t_l, d_l = [], []
+    len_rem = 0
+    for d in removed.tolist():
+        tokens = doc_tokens(d)
+        len_rem += len(tokens)
+        for word in dict.fromkeys(tokens):
+            t = vocab.get(word)
+            if t is None:
+                raise ValueError(f"document {d}: token {word!r} is not in the index's vocabulary")
+            t_l.append(t); d_l.append(d)
+    t = np.asarray(t_l, dtype=np.int64)
+    d = np.asarray(d_l, dtype=np.int64)
+    order = np.lexsort((d, t))
+    t, d = t[order], d[order]
+    r = np.bincount(t, minlength=V).astype(np.int64)
+    rem_ptr = np.zeros(V + 1, dtype=np.int64)
+    np.cumsum(r, out=rem_ptr[1:])
+    df_after = np.asarray(df, dtype=np.int64) - r
+    if (df_after < 0).any():
+        raise ValueError("the removed documents' tokens do not match the index's postings")
+    alive = df_after > 0
+    first = np.asarray(first_doc, dtype=np.int64)
+    is_removed = lambda a: removed[np.minimum(np.searchsorted(removed, a), len(removed) - 1)] == a
+    # affected: alive terms whose first document is removed (only terms with r_t > 0 can be)
+    cand = np.nonzero(r)[0]
+    aff = cand[alive[cand] & is_removed(first[cand])] if len(removed) else cand[:0]
+    first_after = first.copy()
+    if len(aff):
+        counts = r[aff] + 1
+        docs = np.asarray(first_postings(aff, counts), dtype=np.int64)
+        idx = np.where(is_removed(docs), len(docs), np.arange(len(docs)))
+        pick = np.minimum.reduceat(idx, np.cumsum(counts) - counts)
+        if (pick >= len(docs)).any():
+            raise ValueError("the removed documents' tokens do not match the index's postings")
+        first_after[aff] = docs[pick]
+    # within-document positions, from the new first documents of the affected terms
+    pos = np.zeros(V, dtype=np.int64)
+    for f in np.unique(first_after[aff]).tolist():
+        for p, word in enumerate(dict.fromkeys(doc_tokens(f))):
+            t = vocab.get(word)
+            if t is None:
+                raise ValueError(f"document {f}: token {word!r} is not in the index's vocabulary")
+            if first_after[t] == f:
+                pos[t] = p
+    key = (first_after << 17) + pos                     # a document has < 2^16 distinct tokens
+    is_aff = np.zeros(V, dtype=bool)
+    is_aff[aff] = True
+    keep = np.nonzero(alive & ~is_aff)[0]               # already in key order
+    a_sorted = aff[np.argsort(key[aff], kind="stable")]
+    new_order = np.insert(keep, np.searchsorted(key[keep], key[a_sorted]), a_sorted)
+    term_map = np.full(V, -1, dtype=np.int32)
+    term_map[new_order] = np.arange(len(new_order), dtype=np.int32)
+    df_out = df_after[new_order]
+    term_ptr = np.zeros(len(new_order) + 1, dtype=np.int64)
+    np.cumsum(df_out, out=term_ptr[1:])
+    words = list(vocab)
+    f_new = first_after[new_order]
+    len_out = int(total_len) - len_rem
+    idf, _ = okapi_idf(df_out, n_out, epsilon)
+    return BM25Remove(removed, rem_ptr, d.astype(np.uint32), term_map, term_ptr,
+                      [words[i] for i in new_order.tolist()], f_new - np.searchsorted(removed, f_new), df_out,
+                      n_out, len_out, idf, len_out / n_out)
+
+
+def compact_csr(term_ptr: np.ndarray, postings: np.ndarray, n_docs: int, removed: np.ndarray,
+                term_map: np.ndarray, term_ptr_out: np.ndarray):
+    """Host compaction (the device does the same in lrx_bm25_remove_postings), linear in the postings:
+    a document map (new id, -1 = removed) renumbers every posting, and kept posting i of term t goes
+    to ``term_ptr_out[term_map[t]] + (i - term_ptr[t]) - k`` with k the removed postings of t before
+    it (a running count).  Returns (term_ptr uint64 [V_out+1], postings uint32 [nnz_out, 2])."""
+    old_ptr = np.asarray(term_ptr, dtype=np.int64)
+    out_ptr = np.asarray(term_ptr_out, dtype=np.int64)
+    mark = np.zeros(n_docs, dtype=bool)
+    mark[removed] = True
+    doc_map = np.arange(n_docs, dtype=np.int64) - np.cumsum(mark)
+    doc_map[mark] = -1
+    new_doc = doc_map[postings[:, 0]]
+    gone = new_doc < 0
+    k = np.cumsum(gone)                                  # removed postings up to posting i ...
+    before = np.concatenate([[0], k])[old_ptr[:-1]]      # ... and before each term's first posting
+    dst = np.arange(len(postings), dtype=np.int64) - k
+    dst += np.repeat(out_ptr[np.maximum(term_map, 0)] - old_ptr[:-1] + before, np.diff(old_ptr))
+    keep = ~gone
+    out = np.empty((int(out_ptr[-1]), 2), dtype=np.uint32)
+    assert int(keep.sum()) == len(out), "the removal plan does not describe these postings"
+    out[dst[keep], 0] = new_doc[keep]
+    out[dst[keep], 1] = postings[keep, 1]
+    return out_ptr.astype(np.uint64), out
+
+
+def remove_csr(term_ptr: np.ndarray, postings: np.ndarray, rem: BM25Remove):
+    """compact_csr for a removal plan: the postings of the removed documents dropped, the others
+    renumbered and moved to their term's new id."""
+    return compact_csr(term_ptr, postings, rem.n_docs + len(rem.removed), rem.removed, rem.term_map,
+                       rem.term_ptr)
+
+
 @dataclass
 class BM25Index:
     n_docs: int
@@ -217,6 +381,23 @@ class BM25Index:
         vocab.update((w, len(self.vocab) + i) for i, w in enumerate(app.new_words))
         return BM25Index(app.n_docs, np.concatenate([self.doc_len, app.doc_len]), term_ptr, postings,
                          app.idf, app.avgdl, vocab, self.k1, self.b, self.epsilon)
+
+    # ------------------------------------------------------------------ remove
+    def remove(self, ids: Sequence[int], doc_tokens: Callable[[int], Sequence[str]]) -> "BM25Index":
+        """This index without documents ``ids`` (the others renumbered by rank): equal, field by field
+        and bit for bit, to ``from_token_lists(remaining documents)``, vocabulary order included.
+        ``doc_tokens(d)`` tokenises document d; only the removed documents and the new first
+        documents of the terms that lose theirs are read (``csr_remove``)."""
+        if self.vocab is None:
+            raise ValueError("index has no string vocabulary")
+        tp = self.term_ptr.astype(np.int64)
+        first = self.postings[np.minimum(tp[:-1], max(self.nnz - 1, 0)), 0].astype(np.int64)
+        gather = lambda terms, counts: self.postings[_ranges(tp[terms], counts), 0]
+        rem = csr_remove(self.vocab, np.diff(tp), first, self.n_docs, int(self.doc_len.astype(np.int64).sum()),
+                         ids, doc_tokens, gather, self.epsilon)
+        term_ptr, postings = remove_csr(self.term_ptr, self.postings, rem)
+        return BM25Index(rem.n_docs, np.delete(self.doc_len, rem.removed), term_ptr, postings, rem.idf, rem.avgdl,
+                         {w: i for i, w in enumerate(rem.words)}, self.k1, self.b, self.epsilon)
 
     # ------------------------------------------------------------------ query
     def term_ids(self, tokens: Sequence[str]) -> List[int]:

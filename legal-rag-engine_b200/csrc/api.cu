@@ -165,7 +165,7 @@ int lrx_close(lrx_handle* h) {
         for (cudaEvent_t e : h->prof_ev[w]) cudaEventDestroy(e);
     if (h->cap) cudaStreamDestroy(h->cap);
     if (h->pack_done) cudaFree(h->pack_done);
-    void* ws[] = {h->ws_dense_part, h->ws_bm_part, h->ws_bm_max, h->ws_misc, h->ws_io};
+    void* ws[] = {h->ws_dense_part, h->ws_bm_part, h->ws_bm_max, h->ws_misc, h->ws_io, h->ws_rm};
     for (void* p : ws)
         if (p != nullptr) cudaFree(p);
     encoder_free(h);
@@ -386,6 +386,42 @@ int lrx_bm25_append_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const 
     if (bad)
         return fail(h, LRX_E_ARG, "lrx_bm25_append_postings: a term frequency or document length "
                                   "exceeds 65535, or an appended doc id is outside [n_docs_old, n_docs_out)");
+    return LRX_OK;
+}
+
+int lrx_bm25_remove_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const void* dev_postings,
+                             int64_t n_terms, int64_t nnz, int64_t n_docs_old,
+                             const uint32_t* dev_removed_docs, int64_t n_removed,
+                             const uint64_t* dev_rem_ptr, const uint32_t* dev_rem_doc,
+                             const int32_t* dev_term_map, const uint64_t* dev_term_ptr_out,
+                             int64_t n_terms_out, void* dev_postings_out) {
+    if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_bm25_remove_postings: null handle");
+    std::lock_guard<std::mutex> g(h->mu);
+    if (n_terms < 0 || nnz < 0 || n_docs_old < 0 || n_docs_old >= (1ll << 32) || n_removed < 0 ||
+        n_removed > n_docs_old || n_terms_out < 0 || n_terms_out > n_terms)
+        return fail(h, LRX_E_ARG, "lrx_bm25_remove_postings: bad size");
+    if (dev_term_ptr == nullptr || dev_rem_ptr == nullptr || dev_term_ptr_out == nullptr ||
+        (n_terms > 0 && dev_term_map == nullptr) || (n_removed > 0 && dev_removed_docs == nullptr) ||
+        (nnz > 0 && (dev_postings == nullptr || dev_postings_out == nullptr)))
+        return fail(h, LRX_E_ARG, "lrx_bm25_remove_postings: null pointer");
+    if ((((uintptr_t)dev_postings | (uintptr_t)dev_postings_out) & 15) != 0 ||
+        (((uintptr_t)dev_term_ptr | (uintptr_t)dev_rem_ptr | (uintptr_t)dev_term_ptr_out) & 7) != 0 ||
+        (((uintptr_t)dev_removed_docs | (uintptr_t)dev_rem_doc | (uintptr_t)dev_term_map) & 3) != 0)
+        return fail(h, LRX_E_ARG, "lrx_bm25_remove_postings: postings must be 16-byte aligned, pointer "
+                                  "tables 8-byte aligned, id arrays 4-byte aligned");
+    LRX_CUDA(h, cudaSetDevice(h->device));
+    int bad = 0;
+    LRX_CUDA(h, launch_bm25_remove(h, dev_term_ptr, dev_postings, n_terms, nnz, n_docs_old, dev_removed_docs,
+                                   n_removed, dev_rem_ptr, dev_rem_doc, dev_term_map, dev_term_ptr_out,
+                                   n_terms_out, dev_postings_out, &bad));
+    if (bad == 2)
+        return fail(h, LRX_E_ARG, "lrx_bm25_remove_postings: term_ptr[n_terms] != nnz, term_ptr_out[0] != 0 "
+                                  "or term_ptr_out[n_terms_out] != nnz - rem_ptr[n_terms]");
+    if (bad)
+        return fail(h, LRX_E_ARG, "lrx_bm25_remove_postings: the removal does not describe the index (removed "
+                                  "ids unsorted or out of range, a removed list unsorted or not the term's "
+                                  "removed postings, term_map not a bijection onto the surviving terms, or an "
+                                  "output range of the wrong length)");
     return LRX_OK;
 }
 

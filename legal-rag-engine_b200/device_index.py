@@ -193,6 +193,77 @@ class DeviceIndex:
         self.doc_len = dl if dl.numel() else self.doc_len
         self.n_terms, self.n_docs = n_terms_out, n_old + m
 
+    def remove_rows(self, keep, prefilter: Optional[bool] = None, chunk: int = 1 << 20):
+        """Keep only the rows `keep` (ascending local ids, or a bool mask over n_local), moved to the
+        front of the capacity buffer in order.  The kept ids ascend, so every row moves toward the
+        front: the move runs in place, `chunk` rows at a time through one temporary allocated before
+        the first row moves.  `prefilter` (default: as before) rebuilds the int8 shadow."""
+        keep = keep.to(self.device) if isinstance(keep, torch.Tensor) else torch.as_tensor(np.asarray(keep),
+                                                                                          device=self.device)
+        idx = torch.nonzero(keep).flatten() if keep.dtype == torch.bool else keep.to(torch.int64)
+        n, buf = int(idx.numel()), self._xbuf
+        tmp = torch.empty((min(n, chunk), LRX_DIM), dtype=torch.float16, device=self.device)
+        for a in range(0, n, chunk):                        # sources of later chunks lie past a + chunk
+            c = min(chunk, n - a)
+            torch.index_select(self.x, 0, idx[a:a + c], out=tmp[:c])
+            buf[a:a + c].copy_(tmp[:c])
+        del tmp
+        if prefilter is None:
+            prefilter = self._prefilter_on
+        self._q8 = None                                     # the shadow of the old matrix
+        self.set_corpus(buf[:n], self.id_base, prefilter=prefilter)
+        self._xbuf = buf
+
+    def posting_docs(self, terms: np.ndarray, counts: np.ndarray) -> np.ndarray:
+        """Documents of the first counts[i] resident postings of each terms[i], concatenated."""
+        tp, p8, _ = self._post
+        t = torch.from_numpy(np.ascontiguousarray(terms, dtype=np.int64)).to(self.device)
+        c = torch.from_numpy(np.ascontiguousarray(counts, dtype=np.int64)).to(self.device)
+        excl = torch.cumsum(c, 0) - c
+        idx = torch.repeat_interleave(tp[t] - excl, c) + torch.arange(int(counts.sum()), device=self.device)
+        return (p8[idx, 0].to(torch.int64) & 0xFFFFFFFF).cpu().numpy()
+
+    def compact_postings(self, rem):
+        """The resident postings without the documents of a removal plan (bm25_index.BM25Remove),
+        compacted on the device into new buffers (lrx_bm25_remove_postings), with the compacted
+        doc_len: a staged index for `commit_postings`.  The handle is not changed; a plan that does
+        not describe the postings raises LrxError (LRX_E_ARG)."""
+        tp, p8, _ = self._post
+        nnz = self._post_args[0]
+        up = lambda a, dt, v: torch.from_numpy(np.ascontiguousarray(a, dtype=dt).view(v)).to(self.device)
+        removed = up(rem.removed, np.uint32, np.int32)
+        rem_ptr = up(rem.rem_ptr, np.int64, np.int64)
+        rem_doc = up(rem.rem_doc, np.uint32, np.int32)
+        term_map = up(rem.term_map, np.int32, np.int32)
+        tp_out = up(rem.term_ptr, np.int64, np.int64)
+        n_terms_out, nnz_out = rem.n_terms, rem.nnz
+        p8_out = torch.empty((nnz_out + 2, 2), dtype=torch.int32, device=self.device)
+        self._ck(self.lib.lrx_bm25_remove_postings(
+            self.h, _ptr(tp), _ptr(p8), self.n_terms, nnz, self.n_docs, _ptr(removed), len(rem.removed),
+            _ptr(rem_ptr), _ptr(rem_doc), _ptr(term_map), _ptr(tp_out), n_terms_out, _ptr(p8_out)))
+        keep = torch.ones(self.n_docs, dtype=torch.bool, device=self.device)
+        keep[removed.to(torch.int64)] = False
+        dl = self.doc_len[:self.n_docs][keep]
+        idf_t = torch.from_numpy(np.ascontiguousarray(rem.idf, dtype=np.float64)).to(self.device)
+        return tp_out, p8_out, idf_t, dl, float(rem.avgdl), int(dl.max().item())
+
+    def commit_postings(self, staged):
+        """Make a staged index of `compact_postings` resident (lrx_set_postings); the old buffers are
+        dropped after the handle has taken the new ones."""
+        tp_out, p8_out, idf_t, dl, avgdl, max_len = staged
+        _, _, k1, b, _ = self._post_args
+        n_terms_out, nnz_out = int(tp_out.numel() - 1), int(p8_out.shape[0] - 2)
+        self._ck(self.lib.lrx_set_postings(self.h, _ptr(tp_out), _ptr(p8_out), _ptr(idf_t), n_terms_out, nnz_out,
+                                           avgdl, k1, b, max_len))
+        self._post = (tp_out, p8_out, idf_t)
+        self._post_args = (nnz_out, avgdl, k1, b, max_len)
+        self.doc_len = dl
+        self.n_terms, self.n_docs = n_terms_out, int(dl.numel())
+
+    def remove_postings(self, rem):
+        """compact_postings + commit_postings: a failure leaves the index as it was."""
+        self.commit_postings(self.compact_postings(rem))
+
     def clone_view(self) -> "DeviceIndex":
         """A second handle (own stream binding, workspaces, exchange region) over the SAME resident
         matrix and postings -- no copies: lets two query batches be in flight on two streams, one

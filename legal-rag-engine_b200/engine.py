@@ -6,8 +6,8 @@ store directory; everything numeric runs in the CUDA library behind include/lrx.
 
 Additive surface only: ``search_batch`` (the orchestrator's concept-expansion fan-out in one
 launch chain, orchestrator.py:38-62), ``fusion="linear"|"rrf"`` (default "linear" = the
-reference's behaviour, retrieval_engine.py:71-96), ``encode``, ``add_chunks`` / ``save`` (grow a
-loaded index without a rebuild; results stay bit-identical to a rebuild).
+reference's behaviour, retrieval_engine.py:71-96), ``encode``, ``add_chunks`` / ``remove_chunks`` /
+``save`` (grow or shrink a loaded index without a rebuild; results stay bit-identical to a rebuild).
 
 There is no CPU fallback: without a CUDA device or the built library the constructor raises.
 """
@@ -28,7 +28,7 @@ import torch
 
 from . import store as _store
 from ._lib import LRX_MAX_BATCH, LRX_MAX_DEPTH
-from .bm25_index import BM25Index, csr_append, merge_csr, tokenize
+from .bm25_index import BM25Index, BM25Append, compact_csr, csr_append, csr_remove, merge_csr, tokenize
 from .device_index import FUSION, DeviceIndex
 from .encoder import SentenceEncoder
 from .sharding import shard_range
@@ -98,11 +98,13 @@ class RetrievalEngine:
         self.chunks, xh, bm25 = _store.load_store(self.store_dir, mmap=self.world > 1)
         self.n_total = len(self.chunks)
         self.lo, self.hi = shard_range(self.n_total, self.rank, self.world)
-        self._lock = threading.Lock()                      # searches see the index before or after an add
+        self._lock = threading.Lock()                      # searches see the index before or after a change
         self._bm25 = bm25                                  # whole-corpus statistics + vocabulary
-        self._bm25_pending = []                            # appended CSRs not yet merged into _bm25's postings
-        self._df = np.diff(bm25.term_ptr.astype(np.int64))
+        self._bm25_pending = []                            # appends / removals not yet applied to _bm25's postings
+        tp = bm25.term_ptr.astype(np.int64)
+        self._df = np.diff(tp)
         self._total_len = int(bm25.doc_len.astype(np.int64).sum())
+        self._first = bm25.postings[np.minimum(tp[:-1], max(bm25.nnz - 1, 0)), 0].astype(np.int64)
         local = bm25 if self.world == 1 else bm25.shard(self.lo, self.hi)
         self._x = torch.from_numpy(np.ascontiguousarray(xh[self.lo:self.hi])).to(self.dev.device)
         self.dev.set_corpus(self._x, self.lo)
@@ -217,9 +219,15 @@ class RetrievalEngine:
 
     def _bm25_current(self) -> BM25Index:
         b = self._bm25
-        for app in self._bm25_pending:
-            b.term_ptr, b.postings = merge_csr(b.term_ptr, b.postings, app)
-            b.doc_len = np.concatenate([b.doc_len, app.doc_len])
+        for op in self._bm25_pending:                      # in the order they were made
+            if isinstance(op, BM25Append):
+                b.term_ptr, b.postings = merge_csr(b.term_ptr, b.postings, op)
+                b.doc_len = np.concatenate([b.doc_len, op.doc_len])
+            else:
+                _, n_old, removed, term_map, term_ptr_out = op
+                b.term_ptr, b.postings = compact_csr(b.term_ptr, b.postings, n_old, removed, term_map,
+                                                     term_ptr_out)
+                b.doc_len = np.delete(b.doc_len, removed)
         self._bm25_pending = []
         return b
 
@@ -256,10 +264,63 @@ class RetrievalEngine:
             b.n_docs, b.idf, b.avgdl = app.n_docs, app.idf, app.avgdl
             self._bm25_pending.append(app)
             self._df, self._total_len = app.df, app.total_len
+            self._first = np.concatenate([self._first, app.postings[app.term_ptr[base:-1], 0].astype(np.int64)])
             self.chunks.extend(chunks)
             self.n_total = self.hi = len(self.chunks)
             self._x = self.dev.x
             return range(n, self.n_total)
+
+    def remove_chunks(self, ids: Sequence[int]) -> np.ndarray:
+        """Remove chunks (positions in ``self.chunks``) from the loaded index.  Returns the map from
+        old to new ids (int64, -1 for a removed chunk): the remaining chunks keep their order and are
+        numbered by rank.  Searches afterwards return exactly what an engine over a store rebuilt
+        from the remaining chunks (with their current rows) returns.  Ids must be ints, in range and
+        unique, and at least one chunk must remain; a rejected call raises and leaves the engine as
+        it was.  To replace a chunk, remove it and add the new version.  Not supported on a sharded
+        engine (world > 1)."""
+        if self.world > 1:
+            raise NotImplementedError("remove_chunks on a sharded engine: rebuild the store instead")
+        ids = list(ids)
+        for i in ids:
+            if isinstance(i, (bool, np.bool_)) or not isinstance(i, (int, np.integer)):
+                raise TypeError(f"chunk ids must be ints, got {i!r}")
+        with self._lock:
+            n = self.n_total
+            ids_arr = np.asarray(ids, dtype=np.int64).reshape(-1)
+            if len(ids_arr) and (ids_arr.min() < 0 or ids_arr.max() >= n):
+                raise ValueError(f"chunk ids must lie in [0, {n})")
+            if len(np.unique(ids_arr)) != len(ids_arr):
+                raise ValueError("duplicate chunk ids")
+            if len(ids_arr) >= n:
+                raise ValueError("removing every chunk: the BM25 statistics of an empty corpus are undefined")
+            ids_map = np.arange(n, dtype=np.int64)
+            if not len(ids_arr):
+                return ids_map
+            b = self._bm25
+            rem = csr_remove(b.vocab, self._df, self._first, b.n_docs, self._total_len, ids_arr,
+                             lambda d: tokenize(self.chunks[d]["text"]), self.dev.posting_docs, b.epsilon)
+            keep = np.ones(n, dtype=bool)
+            keep[rem.removed] = False
+            # every step that allocates or checks runs before the handle takes the new postings: the
+            # compaction into new buffers (which validates the plan), then the in-place row move
+            # through one bounded temporary; the int8 shadow is rebuilt last, over a consistent index
+            staged = self.dev.compact_postings(rem)
+            prefilter = self.dev._prefilter_on
+            self.dev.remove_rows(keep, prefilter=False)
+            self.dev.commit_postings(staged)
+            del staged
+            b.vocab = {w: i for i, w in enumerate(rem.words)}
+            b.n_docs, b.idf, b.avgdl = rem.n_docs, rem.idf, rem.avgdl
+            self._bm25_pending.append(("remove", n, rem.removed, rem.term_map, rem.term_ptr))
+            self._df, self._total_len, self._first = rem.df, rem.total_len, rem.first_doc
+            self.chunks = [c for c, k in zip(self.chunks, keep.tolist()) if k]
+            self.n_total = self.hi = len(self.chunks)
+            self._x = self.dev.x
+            ids_map[~keep] = -1
+            ids_map[keep] = np.arange(self.n_total, dtype=np.int64)
+            if prefilter:
+                self.dev.build_prefilter()
+            return ids_map
 
     def save(self, store_dir: Optional[str] = None) -> Path:
         """Write the current index (added chunks included) as a store that ``RetrievalEngine`` and
