@@ -39,18 +39,31 @@ def okapi_idf(df: np.ndarray, n_docs: int, epsilon: float = EPSILON):
 
 
 @dataclass
+class BM25Stats:
+    """What planning an add or a removal reads.  A plan's ``stats`` describe the corpus after the
+    change except its ``vocab``, the planner's input dict left as it was (an abandoned plan changes
+    nothing, and a small plan does not pay for a copy of a large dict): ``commit_vocab`` updates it."""
+    vocab: Dict[str, int]
+    df: np.ndarray               # int64 [V]
+    first_doc: np.ndarray        # int64 [V] each term's first document (postings[term_ptr[t]])
+    n_docs: int
+    total_len: int               # tokens
+    idf: np.ndarray              # float64 [V]
+    avgdl: float
+    k1: float = K1
+    b: float = B
+    epsilon: float = EPSILON
+
+
+@dataclass
 class BM25Append:
     """Documents appended to an index: their own term-major CSR over the extended vocabulary, and
     the whole corpus's statistics after the append."""
-    new_words: List[str]         # vocabulary extension, first-appearance order: ids n_terms, n_terms + 1, ...
     term_ptr: np.ndarray         # int64 [V_out+1]
     postings: np.ndarray         # uint32 [nnz_add, 2] = (doc id, tf), doc ids >= the old n_docs
     doc_len: np.ndarray          # uint32 [m]
-    df: np.ndarray               # int64 [V_out] document frequencies, old + appended documents
-    n_docs: int                  # after the append
-    total_len: int               # tokens after the append
-    idf: np.ndarray              # float64 [V_out]
-    avgdl: float
+    new_words: List[str]         # vocabulary extension, first-appearance order: ids V, V + 1, ...
+    stats: BM25Stats
 
     @property
     def n_terms(self) -> int:
@@ -60,18 +73,23 @@ class BM25Append:
     def nnz(self) -> int:
         return int(self.term_ptr[-1])
 
+    def commit_vocab(self):
+        """Extend ``stats.vocab`` in place by the new words."""
+        base = len(self.stats.vocab)
+        self.stats.vocab.update((w, base + i) for i, w in enumerate(self.new_words))
 
-def csr_append(vocab: Dict[str, int], df: np.ndarray, n_docs: int, total_len: int,
-               token_lists: Sequence[Sequence[str]], epsilon: float = EPSILON) -> BM25Append:
+
+def csr_append(stats: BM25Stats, token_lists: Sequence[Sequence[str]]) -> BM25Append:
     """The appended documents' CSR and the updated statistics, in O(new tokens + V): no pass over
-    the existing postings.  ``vocab`` is read, not changed.  A rebuild numbers terms in first
+    the existing postings.  ``stats`` is read, not changed.  A rebuild numbers terms in first
     appearance order over all documents in order; the old documents come first, so it keeps every
     old id and numbers the new terms in first-appearance order over the appended documents -- the
     order used here -- and okapi_idf's sequential mean, hence every idf bit, comes out the same."""
+    vocab = stats.vocab
     new: Dict[str, int] = {}
     n_old = len(vocab)
     t_l, d_l, f_l, lens = [], [], [], []
-    for d, document in enumerate(token_lists, start=n_docs):
+    for d, document in enumerate(token_lists, start=stats.n_docs):
         lens.append(len(document))
         freqs: Dict[str, int] = {}
         for word in document:
@@ -96,13 +114,15 @@ def csr_append(vocab: Dict[str, int], df: np.ndarray, n_docs: int, total_len: in
     postings[:, 0] = d
     postings[:, 1] = f
     df_out = np.zeros(n_out, dtype=np.int64)
-    df_out[:n_old] = df
+    df_out[:n_old] = stats.df
     df_out += count
-    n_all = int(n_docs) + len(lens)
-    len_all = int(total_len) + sum(lens)
-    idf, _ = okapi_idf(df_out, n_all, epsilon)
-    return BM25Append(list(new), term_ptr, postings, np.asarray(lens, dtype=np.uint32), df_out, n_all,
-                      len_all, idf, len_all / n_all)
+    first = np.concatenate([stats.first_doc, d[term_ptr[n_old:-1]]])
+    n_all = int(stats.n_docs) + len(lens)
+    len_all = int(stats.total_len) + sum(lens)
+    idf, _ = okapi_idf(df_out, n_all, stats.epsilon)
+    return BM25Append(term_ptr, postings, np.asarray(lens, dtype=np.uint32), list(new),
+                      BM25Stats(vocab, df_out, first, n_all, len_all, idf, len_all / n_all, stats.k1, stats.b,
+                                stats.epsilon))
 
 
 def merge_csr(term_ptr: np.ndarray, postings: np.ndarray, app: BM25Append):
@@ -137,13 +157,7 @@ class BM25Remove:
     rem_doc: np.ndarray          # uint32 [nnz_rem] ... ascending
     term_map: np.ndarray         # int32 [V] old term id -> new id, -1 = no surviving posting
     term_ptr: np.ndarray         # int64 [V_out+1] the compacted CSR's pointers
-    words: List[str]             # the new vocabulary, new id order
-    first_doc: np.ndarray        # int64 [V_out] each term's first document (new ids)
-    df: np.ndarray               # int64 [V_out]
-    n_docs: int                  # after the removal
-    total_len: int               # tokens after the removal
-    idf: np.ndarray              # float64 [V_out]
-    avgdl: float
+    stats: BM25Stats             # after the removal, new term and document ids
 
     @property
     def n_terms(self) -> int:
@@ -157,14 +171,19 @@ class BM25Remove:
     def nnz_rem(self) -> int:
         return int(self.rem_ptr[-1])
 
+    def commit_vocab(self):
+        """Renumber ``stats.vocab`` in place: the surviving terms, in new id order."""
+        words = list(self.stats.vocab)
+        live = np.flatnonzero(self.term_map >= 0)
+        order = live[np.argsort(self.term_map[live])]
+        self.stats.vocab.clear()
+        self.stats.vocab.update(zip(map(words.__getitem__, order.tolist()), range(len(order))))
 
-def csr_remove(vocab: Dict[str, int], df: np.ndarray, first_doc: np.ndarray, n_docs: int, total_len: int,
-               ids: Sequence[int], doc_tokens: Callable[[int], Sequence[str]],
-               first_postings: Callable[[np.ndarray, np.ndarray], np.ndarray],
-               epsilon: float = EPSILON) -> BM25Remove:
+
+def csr_remove(stats: BM25Stats, ids: Sequence[int], doc_tokens: Callable[[int], Sequence[str]],
+               first_postings: Callable[[np.ndarray, np.ndarray], np.ndarray]) -> BM25Remove:
     """The plan of removing documents ``ids`` from an index, equal to what a rebuild over the
-    remaining documents computes.  ``vocab`` (insertion order = id order) and ``df`` describe the
-    index, ``first_doc[t]`` is the first document of term t (``postings[term_ptr[t]]``);
+    remaining documents computes.  ``stats`` describes the index and is read, not changed;
     ``doc_tokens(d)`` tokenises document d; ``first_postings(terms, counts)`` returns the documents of
     the first ``counts[i]`` postings of each ``terms[i]``, concatenated.
 
@@ -177,6 +196,7 @@ def csr_remove(vocab: Dict[str, int], df: np.ndarray, first_doc: np.ndarray, n_d
     key, are merged into the others; okapi_idf over the document frequencies in that order gives
     every idf bit of the rebuild.  Work: O(removed tokens + affected terms + tokens of their new first
     documents + V); no pass over the postings, no other document read."""
+    vocab, n_docs = stats.vocab, stats.n_docs
     V = len(vocab)
     ids = np.asarray(ids, dtype=np.int64).reshape(-1)
     removed = np.unique(ids)
@@ -204,11 +224,11 @@ def csr_remove(vocab: Dict[str, int], df: np.ndarray, first_doc: np.ndarray, n_d
     r = np.bincount(t, minlength=V).astype(np.int64)
     rem_ptr = np.zeros(V + 1, dtype=np.int64)
     np.cumsum(r, out=rem_ptr[1:])
-    df_after = np.asarray(df, dtype=np.int64) - r
+    df_after = stats.df - r
     if (df_after < 0).any():
         raise ValueError("the removed documents' tokens do not match the index's postings")
     alive = df_after > 0
-    first = np.asarray(first_doc, dtype=np.int64)
+    first = stats.first_doc
     is_removed = lambda a: removed[np.minimum(np.searchsorted(removed, a), len(removed) - 1)] == a
     # affected: alive terms whose first document is removed (only terms with r_t > 0 can be)
     cand = np.nonzero(r)[0]
@@ -242,25 +262,25 @@ def csr_remove(vocab: Dict[str, int], df: np.ndarray, first_doc: np.ndarray, n_d
     df_out = df_after[new_order]
     term_ptr = np.zeros(len(new_order) + 1, dtype=np.int64)
     np.cumsum(df_out, out=term_ptr[1:])
-    words = list(vocab)
     f_new = first_after[new_order]
-    len_out = int(total_len) - len_rem
-    idf, _ = okapi_idf(df_out, n_out, epsilon)
+    len_out = int(stats.total_len) - len_rem
+    idf, _ = okapi_idf(df_out, n_out, stats.epsilon)
     return BM25Remove(removed, rem_ptr, d.astype(np.uint32), term_map, term_ptr,
-                      [words[i] for i in new_order.tolist()], f_new - np.searchsorted(removed, f_new), df_out,
-                      n_out, len_out, idf, len_out / n_out)
+                      BM25Stats(vocab, df_out, f_new - np.searchsorted(removed, f_new), n_out, len_out, idf,
+                                len_out / n_out, stats.k1, stats.b, stats.epsilon))
 
 
-def compact_csr(term_ptr: np.ndarray, postings: np.ndarray, n_docs: int, removed: np.ndarray,
-                term_map: np.ndarray, term_ptr_out: np.ndarray):
+def remove_csr(term_ptr: np.ndarray, postings: np.ndarray, rem: BM25Remove):
     """Host compaction (the device does the same in lrx_bm25_remove_postings), linear in the postings:
-    a document map (new id, -1 = removed) renumbers every posting, and kept posting i of term t goes
-    to ``term_ptr_out[term_map[t]] + (i - term_ptr[t]) - k`` with k the removed postings of t before
-    it (a running count).  Returns (term_ptr uint64 [V_out+1], postings uint32 [nnz_out, 2])."""
+    the postings of the removed documents dropped, the others renumbered and moved to their term's
+    new id.  A document map (new id, -1 = removed) renumbers every posting, and kept posting i of term
+    t goes to ``rem.term_ptr[term_map[t]] + (i - term_ptr[t]) - k`` with k the removed postings of t
+    before it (a running count).  Returns (term_ptr uint64 [V_out+1], postings uint32 [nnz_out, 2])."""
     old_ptr = np.asarray(term_ptr, dtype=np.int64)
-    out_ptr = np.asarray(term_ptr_out, dtype=np.int64)
+    out_ptr = np.asarray(rem.term_ptr, dtype=np.int64)
+    n_docs = rem.stats.n_docs + len(rem.removed)
     mark = np.zeros(n_docs, dtype=bool)
-    mark[removed] = True
+    mark[rem.removed] = True
     doc_map = np.arange(n_docs, dtype=np.int64) - np.cumsum(mark)
     doc_map[mark] = -1
     new_doc = doc_map[postings[:, 0]]
@@ -268,20 +288,13 @@ def compact_csr(term_ptr: np.ndarray, postings: np.ndarray, n_docs: int, removed
     k = np.cumsum(gone)                                  # removed postings up to posting i ...
     before = np.concatenate([[0], k])[old_ptr[:-1]]      # ... and before each term's first posting
     dst = np.arange(len(postings), dtype=np.int64) - k
-    dst += np.repeat(out_ptr[np.maximum(term_map, 0)] - old_ptr[:-1] + before, np.diff(old_ptr))
+    dst += np.repeat(out_ptr[np.maximum(rem.term_map, 0)] - old_ptr[:-1] + before, np.diff(old_ptr))
     keep = ~gone
     out = np.empty((int(out_ptr[-1]), 2), dtype=np.uint32)
     assert int(keep.sum()) == len(out), "the removal plan does not describe these postings"
     out[dst[keep], 0] = new_doc[keep]
     out[dst[keep], 1] = postings[keep, 1]
     return out_ptr.astype(np.uint64), out
-
-
-def remove_csr(term_ptr: np.ndarray, postings: np.ndarray, rem: BM25Remove):
-    """compact_csr for a removal plan: the postings of the removed documents dropped, the others
-    renumbered and moved to their term's new id."""
-    return compact_csr(term_ptr, postings, rem.n_docs + len(rem.removed), rem.removed, rem.term_map,
-                       rem.term_ptr)
 
 
 @dataclass
@@ -305,7 +318,22 @@ class BM25Index:
     def nnz(self) -> int:
         return int(self.term_ptr[-1])
 
+    def stats(self) -> BM25Stats:
+        """The statistics planning reads (csr_append, csr_remove), with a copy of the vocabulary."""
+        if self.vocab is None:
+            raise ValueError("index has no string vocabulary")
+        tp = self.term_ptr.astype(np.int64)
+        first = self.postings[np.minimum(tp[:-1], max(self.nnz - 1, 0)), 0].astype(np.int64)
+        return BM25Stats(dict(self.vocab), np.diff(tp), first, self.n_docs, int(self.doc_len.astype(np.int64).sum()),
+                         self.idf, self.avgdl, self.k1, self.b, self.epsilon)
+
     # ------------------------------------------------------------------ build
+    @classmethod
+    def from_stats(cls, stats: BM25Stats, term_ptr, postings, doc_len) -> "BM25Index":
+        """The index with these statistics over these postings, with a copy of the vocabulary."""
+        return cls(stats.n_docs, doc_len, term_ptr, postings, stats.idf, stats.avgdl, dict(stats.vocab), stats.k1,
+                   stats.b, stats.epsilon)
+
     @classmethod
     def from_postings(cls, n_docs, doc_len, term_ptr, post_doc, post_tf, vocab=None,
                       k1=K1, b=B, epsilon=EPSILON, total_docs=None, total_len=None, df=None):
@@ -372,15 +400,10 @@ class BM25Index:
     def append(self, token_lists: Sequence[Sequence[str]]) -> "BM25Index":
         """This index with the tokenised documents appended (ids n_docs, n_docs + 1, ...): equal,
         field by field and bit for bit, to ``from_token_lists(old documents + token_lists)``."""
-        if self.vocab is None:
-            raise ValueError("index has no string vocabulary")
-        app = csr_append(self.vocab, np.diff(self.term_ptr.astype(np.int64)), self.n_docs,
-                         int(self.doc_len.astype(np.int64).sum()), token_lists, self.epsilon)
+        app = csr_append(self.stats(), token_lists)
+        app.commit_vocab()
         term_ptr, postings = merge_csr(self.term_ptr, self.postings, app)
-        vocab = dict(self.vocab)
-        vocab.update((w, len(self.vocab) + i) for i, w in enumerate(app.new_words))
-        return BM25Index(app.n_docs, np.concatenate([self.doc_len, app.doc_len]), term_ptr, postings,
-                         app.idf, app.avgdl, vocab, self.k1, self.b, self.epsilon)
+        return BM25Index.from_stats(app.stats, term_ptr, postings, np.concatenate([self.doc_len, app.doc_len]))
 
     # ------------------------------------------------------------------ remove
     def remove(self, ids: Sequence[int], doc_tokens: Callable[[int], Sequence[str]]) -> "BM25Index":
@@ -388,16 +411,12 @@ class BM25Index:
         and bit for bit, to ``from_token_lists(remaining documents)``, vocabulary order included.
         ``doc_tokens(d)`` tokenises document d; only the removed documents and the new first
         documents of the terms that lose theirs are read (``csr_remove``)."""
-        if self.vocab is None:
-            raise ValueError("index has no string vocabulary")
         tp = self.term_ptr.astype(np.int64)
-        first = self.postings[np.minimum(tp[:-1], max(self.nnz - 1, 0)), 0].astype(np.int64)
         gather = lambda terms, counts: self.postings[_ranges(tp[terms], counts), 0]
-        rem = csr_remove(self.vocab, np.diff(tp), first, self.n_docs, int(self.doc_len.astype(np.int64).sum()),
-                         ids, doc_tokens, gather, self.epsilon)
+        rem = csr_remove(self.stats(), ids, doc_tokens, gather)
+        rem.commit_vocab()
         term_ptr, postings = remove_csr(self.term_ptr, self.postings, rem)
-        return BM25Index(rem.n_docs, np.delete(self.doc_len, rem.removed), term_ptr, postings, rem.idf, rem.avgdl,
-                         {w: i for i, w in enumerate(rem.words)}, self.k1, self.b, self.epsilon)
+        return BM25Index.from_stats(rem.stats, term_ptr, postings, np.delete(self.doc_len, rem.removed))
 
     # ------------------------------------------------------------------ query
     def term_ids(self, tokens: Sequence[str]) -> List[int]:

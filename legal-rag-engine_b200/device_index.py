@@ -19,6 +19,18 @@ def _ptr(t: Optional[torch.Tensor]):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
+def _to(a, dt: torch.dtype, device) -> torch.Tensor:
+    """A tensor, or a numpy array uploaded (unsigned integers as the signed type of their width),
+    on `device` as `dt`."""
+    if isinstance(a, np.ndarray):
+        if a.dtype == np.uint64:
+            a = a.view(np.int64)
+        elif a.dtype == np.uint32:
+            a = a.view(np.int32)
+        a = torch.from_numpy(np.ascontiguousarray(a))
+    return a.to(device, dtype=dt).contiguous()
+
+
 class DeviceIndex:
     def __init__(self, device: int = 0, rank: int = 0, world: int = 1):
         if not torch.cuda.is_available():
@@ -77,11 +89,12 @@ class DeviceIndex:
         if prefilter and self.n_local > 0:
             self.build_prefilter()
 
-    def append_rows(self, x_new: torch.Tensor):
+    def append_rows(self, x_new: torch.Tensor, prefilter: Optional[bool] = None):
         """Append fp16 rows (local ids n_local, n_local + 1, ...).  The matrix is the prefix of a
         capacity buffer; a buffer too small is replaced by one 1/16 larger than needed (the old rows
-        are copied on the device, the old buffer freed).  An index whose pre-filter is on gets its
-        int8 shadow rebuilt (its row scales sit after the padded rows, so it cannot grow in place)."""
+        are copied on the device, the old buffer freed) before the handle takes the new matrix.
+        `prefilter` (default: as before) rebuilds the int8 shadow (its row scales sit after the
+        padded rows, so it cannot grow in place)."""
         assert x_new.dtype == torch.float16 and x_new.is_cuda and x_new.dim() == 2
         assert x_new.shape[1] == LRX_DIM
         n, m = self.n_local, int(x_new.shape[0])
@@ -94,7 +107,8 @@ class DeviceIndex:
                 grown[:n].copy_(self.x)
             buf = grown
         buf[n:n + m].copy_(x_new)
-        prefilter = self._prefilter_on
+        if prefilter is None:
+            prefilter = self._prefilter_on
         self._q8 = None                                     # the shadow of the old matrix
         self.set_corpus(buf[:n + m], self.id_base, prefilter=prefilter)
         self._xbuf = buf
@@ -135,63 +149,52 @@ class DeviceIndex:
         int32/uint32 [nnz,2] = (local doc, tf); doc_len int32/uint32 [n]; idf float64 [V]
         (GLOBAL statistics) -- torch CUDA tensors or numpy arrays (uploaded).  The 8-byte
         scoring layout {doc, u16 tf, u16 len} is built on the device (index-build step)."""
-        def dev(a, dt):
-            if isinstance(a, np.ndarray):
-                if a.dtype == np.uint64:
-                    a = a.view(np.int64)
-                elif a.dtype == np.uint32:
-                    a = a.view(np.int32)
-                a = torch.from_numpy(np.ascontiguousarray(a))
-            return a.to(self.device, dtype=dt).contiguous()
-        tp = dev(term_ptr, torch.int64)
-        po = dev(postings, torch.int32)
-        dl = dev(doc_len, torch.int32)
-        idf_t = dev(idf, torch.float64)
+        tp = _to(term_ptr, torch.int64, self.device)
+        po = _to(postings, torch.int32, self.device)
+        dl = _to(doc_len, torch.int32, self.device)
+        idf_t = _to(idf, torch.float64, self.device)
         nnz = int(tp[-1].item())
         assert po.shape[0] == nnz, (po.shape, nnz)
-        self.n_docs = int(dl.numel())
-        if dl.numel() == 0:
-            dl = torch.zeros(1, dtype=torch.int32, device=self.device)
-        max_len = int(dl.max().item())
+        dl1 = dl if dl.numel() else torch.zeros(1, dtype=torch.int32, device=self.device)   # no documents: one 0
         p8 = torch.zeros((nnz + 2, 2), dtype=torch.int32, device=self.device)   # 8 B / posting, padded
-        self._ck(self.lib.lrx_bm25_build_postings(self.h, _ptr(po), nnz, _ptr(dl), _ptr(p8)))
+        self._ck(self.lib.lrx_bm25_build_postings(self.h, _ptr(po), nnz, _ptr(dl1), _ptr(p8)))
         del po
+        self._install(tp, p8, idf_t, dl, avgdl, k1, b, int(dl1.max().item()))
+
+    def _install(self, tp, p8, idf_t, doc_len, avgdl: float, k1: float, b: float, max_len: int):
+        """Hand the handle these postings (lrx_set_postings): the one place that does, and the one
+        writer of the fields that describe them.  Buffers it replaces are dropped only after the
+        handle has taken the new ones, so a failure leaves the index as it was."""
+        n_terms, nnz = int(tp.numel()) - 1, int(p8.shape[0]) - 2
+        self._ck(self.lib.lrx_set_postings(self.h, _ptr(tp), _ptr(p8), _ptr(idf_t), n_terms, nnz, float(avgdl),
+                                           float(k1), float(b), max_len))
         self._post = (tp, p8, idf_t)
         self._post_args = (nnz, float(avgdl), float(k1), float(b), max_len)
-        self.doc_len = dl
-        self.n_terms = int(tp.numel() - 1)
-        self._ck(self.lib.lrx_set_postings(self.h, _ptr(tp), _ptr(p8), _ptr(idf_t), self.n_terms, nnz,
-                                           float(avgdl), float(k1), float(b), max_len))
+        self.doc_len, self.n_terms, self.n_docs = doc_len, n_terms, int(doc_len.numel())
 
-    def append_postings(self, add_ptr, add_postings, add_doc_len, idf, avgdl: float):
-        """Append documents n_docs, n_docs + 1, ... to the resident postings: their own term-major
-        CSR (add_ptr int64 [V_out+1], add_postings uint32 [nnz_add, 2] = (local doc, tf)), their
-        lengths, and the whole corpus's new idf float64 [V_out] / avgdl.  The merge runs on the
-        device into new buffers (lrx_bm25_append_postings); the old ones are dropped only after
-        lrx_set_postings has taken the new ones, so a failure leaves the index as it was."""
+    def stage_append(self, add_ptr, add_postings, add_doc_len, idf, avgdl: float):
+        """Documents n_docs, n_docs + 1, ... merged on the device (lrx_bm25_append_postings) into new
+        buffers: a staged index for `commit_postings`; the handle is not changed.  Their own CSR (add_ptr
+        int64 [V_out+1], add_postings uint32 [nnz_add, 2] = (local doc, tf)), lengths, and the whole
+        corpus's new idf float64 [V_out] / avgdl."""
         tp, p8, _ = self._post
-        nnz, _, k1, b, max_len = self._post_args
-        up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a).view(dt)).to(self.device)
-        add_ptr = np.ascontiguousarray(add_ptr, dtype=np.int64)
-        add_len = np.ascontiguousarray(add_doc_len, dtype=np.uint32)
-        ap = up(add_ptr, np.int64)
-        ad = up(np.ascontiguousarray(add_postings, dtype=np.uint32).reshape(-1, 2), np.int32)
-        n_old, m = self.n_docs, len(add_len)
-        dl = torch.cat([self.doc_len[:n_old], up(add_len, np.int32)])
+        nnz, max_len = self._post_args[0], self._post_args[4]
+        add_len = np.asarray(add_doc_len, dtype=np.uint32)
+        ap = _to(add_ptr, torch.int64, self.device)
+        ad = _to(np.asarray(add_postings, dtype=np.uint32).reshape(-1, 2), torch.int32, self.device)
+        dl = torch.cat([self.doc_len[:self.n_docs], _to(add_len, torch.int32, self.device)])
         n_terms_out, nnz_add = len(add_ptr) - 1, int(add_ptr[-1])
         tp_out = torch.empty(n_terms_out + 1, dtype=torch.int64, device=self.device)
         p8_out = torch.empty((nnz + nnz_add + 2, 2), dtype=torch.int32, device=self.device)
         self._ck(self.lib.lrx_bm25_append_postings(
-            self.h, _ptr(tp), _ptr(p8), self.n_terms, nnz, n_old, _ptr(ap), _ptr(ad), n_terms_out, nnz_add,
-            _ptr(dl), n_old + m, _ptr(tp_out), _ptr(p8_out)))
-        idf_t = torch.from_numpy(np.ascontiguousarray(idf, dtype=np.float64)).to(self.device)
-        max_len = max(max_len, int(add_len.max()) if m else 0)
-        self._ck(self.lib.lrx_set_postings(self.h, _ptr(tp_out), _ptr(p8_out), _ptr(idf_t), n_terms_out,
-                                           nnz + nnz_add, float(avgdl), k1, b, max_len))
-        self._post = (tp_out, p8_out, idf_t)
-        self._post_args = (nnz + nnz_add, float(avgdl), k1, b, max_len)
-        self.doc_len = dl if dl.numel() else self.doc_len
-        self.n_terms, self.n_docs = n_terms_out, n_old + m
+            self.h, _ptr(tp), _ptr(p8), self.n_terms, nnz, self.n_docs, _ptr(ap), _ptr(ad), n_terms_out, nnz_add,
+            _ptr(dl), int(dl.numel()), _ptr(tp_out), _ptr(p8_out)))
+        max_len = max(max_len, int(add_len.max()) if len(add_len) else 0)
+        return tp_out, p8_out, _to(idf, torch.float64, self.device), dl, float(avgdl), max_len
+
+    def append_postings(self, add_ptr, add_postings, add_doc_len, idf, avgdl: float):
+        """stage_append + commit_postings: a failure leaves the index as it was."""
+        self.commit_postings(self.stage_append(add_ptr, add_postings, add_doc_len, idf, avgdl))
 
     def remove_rows(self, keep, prefilter: Optional[bool] = None, chunk: int = 1 << 20):
         """Keep only the rows `keep` (ascending local ids, or a bool mask over n_local), moved to the
@@ -230,39 +233,41 @@ class DeviceIndex:
         not describe the postings raises LrxError (LRX_E_ARG)."""
         tp, p8, _ = self._post
         nnz = self._post_args[0]
-        up = lambda a, dt, v: torch.from_numpy(np.ascontiguousarray(a, dtype=dt).view(v)).to(self.device)
-        removed = up(rem.removed, np.uint32, np.int32)
-        rem_ptr = up(rem.rem_ptr, np.int64, np.int64)
-        rem_doc = up(rem.rem_doc, np.uint32, np.int32)
-        term_map = up(rem.term_map, np.int32, np.int32)
-        tp_out = up(rem.term_ptr, np.int64, np.int64)
-        n_terms_out, nnz_out = rem.n_terms, rem.nnz
-        p8_out = torch.empty((nnz_out + 2, 2), dtype=torch.int32, device=self.device)
+        removed = _to(np.asarray(rem.removed).astype(np.uint32), torch.int32, self.device)
+        rem_ptr = _to(np.asarray(rem.rem_ptr, dtype=np.int64), torch.int64, self.device)
+        rem_doc = _to(np.asarray(rem.rem_doc, dtype=np.uint32), torch.int32, self.device)
+        term_map = _to(np.asarray(rem.term_map, dtype=np.int32), torch.int32, self.device)
+        tp_out = _to(np.asarray(rem.term_ptr, dtype=np.int64), torch.int64, self.device)
+        p8_out = torch.empty((rem.nnz + 2, 2), dtype=torch.int32, device=self.device)
         self._ck(self.lib.lrx_bm25_remove_postings(
             self.h, _ptr(tp), _ptr(p8), self.n_terms, nnz, self.n_docs, _ptr(removed), len(rem.removed),
-            _ptr(rem_ptr), _ptr(rem_doc), _ptr(term_map), _ptr(tp_out), n_terms_out, _ptr(p8_out)))
+            _ptr(rem_ptr), _ptr(rem_doc), _ptr(term_map), _ptr(tp_out), rem.n_terms, _ptr(p8_out)))
         keep = torch.ones(self.n_docs, dtype=torch.bool, device=self.device)
         keep[removed.to(torch.int64)] = False
         dl = self.doc_len[:self.n_docs][keep]
-        idf_t = torch.from_numpy(np.ascontiguousarray(rem.idf, dtype=np.float64)).to(self.device)
-        return tp_out, p8_out, idf_t, dl, float(rem.avgdl), int(dl.max().item())
+        idf_t = _to(rem.stats.idf, torch.float64, self.device)
+        return tp_out, p8_out, idf_t, dl, float(rem.stats.avgdl), int(dl.max().item())
 
     def commit_postings(self, staged):
-        """Make a staged index of `compact_postings` resident (lrx_set_postings); the old buffers are
-        dropped after the handle has taken the new ones."""
+        """Make a staged index of `stage_append` or `compact_postings` resident."""
         tp_out, p8_out, idf_t, dl, avgdl, max_len = staged
         _, _, k1, b, _ = self._post_args
-        n_terms_out, nnz_out = int(tp_out.numel() - 1), int(p8_out.shape[0] - 2)
-        self._ck(self.lib.lrx_set_postings(self.h, _ptr(tp_out), _ptr(p8_out), _ptr(idf_t), n_terms_out, nnz_out,
-                                           avgdl, k1, b, max_len))
-        self._post = (tp_out, p8_out, idf_t)
-        self._post_args = (nnz_out, avgdl, k1, b, max_len)
-        self.doc_len = dl
-        self.n_terms, self.n_docs = n_terms_out, int(dl.numel())
+        self._install(tp_out, p8_out, idf_t, dl, avgdl, k1, b, max_len)
 
     def remove_postings(self, rem):
         """compact_postings + commit_postings: a failure leaves the index as it was."""
         self.commit_postings(self.compact_postings(rem))
+
+    def read_postings(self):
+        """The resident postings on the host as an index build holds them: (term_ptr uint64 [V+1],
+        postings uint32 [nnz, 2] = (doc, tf), doc_len uint32 [n_docs]).  The 8-byte entries
+        {u32 doc, u16 tf, u16 len} are copied as they are and the tf split off on the host, so the
+        device needs no temporary the size of the postings."""
+        tp, p8, _ = self._post
+        postings = p8[:self._post_args[0]].cpu().numpy().view(np.uint32)
+        postings[:, 1] &= 0xFFFF
+        return (tp.cpu().numpy().view(np.uint64), postings,
+                self.doc_len[:self.n_docs].cpu().numpy().view(np.uint32))
 
     def clone_view(self) -> "DeviceIndex":
         """A second handle (own stream binding, workspaces, exchange region) over the SAME resident
@@ -275,12 +280,7 @@ class DeviceIndex:
                 other._q8 = self._q8
                 other.set_prefilter(True)
         if self._post is not None:
-            tp, p8, idf_t = self._post
-            nnz, avgdl, k1, b, max_len = self._post_args
-            other._post, other._post_args = self._post, self._post_args
-            other.doc_len, other.n_terms = self.doc_len, self.n_terms
-            other._ck(self.lib.lrx_set_postings(other.h, _ptr(tp), _ptr(p8), _ptr(idf_t), self.n_terms,
-                                                nnz, avgdl, k1, b, max_len))
+            other._install(*self._post, self.doc_len, *self._post_args[1:])
         return other
 
     def _cap(self, q_terms: Optional[torch.Tensor], B: int):

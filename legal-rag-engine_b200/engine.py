@@ -28,7 +28,7 @@ import torch
 
 from . import store as _store
 from ._lib import LRX_MAX_BATCH, LRX_MAX_DEPTH
-from .bm25_index import BM25Index, BM25Append, compact_csr, csr_append, csr_remove, merge_csr, tokenize
+from .bm25_index import BM25Index, csr_append, csr_remove, tokenize
 from .device_index import FUSION, DeviceIndex
 from .encoder import SentenceEncoder
 from .sharding import shard_range
@@ -98,13 +98,9 @@ class RetrievalEngine:
         self.chunks, xh, bm25 = _store.load_store(self.store_dir, mmap=self.world > 1)
         self.n_total = len(self.chunks)
         self.lo, self.hi = shard_range(self.n_total, self.rank, self.world)
-        self._lock = threading.Lock()                      # searches see the index before or after a change
-        self._bm25 = bm25                                  # whole-corpus statistics + vocabulary
-        self._bm25_pending = []                            # appends / removals not yet applied to _bm25's postings
-        tp = bm25.term_ptr.astype(np.int64)
-        self._df = np.diff(tp)
-        self._total_len = int(bm25.doc_len.astype(np.int64).sum())
-        self._first = bm25.postings[np.minimum(tp[:-1], max(bm25.nnz - 1, 0)), 0].astype(np.int64)
+        self._lock = threading.RLock()                     # searches see the index before or after a change
+        self._stats = bm25.stats()                         # whole-corpus statistics + vocabulary (postings: on the GPU)
+        self._sharded_bm25 = bm25 if self.world > 1 else None   # a shard's device holds only its own rows
         local = bm25 if self.world == 1 else bm25.shard(self.lo, self.hi)
         self._x = torch.from_numpy(np.ascontiguousarray(xh[self.lo:self.hi])).to(self.dev.device)
         self.dev.set_corpus(self._x, self.lo)
@@ -195,7 +191,7 @@ class RetrievalEngine:
         # BM25 side: query.lower().split() -> term ids (retrieval_engine.py:67).  EVERY token is
         # scored, in order, repeats included, as rank_bm25 does; out-of-vocabulary tokens are
         # dropped here because `idf.get(q) or 0` makes them add exactly 0.0.
-        term_lists = [[t for t in self._bm25.term_ids(tokenize(q)) if t >= 0] for q in queries]
+        term_lists = [[self._stats.vocab[w] for w in tokenize(q) if w in self._stats.vocab] for q in queries]
         o_ids, o_score, o_sem, o_kw = self.dev.search_text_host(ids, lens, term_lists, k, weights, mode)
         results = []
         for b in range(B):
@@ -212,24 +208,13 @@ class RetrievalEngine:
     # ------------------------------------------------------------------ growth
     @property
     def bm25(self) -> BM25Index:
-        """The BM25 index of the whole current corpus (host postings of added chunks are merged in
-        when this is read)."""
+        """The BM25 index of the whole current corpus, a snapshot that later adds and removals leave as
+        it is: on one GPU, the host statistics with the postings read back from the device; on a
+        sharded engine (which cannot change), the index it loaded."""
+        if self.world > 1:
+            return self._sharded_bm25
         with self._lock:
-            return self._bm25_current()
-
-    def _bm25_current(self) -> BM25Index:
-        b = self._bm25
-        for op in self._bm25_pending:                      # in the order they were made
-            if isinstance(op, BM25Append):
-                b.term_ptr, b.postings = merge_csr(b.term_ptr, b.postings, op)
-                b.doc_len = np.concatenate([b.doc_len, op.doc_len])
-            else:
-                _, n_old, removed, term_map, term_ptr_out = op
-                b.term_ptr, b.postings = compact_csr(b.term_ptr, b.postings, n_old, removed, term_map,
-                                                     term_ptr_out)
-                b.doc_len = np.delete(b.doc_len, removed)
-        self._bm25_pending = []
-        return b
+            return BM25Index.from_stats(self._stats, *self.dev.read_postings())
 
     def add_chunks(self, chunks: Sequence[dict]) -> range:
         """Append chunks to the loaded index; returns their ids (positions in ``self.chunks``).
@@ -255,19 +240,19 @@ class RetrievalEngine:
             if not chunks:
                 return range(n, n)
             x16 = self.model.encode([c["text"] for c in chunks]).astype(np.float16)
-            b = self._bm25
-            app = csr_append(b.vocab, self._df, b.n_docs, self._total_len, tokens, b.epsilon)
-            self.dev.append_postings(app.term_ptr, app.postings, app.doc_len, app.idf, app.avgdl)
-            self.dev.append_rows(torch.from_numpy(x16).to(self.dev.device))
-            base = len(b.vocab)
-            b.vocab.update((w, base + i) for i, w in enumerate(app.new_words))
-            b.n_docs, b.idf, b.avgdl = app.n_docs, app.idf, app.avgdl
-            self._bm25_pending.append(app)
-            self._df, self._total_len = app.df, app.total_len
-            self._first = np.concatenate([self._first, app.postings[app.term_ptr[base:-1], 0].astype(np.int64)])
+            app = csr_append(self._stats, tokens)
+            # the steps in the order remove_chunks gives them, for the same reason
+            staged = self.dev.stage_append(app.term_ptr, app.postings, app.doc_len, app.stats.idf, app.stats.avgdl)
+            prefilter = self.dev._prefilter_on
+            self.dev.append_rows(torch.from_numpy(x16).to(self.dev.device), prefilter=False)
+            self.dev.commit_postings(staged)
+            app.commit_vocab()
+            self._stats = app.stats
             self.chunks.extend(chunks)
             self.n_total = self.hi = len(self.chunks)
             self._x = self.dev.x
+            if prefilter:
+                self.dev.build_prefilter()
             return range(n, self.n_total)
 
     def remove_chunks(self, ids: Sequence[int]) -> np.ndarray:
@@ -296,9 +281,7 @@ class RetrievalEngine:
             ids_map = np.arange(n, dtype=np.int64)
             if not len(ids_arr):
                 return ids_map
-            b = self._bm25
-            rem = csr_remove(b.vocab, self._df, self._first, b.n_docs, self._total_len, ids_arr,
-                             lambda d: tokenize(self.chunks[d]["text"]), self.dev.posting_docs, b.epsilon)
+            rem = csr_remove(self._stats, ids_arr, lambda d: tokenize(self.chunks[d]["text"]), self.dev.posting_docs)
             keep = np.ones(n, dtype=bool)
             keep[rem.removed] = False
             # every step that allocates or checks runs before the handle takes the new postings: the
@@ -308,11 +291,8 @@ class RetrievalEngine:
             prefilter = self.dev._prefilter_on
             self.dev.remove_rows(keep, prefilter=False)
             self.dev.commit_postings(staged)
-            del staged
-            b.vocab = {w: i for i, w in enumerate(rem.words)}
-            b.n_docs, b.idf, b.avgdl = rem.n_docs, rem.idf, rem.avgdl
-            self._bm25_pending.append(("remove", n, rem.removed, rem.term_map, rem.term_ptr))
-            self._df, self._total_len, self._first = rem.df, rem.total_len, rem.first_doc
+            rem.commit_vocab()
+            self._stats = rem.stats
             self.chunks = [c for c, k in zip(self.chunks, keep.tolist()) if k]
             self.n_total = self.hi = len(self.chunks)
             self._x = self.dev.x
@@ -331,13 +311,13 @@ class RetrievalEngine:
             raise NotImplementedError("save on a sharded engine: each rank holds only its rows")
         target = Path(store_dir) if store_dir is not None else self.store_dir
         target.parent.mkdir(parents=True, exist_ok=True)
-        with self._lock:
+        with self._lock:                                  # re-entrant: self.bm25 below takes it too
             tmp = Path(tempfile.mkdtemp(prefix=f".{target.name}.", dir=target.parent))
             os.chmod(tmp, 0o755)                          # mkdtemp's 0700 would follow the store
             old = None
             try:
                 x = self._x.cpu().numpy().astype(np.float32)
-                _store.save_store(tmp, self.chunks, x, self._bm25_current())
+                _store.save_store(tmp, self.chunks, x, self.bm25)
                 if target.exists():
                     old = Path(tempfile.mkdtemp(prefix=f".{target.name}.old.", dir=target.parent))
                     os.rename(target, old / target.name)

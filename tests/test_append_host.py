@@ -19,6 +19,20 @@ def _same(a: BM25Index, b: BM25Index):
     assert a.avgdl == b.avgdl and (a.k1, a.b, a.epsilon) == (b.k1, b.b, b.epsilon)
 
 
+def _stats_copy(s):
+    return list(s.vocab.items()), s.df.copy(), s.first_doc.copy(), s.idf.view(np.uint64).copy()
+
+
+def _assert_stats_unchanged(s, kept):
+    """A plan leaves the statistics it was given as they were: vocabulary items and order, df,
+    first_doc, idf bits."""
+    items, df, first, idf = kept
+    assert list(s.vocab.items()) == items
+    np.testing.assert_array_equal(s.df, df)
+    np.testing.assert_array_equal(s.first_doc, first)
+    np.testing.assert_array_equal(s.idf.view(np.uint64), idf)
+
+
 @pytest.fixture(scope="module")
 def docs(legal_texts):
     return [tokenize(t) for t in legal_texts]
@@ -46,14 +60,17 @@ def test_append_of_new_terms_only_empty_document_and_nothing():
 
 def test_csr_append_is_the_appended_documents_alone(docs):
     old = BM25Index.from_token_lists(docs[:2000])
-    app = csr_append(old.vocab, np.diff(old.term_ptr.astype(np.int64)), old.n_docs,
-                     int(old.doc_len.sum()), docs[2000:2100])
+    stats = old.stats()
+    kept = _stats_copy(stats)
+    app = csr_append(stats, docs[2000:2100])
+    _assert_stats_unchanged(stats, kept)
     full = BM25Index.from_token_lists(docs[:2100])
-    assert app.n_terms == full.n_terms and app.n_docs == 2100 and app.nnz == len(app.postings)
+    assert app.n_terms == full.n_terms and app.stats.n_docs == 2100 and app.nnz == len(app.postings)
     assert app.new_words == list(full.vocab)[old.n_terms:]
-    np.testing.assert_array_equal(app.df, np.diff(full.term_ptr.astype(np.int64)))
-    np.testing.assert_array_equal(app.idf.view(np.uint64), full.idf.view(np.uint64))
-    assert app.avgdl == full.avgdl and app.total_len == int(full.doc_len.sum())
+    np.testing.assert_array_equal(app.stats.df, np.diff(full.term_ptr.astype(np.int64)))
+    np.testing.assert_array_equal(app.stats.first_doc, full.postings[full.term_ptr[:-1].astype(np.int64), 0])
+    np.testing.assert_array_equal(app.stats.idf.view(np.uint64), full.idf.view(np.uint64))
+    assert app.stats.avgdl == full.avgdl and app.stats.total_len == int(full.doc_len.sum())
     # its own CSR = the rebuild's postings of documents >= 2000
     keep = full.postings[:, 0] >= 2000
     np.testing.assert_array_equal(app.postings, full.postings[keep])
@@ -62,6 +79,8 @@ def test_csr_append_is_the_appended_documents_alone(docs):
     tp, po = merge_csr(old.term_ptr, old.postings, app)
     np.testing.assert_array_equal(tp, full.term_ptr)
     np.testing.assert_array_equal(po, full.postings)
+    app.commit_vocab()
+    assert stats.vocab is app.stats.vocab and list(stats.vocab.items()) == list(full.vocab.items())
 
 
 def test_add_chunks_on_a_sharded_engine_raises_before_touching_anything():

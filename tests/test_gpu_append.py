@@ -196,6 +196,58 @@ def test_added_chunk_is_found_after_captured_chains(env, legal_chunks):
         eng.close()
 
 
+def _same_index(a, b):
+    assert a.n_docs == b.n_docs
+    assert list(a.vocab.items()) == list(b.vocab.items())            # ids AND insertion order
+    for name in ("term_ptr", "postings", "doc_len"):
+        x, y = getattr(a, name), getattr(b, name)
+        assert x.dtype == y.dtype and x.shape == y.shape, name
+        np.testing.assert_array_equal(x, y, err_msg=name)
+    np.testing.assert_array_equal(a.idf.view(np.uint64), b.idf.view(np.uint64))
+    assert a.avgdl == b.avgdl and (a.k1, a.b, a.epsilon) == (b.k1, b.b, b.epsilon)
+
+
+def test_failed_add_changes_nothing(env, reference_queries, monkeypatch):
+    """A failure after the postings are staged -- here the matrix append raising -- leaves the engine
+    as it was.  The state is checked before any search, so no search runs over a handle whose
+    postings and matrix could disagree."""
+    eng = _engine(env)
+    try:
+        before = _answers(eng, reference_queries)
+        b = eng.bm25
+        post, n_docs, n_local, n = eng.dev._post, eng.dev.n_docs, eng.dev.n_local, eng.n_total
+
+        def fail(*args, **kwargs):
+            raise RuntimeError("injected failure of the matrix append")
+        monkeypatch.setattr(eng.dev, "append_rows", fail)
+        with pytest.raises(RuntimeError, match="injected"):
+            eng.add_chunks([{"text": "quokka tribunal zebra amendment ordinance"}])
+        monkeypatch.undo()
+        assert eng.dev._post is post and eng.dev.n_docs == n_docs and eng.dev.n_local == n_local
+        assert eng.n_total == n and len(eng.chunks) == n
+        _same_index(eng.bm25, b)
+        assert _answers(eng, reference_queries) == before
+    finally:
+        eng.close()
+
+
+def test_bm25_is_a_snapshot(env, legal_chunks):
+    """engine.bm25 taken before an add and a removal still describes the index it was taken from;
+    read again, it equals a rebuild."""
+    import copy
+    from legal_rag_engine_b200.bm25_index import BM25Index
+    eng = _engine(env)
+    try:
+        b = eng.bm25
+        kept = copy.deepcopy(b)
+        eng.add_chunks(legal_chunks[2000:2010])
+        eng.remove_chunks([0, 5, 2003])
+        _same_index(b, kept)
+        _same_index(eng.bm25, BM25Index.from_texts([c["text"] for c in eng.chunks]))
+    finally:
+        eng.close()
+
+
 def test_rejected_input_changes_nothing(env, reference_queries):
     eng = _engine(env)
     try:

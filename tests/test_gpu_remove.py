@@ -266,7 +266,7 @@ def _synthetic(n, seed, planted_block, planted_terms=6):
 def _plan(idx, removed, rng):
     """A removal plan over an index without a string vocabulary, surviving terms numbered by a
     random permutation (the kernel takes any bijection)."""
-    from legal_rag_engine_b200.bm25_index import BM25Remove, okapi_idf
+    from legal_rag_engine_b200.bm25_index import BM25Remove, BM25Stats, okapi_idf
     tp = idx.term_ptr.astype(np.int64)
     V = idx.n_terms
     doc = idx.postings[:, 0].astype(np.int64)
@@ -288,7 +288,7 @@ def _plan(idx, removed, rng):
     total = int(doc_len.astype(np.int64).sum())
     idf, _ = okapi_idf(df_out, n_out)
     return BM25Remove(np.asarray(removed, dtype=np.int64), rem_ptr, doc[gone].astype(np.uint32), term_map, term_ptr,
-                      [], np.zeros(0, np.int64), df_out, n_out, total, idf, total / n_out), doc_len
+                      BM25Stats({}, df_out, np.zeros(0, np.int64), n_out, total, idf, total / n_out)), doc_len
 
 
 def test_one_million_rows_remove(tmp_path):
@@ -330,7 +330,7 @@ def test_one_million_rows_remove(tmp_path):
             dev.remove_rows(keep)
             x = x[keep]
             tp, po = remove_csr(idx.term_ptr, idx.postings, rem)
-            idx = BM25Index(rem.n_docs, doc_len, tp, po, rem.idf, rem.avgdl)
+            idx = BM25Index(rem.stats.n_docs, doc_len, tp, po, rem.stats.idf, rem.stats.avgdl)
             lists = [[int(rem.term_map[t]) for t in l if rem.term_map[t] >= 0] for l in lists]
             assert dev.n_local == n - len(removed) == idx.n_docs
             csr = obm25.BM25OkapiCSR.from_postings(idx.n_docs, idx.doc_len, tp.astype(np.int64), po[:, 0], po[:, 1])
@@ -348,7 +348,7 @@ def test_one_million_rows_remove(tmp_path):
             try:
                 fresh.set_corpus(torch.from_numpy(x).cuda(), 0, prefilter=True)
                 assert dev.prefilter_bounds == fresh.prefilter_bounds
-                fresh.set_postings(tp, po, doc_len, rem.idf, rem.avgdl)
+                fresh.set_postings(tp, po, doc_len, rem.stats.idf, rem.stats.avgdl)
                 nnz = rem.nnz
                 assert dev._post_args == fresh._post_args
                 assert torch.equal(dev._post[0], fresh._post[0])
@@ -379,8 +379,7 @@ def test_inconsistent_plan_is_refused_and_the_index_keeps_answering(legal_texts)
     lists = [[t for t in l if t >= 0] for l in lists]
 
     def plan():
-        return csr_remove(full.vocab, np.diff(tp), full.postings[tp[:-1], 0], full.n_docs, int(full.doc_len.sum()),
-                          [0, 5, 17, 900], docs.__getitem__, lambda t, c: full.postings[_ranges(tp[t], c), 0])
+        return csr_remove(full.stats(), [0, 5, 17, 900], docs.__getitem__, lambda t, c: full.postings[_ranges(tp[t], c), 0])
 
     def unsorted_list(p):
         t = int(np.nonzero(np.diff(p.rem_ptr) >= 2)[0][0])
@@ -408,7 +407,7 @@ def test_inconsistent_plan_is_refused_and_the_index_keeps_answering(legal_texts)
 
     def term_map_swapped(p):                             # a bijection whose ranges have the wrong lengths
         live = np.nonzero(p.term_map >= 0)[0]
-        a, b = live[0], next(t for t in live if p.df[p.term_map[t]] != p.df[p.term_map[live[0]]])
+        a, b = live[0], next(t for t in live if p.stats.df[p.term_map[t]] != p.stats.df[p.term_map[live[0]]])
         p.term_map[a], p.term_map[b] = p.term_map[b], p.term_map[a]
 
     def removed_unsorted(p):

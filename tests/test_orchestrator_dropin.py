@@ -80,6 +80,11 @@ class OracleDevice:
                                                     postings[:, 0], postings[:, 1])
         np.testing.assert_array_equal(self.csr.idf, idf)
         assert self.csr.avgdl == avgdl
+        self.postings = (np.asarray(term_ptr, dtype=np.uint64), np.asarray(postings, dtype=np.uint32),
+                         np.asarray(doc_len, dtype=np.uint32))
+
+    def read_postings(self):
+        return self.postings
 
     def search_text_host(self, tok_ids, tok_lens, term_lists, k, weights, fusion):
         from oracle import encoder as oenc

@@ -19,6 +19,20 @@ def _same(a: BM25Index, b: BM25Index):
     assert a.avgdl == b.avgdl and (a.k1, a.b, a.epsilon) == (b.k1, b.b, b.epsilon)
 
 
+def _stats_copy(s):
+    return list(s.vocab.items()), s.df.copy(), s.first_doc.copy(), s.idf.view(np.uint64).copy()
+
+
+def _assert_stats_unchanged(s, kept):
+    """A plan leaves the statistics it was given as they were: vocabulary items and order, df,
+    first_doc, idf bits."""
+    items, df, first, idf = kept
+    assert list(s.vocab.items()) == items
+    np.testing.assert_array_equal(s.df, df)
+    np.testing.assert_array_equal(s.first_doc, first)
+    np.testing.assert_array_equal(s.idf.view(np.uint64), idf)
+
+
 @pytest.fixture(scope="module")
 def docs(legal_texts):
     return [tokenize(t) for t in legal_texts]
@@ -76,14 +90,18 @@ def test_csr_remove_plan_and_host_compaction(docs):
     full = BM25Index.from_token_lists(docs)
     removed = list(range(50))
     tp = full.term_ptr.astype(np.int64)
-    rem = csr_remove(full.vocab, np.diff(tp), full.postings[tp[:-1], 0], full.n_docs, int(full.doc_len.sum()),
-                     removed, docs.__getitem__, lambda t, c: full.postings[_ranges(tp[t], c), 0])
+    stats = full.stats()
+    kept = _stats_copy(stats)
+    rem = csr_remove(stats, removed, docs.__getitem__, lambda t, c: full.postings[_ranges(tp[t], c), 0])
+    _assert_stats_unchanged(stats, kept)
     want = BM25Index.from_token_lists(docs[50:])
-    assert rem.words == list(want.vocab) and rem.n_docs == want.n_docs and rem.avgdl == want.avgdl
+    s = rem.stats
+    assert s.n_docs == want.n_docs and s.avgdl == want.avgdl
+    assert s.total_len == int(want.doc_len.sum())
     np.testing.assert_array_equal(rem.term_ptr, want.term_ptr.astype(np.int64))
-    np.testing.assert_array_equal(rem.df, np.diff(want.term_ptr.astype(np.int64)))
-    np.testing.assert_array_equal(rem.first_doc, want.postings[want.term_ptr[:-1].astype(np.int64), 0])
-    np.testing.assert_array_equal(rem.idf.view(np.uint64), want.idf.view(np.uint64))
+    np.testing.assert_array_equal(s.df, np.diff(want.term_ptr.astype(np.int64)))
+    np.testing.assert_array_equal(s.first_doc, want.postings[want.term_ptr[:-1].astype(np.int64), 0])
+    np.testing.assert_array_equal(s.idf.view(np.uint64), want.idf.view(np.uint64))
     # per-term removed lists: exactly the postings of the removed documents, ascending
     term_of = np.repeat(np.arange(full.n_terms), np.diff(tp))
     hit = full.postings[:, 0] < 50
@@ -93,6 +111,8 @@ def test_csr_remove_plan_and_host_compaction(docs):
     tp_out, po = remove_csr(full.term_ptr, full.postings, rem)
     np.testing.assert_array_equal(tp_out, want.term_ptr)
     np.testing.assert_array_equal(po, want.postings)
+    rem.commit_vocab()
+    assert s.vocab is stats.vocab and list(s.vocab.items()) == list(want.vocab.items())
 
 
 def test_old_id_order_would_change_the_floored_idf_bits(docs):

@@ -134,11 +134,10 @@ for i, m in enumerate(int(s) for s in a.adds.split(",")):
     # search on the grown index vs an index built from scratch over the same rows and postings
     row["qps_grown"], got = qps(dev, q, lists, iters=a.search_iters)
     ref = DeviceIndex(0)
-    nnz_all = dev._post_args[0]
-    pairs = torch.stack([p8[:nnz_all, 0], p8[:nnz_all, 1] & 0xFFFF], dim=1).contiguous()
+    tp_h, pairs, dl_h = dev.read_postings()
     ref.set_corpus(dev.x.clone(), 0, prefilter=True)
-    ref.set_postings(tp, pairs, dev.doc_len, idf, avgdl)
-    del pairs
+    ref.set_postings(tp_h, pairs, dl_h, idf, avgdl)
+    del tp_h, pairs, dl_h
     row["qps_scratch"], want = qps(ref, q, lists, iters=a.search_iters)
     row["qps_grown_again"], _ = qps(dev, q, lists, iters=a.search_iters)
     row["results_equal"] = all(np.array_equal(u, v) for u, v in zip(got, want))
@@ -159,10 +158,8 @@ texts = [" ".join(t) for t in np.split(toks, np.cumsum(lens)[:-1])]
 t = time.perf_counter()
 BM25Index.from_texts(texts)
 host_s = time.perf_counter() - t
-tp, p8, idf_t = dev._post
-nnz_all = dev._post_args[0]
-pairs = torch.stack([p8[:nnz_all, 0], p8[:nnz_all, 1] & 0xFFFF], dim=1).contiguous().cpu().numpy()
-tp_h, dl_h, idf_h = tp.cpu().numpy(), dev.doc_len.cpu().numpy(), idf_t.cpu().numpy()
+tp_h, pairs, dl_h = dev.read_postings()
+idf_h = dev._post[2].cpu().numpy()
 up = DeviceIndex(0)
 torch.cuda.synchronize()
 t = time.perf_counter()

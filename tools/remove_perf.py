@@ -23,8 +23,8 @@ import torch
 ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
 from legal_rag_engine_b200 import synth                                  # noqa: E402
-from legal_rag_engine_b200.bm25_index import (BM25Index, BM25Remove, _ranges, csr_remove,  # noqa: E402
-                                              okapi_idf, tokenize)
+from legal_rag_engine_b200.bm25_index import (BM25Index, BM25Remove, BM25Stats, _ranges,  # noqa: E402
+                                              csr_remove, okapi_idf, tokenize)
 from legal_rag_engine_b200.device_index import DeviceIndex, _ptr        # noqa: E402
 
 ap = argparse.ArgumentParser()
@@ -93,8 +93,8 @@ def device_plan(dev, removed, df, total_len):
     n_out = dev.n_docs - len(rem_h)
     len_out = total_len - int(dev.doc_len[removed].to(torch.int64).sum().item())
     idf, _ = okapi_idf(df_out, n_out)
-    return BM25Remove(rem_h, rem_ptr, rem_doc, term_map, term_ptr, [], np.zeros(0, np.int64), df_out, n_out,
-                      len_out, idf, len_out / n_out), df_out
+    return BM25Remove(rem_h, rem_ptr, rem_doc, term_map, term_ptr,
+                      BM25Stats({}, df_out, np.zeros(0, np.int64), n_out, len_out, idf, len_out / n_out)), df_out
 
 
 dev = DeviceIndex(0)
@@ -172,17 +172,16 @@ for spec in a.removals.split(","):
     keep[removed] = False
     row["matrix_compaction_ms"], _ = timed(lambda: dev.remove_rows(keep, prefilter=False))   # the shadow: next
     row["shadow_rebuild_ms"], _ = timed(dev.build_prefilter)
-    df, total_len = df_new, rem.total_len
+    df, total_len = df_new, rem.stats.total_len
     term_map_all = np.where(term_map_all >= 0, rem.term_map[np.maximum(term_map_all, 0)], -1)
     lists = [[int(term_map_all[t]) for t in l if term_map_all[t] >= 0] for l in lists0]
     # search on the shrunk index vs an index built from scratch over the same rows and postings
     row["qps_after_removal"], got = qps(dev, q, lists, iters=a.search_iters)
     ref = DeviceIndex(0)
-    nnz_all = dev._post_args[0]
-    pairs = torch.stack([p8[:nnz_all, 0], p8[:nnz_all, 1] & 0xFFFF], dim=1).contiguous()
+    tp_h, pairs, dl_h = dev.read_postings()
     ref.set_corpus(dev.x.clone(), 0, prefilter=True)
-    ref.set_postings(tp, pairs, dev.doc_len, rem.idf, rem.avgdl)
-    del pairs
+    ref.set_postings(tp_h, pairs, dl_h, rem.stats.idf, rem.stats.avgdl)
+    del tp_h, pairs, dl_h
     row["qps_scratch"], want = qps(ref, q, lists, iters=a.search_iters)
     row["qps_after_removal_again"], _ = qps(dev, q, lists, iters=a.search_iters)
     row["results_equal"] = all(np.array_equal(u, v) for u, v in zip(got, want))
@@ -198,19 +197,20 @@ dev.close()
 def host_plan(docs, removed, label):
     full = BM25Index.from_token_lists(docs)
     tp = full.term_ptr.astype(np.int64)
-    first = full.postings[tp[:-1], 0].astype(np.int64)
+    stats = full.stats()
     calls = []
     tok = lambda d: calls.append(d) or docs[d]
     gather = lambda t, c: full.postings[_ranges(tp[t], c), 0]
     t = time.perf_counter()
-    rem = csr_remove(full.vocab, np.diff(tp), first, full.n_docs, int(full.doc_len.astype(np.int64).sum()),
-                     removed, tok, gather)
+    rem = csr_remove(stats, removed, tok, gather)
     plan_s = time.perf_counter() - t
     gone = set(removed)
     t = time.perf_counter()
     want = BM25Index.from_token_lists([d for i, d in enumerate(docs) if i not in gone])
     rebuild_s = time.perf_counter() - t
-    assert rem.words == list(want.vocab) and np.array_equal(rem.idf.view(np.uint64), want.idf.view(np.uint64))
+    rem.commit_vocab()
+    assert list(rem.stats.vocab) == list(want.vocab)
+    assert np.array_equal(rem.stats.idf.view(np.uint64), want.idf.view(np.uint64))
     return {"corpus": label, "docs": len(docs), "removed": len(removed), "plan_s": plan_s,
             "documents_read": len(calls), "host_rebuild_s": rebuild_s}
 
