@@ -21,8 +21,7 @@
  *    GPU or a non-sm_100 device is LRX_E_DEVICE at lrx_open.
  *  - ids are GLOBAL chunk ids (int64) = id_base + local row; -1 pads short lists.
  *  - all kernels run on the stream set with lrx_set_stream (default: the legacy
- *    default stream), so PyTorch code can order them with its own work and with
- *    the NCCL all-gather between lrx_search_local and lrx_search_finish.
+ *    default stream), so PyTorch code can order them with its own work.
  */
 #ifndef LRX_H
 #define LRX_H
@@ -63,14 +62,6 @@ typedef struct lrx_config {
     int32_t rank;          /* shard index of this handle (0 when unsharded) */
     int32_t world;         /* number of shards (1 when unsharded) */
 } lrx_config;
-
-/* One candidate of one sub-query on one shard; the unit the all-gather moves
- * (SURVEY.md section 8e).  24 bytes. */
-typedef struct lrx_record {
-    int64_t id;            /* global chunk id, -1 = empty slot */
-    double dense;          /* exact inner product (see oracle/flat_ip.py)   */
-    double bm25;           /* exact BM25Okapi score of that chunk            */
-} lrx_record;
 
 /* ---- lifetime ---------------------------------------------------------- */
 int lrx_open(const lrx_config* cfg, lrx_handle** out);
@@ -219,9 +210,9 @@ int lrx_dense_topk_batched(lrx_handle* h, const void* dev_q_fp16, int32_t B, int
 int lrx_dense_at(lrx_handle* h, const void* dev_q_fp16, int32_t B, const int64_t* dev_ids,
                  int32_t n, double* dev_out);
 
-/* Token capacity of a query batch for the DEVICE-pointer entry points (lrx_bm25, lrx_search_local*,
- * lrx_search_sharded): the library cannot see dev_q_ptr[B] from the host, so the rows of its
- * per-token tables are sized from this figure; 0 (default) = B * LRX_MAX_QUERY_TERMS.  Every token
+/* Token capacity of a query batch for the DEVICE-pointer entry points (lrx_bm25, lrx_search_sharded):
+ * the library cannot see dev_q_ptr[B] from the host, so the rows of its per-token tables are sized
+ * from this figure; 0 (default) = B * LRX_MAX_QUERY_TERMS.  Every token
  * is scored, in order, as the reference does (retrieval_engine.py:67-68 has no limit).  A batch with
  * MORE tokens than the capacity is never scored short silently: lrx_bm25 returns NaN maxima and the
  * search entry points set bit 2 of the status words.  The host-buffer entry points size the
@@ -238,49 +229,21 @@ int lrx_bm25(lrx_handle* h, const int32_t* dev_q_terms, const int32_t* dev_q_ptr
              const int64_t* dev_cand_ids, int32_t n_cand, double* dev_cand_scores,
              double* dev_max, int32_t K, double* dev_top_scores, int64_t* dev_top_ids);
 
-/* ---- K5: the whole of RetrievalEngine.search for a batch of sub-queries ---
- * lrx_search_local: K2 + K3 on this shard.  Writes, per sub-query b, the shard's
- *   records: dev_records [B][2][K]  ([b][0] = dense list, [b][1] = BM25 list, the
- *   latter all-empty in linear mode) and dev_maxbm25 [B].
- * (all-gather dev_records / dev_maxbm25 across shards -- NCCL, done by the caller)
- * lrx_search_finish: K4.  dev_records_all [world][B][2][K], dev_max_all [world][B];
- *   outputs [B,k]: ids (-1 pad), fused score, semantic, keyword; dev_status [B] is the
- *   OR of the exactness flags (non-zero: rerun with a larger width). */
-int lrx_search_local(lrx_handle* h, const void* dev_q_fp16, const int32_t* dev_q_terms,
-                     const int32_t* dev_q_ptr, int32_t B, int32_t k, int32_t mode,
-                     int32_t width, lrx_record* dev_records, double* dev_maxbm25,
-                     int32_t* dev_flags);
-int lrx_search_finish(lrx_handle* h, const lrx_record* dev_records_all,
-                      const double* dev_max_all, const int32_t* dev_flags_all, int32_t world,
-                      int32_t B, int32_t k, int32_t mode, const double* dev_weights,
-                      int64_t* dev_ids, double* dev_score, double* dev_sem, double* dev_kw,
-                      int32_t* dev_status);
-
-/* Packed form: the shard's records, maxima and flags in ONE contiguous block of
- * lrx_packed_bytes(B,k) bytes ([B][2][2k] records | [B] double | [B] int32, 16-byte
- * padded), so the exchange is a single all-gather per query batch; the gathered buffer
- * [world][packed] goes straight into lrx_search_finish_packed. */
-int64_t lrx_packed_bytes(int32_t B, int32_t k);
-int lrx_search_local_packed(lrx_handle* h, const void* dev_q_fp16, const int32_t* dev_q_terms,
-                            const int32_t* dev_q_ptr, int32_t B, int32_t k, int32_t mode,
-                            int32_t width, void* dev_packed);
-int lrx_search_finish_packed(lrx_handle* h, const void* dev_packed_all, int32_t world, int32_t B,
-                             int32_t k, int32_t mode, const double* dev_weights, int64_t* dev_ids,
-                             double* dev_score, double* dev_sem, double* dev_kw,
-                             int32_t* dev_status);
-
-/* ---- sharded search with the exchange fused into the kernels (world > 1, one box).
- * Replaces "lrx_search_local_packed -> NCCL all-gather -> lrx_search_finish_packed": every rank
- * owns an exchange region (two parities x world slots of one packed block, sequence flags and the
- * call counter); the packing kernel stores the rank's records straight into the slot `rank` of EVERY
- * peer's region over NVLink (peer memory opened through CUDA IPC), its last CTA publishes the
- * call's sequence number with a release store, and the fusion kernel acquires the world flags
- * before it merges.  The sequence number lives on the device, so the whole chain is one captured
- * CUDA graph replayed per batch: no collective library call, no host synchronisation, one launch.
- * Calls must be made in the same order by all ranks (SPMD), each on its own stream.  dev_status[b]:
- * 0 ok, bit 0 = exactness guard (rerun with a larger width), bit 1 = token capacity exceeded,
- * -1 = a peer's block did not arrive within the exchange timeout.  world == 1 is accepted (no
- * exchange): the same call then serves every shard count.
+/* ---- K5: the whole of RetrievalEngine.search for a batch of sub-queries, on one GPU or on the
+ * row shards of one box (world > 1) with the candidate exchange fused into the kernels.
+ * Each shard runs K2 + K3 and packs, per sub-query, its candidate records (the dense list and, in
+ * rrf mode, the BM25 list), its BM25 maximum and its exactness flag into one block.  At world > 1
+ * every rank owns an exchange region (two parities x world slots of one packed block, sequence
+ * flags and the call counter); the packing kernel stores the rank's block straight into the slot
+ * `rank` of EVERY peer's region over NVLink (peer memory opened through CUDA IPC), its last CTA
+ * publishes the call's sequence number with a release store, and the fusion kernel (K4) acquires
+ * the world flags before it merges.  The sequence number lives on the device, so the whole chain
+ * is one captured CUDA graph replayed per batch: no collective library call, no host
+ * synchronisation, one launch.  Calls must be made in the same order by all ranks (SPMD), each on
+ * its own stream.  world == 1 needs no exchange: the same call then serves every shard count.
+ * Outputs [B,k]: ids (-1 pad), fused score, semantic, keyword (replicated on every rank);
+ * dev_status[b]: 0 ok, bit 0 = exactness guard (rerun with a larger width), bit 1 = token capacity
+ * exceeded, -1 = a peer's block did not arrive within the exchange timeout.
  *   lrx_exchange_export  allocates this rank's region for batches up to (B_max, k_max) and
  *                        returns its IPC handle (LRX_IPC_HANDLE_BYTES bytes);
  *   lrx_exchange_import  takes all ranks' handles in rank order (exchanged by the host, e.g. one
@@ -306,12 +269,6 @@ int lrx_search_batch_host(lrx_handle* h, const void* host_q_fp16, const int32_t*
                           const int32_t* host_q_ptr, const double* host_weights, int32_t B,
                           int32_t k, int32_t mode, int64_t* host_ids, double* host_score,
                           double* host_sem, double* host_kw);
-
-/* The same under the name the sharded callers use (world >= 1). */
-int lrx_search_sharded_host(lrx_handle* h, const void* host_q_fp16, const int32_t* host_q_terms,
-                            const int32_t* host_q_ptr, const double* host_weights, int32_t B,
-                            int32_t k, int32_t mode, int64_t* host_ids, double* host_score,
-                            double* host_sem, double* host_kw);
 
 /* Split form for pipelining: _begin stages the inputs in pinned memory and enqueues H2D + the chain
  * + D2H on the handle's stream and returns at once; _end synchronises, checks the status words

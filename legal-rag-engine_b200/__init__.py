@@ -6,7 +6,7 @@ Layout
   engine.py   host-side mirror of the reference's RetrievalEngine / search
   store.py    on-disk vector store (fp16 matrix, CSR postings, metadata.json)
   bm25_index.py  BM25Okapi statistics + CSR postings builder
-  sharding.py multi-GPU: aligned row shards + all-gather of candidate records
+  sharding.py multi-GPU: aligned row shards + in-kernel peer exchange of candidate records
   synth.py    seeded synthetic corpora of the benchmark shapes
 """
 __version__ = "0.1.0"

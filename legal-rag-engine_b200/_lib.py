@@ -37,10 +37,6 @@ class lrx_config(C.Structure):
                 ("world", C.c_int32)]
 
 
-class lrx_record(C.Structure):
-    _fields_ = [("id", C.c_int64), ("dense", C.c_double), ("bm25", C.c_double)]
-
-
 _fp = C.c_void_p   # device pointers to float32 tensors
 
 
@@ -53,10 +49,6 @@ class lrx_bert_weights(C.Structure):
     _fields_ = [("vocab_size", C.c_int32), ("max_positions", C.c_int32),
                 ("word_emb", _fp), ("pos_emb", _fp), ("type_emb", _fp),
                 ("emb_ln_g", _fp), ("emb_ln_b", _fp), ("layers", lrx_bert_layer * 6)]
-
-
-RECORD_BYTES = C.sizeof(lrx_record)
-assert RECORD_BYTES == 24
 
 
 def declared_symbols():
@@ -94,21 +86,12 @@ _SIGNATURES = {
     "lrx_dense_topk_batched": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp]),
     "lrx_dense_at": (C.c_int, [_vp, _vp, _i32, _vp, _i32, _vp]),
     "lrx_bm25": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _i32, _vp, _vp, _i32, _vp, _vp]),
-    "lrx_search_local": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
-    "lrx_search_finish": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp,
-                                    _vp, _vp, _vp]),
-    "lrx_packed_bytes": (_i64, [_i32, _i32]),
-    "lrx_search_local_packed": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp]),
-    "lrx_search_finish_packed": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp,
-                                           _vp, _vp]),
     "lrx_exchange_export": (C.c_int, [_vp, _i32, _i32, _vp]),
     "lrx_exchange_import": (C.c_int, [_vp, _vp]),
     "lrx_search_sharded": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp,
                                      _vp]),
     "lrx_set_query_capacity": (C.c_int, [_vp, _i32]),
     "lrx_set_exchange_timeout": (C.c_int, [_vp, _i32]),
-    "lrx_search_sharded_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp,
-                                          _vp]),
     "lrx_search_host_begin": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32]),
     "lrx_search_text_host_begin": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _i32, _i32]),
     "lrx_search_host_end": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),

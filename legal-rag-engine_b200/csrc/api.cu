@@ -95,7 +95,7 @@ using namespace lrx;
 
 extern "C" {
 
-const char* lrx_version(void) { return "lrx 0.2 sm_100a"; }
+const char* lrx_version(void) { return "lrx 0.3 sm_100a"; }
 
 const char* lrx_last_error(const lrx_handle* h) {
     if (h != nullptr) return h->err.c_str();
@@ -647,7 +647,7 @@ struct LocalScratch {
     int64_t* bm_ids;
     double* maxbm;
     int32_t* flags;
-    unsigned char* block;       // packed block of this shard (world == 1 / unpacked outputs)
+    unsigned char* block;       // packed block of this shard (world == 1)
 };
 
 static int carve_scratch(lrx_handle* h, int B, int k, LocalScratch* s) {
@@ -685,14 +685,16 @@ static int check_search_args(lrx_handle* h, const char* fn, int B, int k, int mo
     return LRX_OK;
 }
 
-// K2 + K3 on this shard and the packed block to `block` (or, to_peers, into every shard's
-// exchange region).  Arguments are checked by the callers.
-static int enqueue_local(lrx_handle* h, const void* q, const int32_t* q_terms, const int32_t* q_ptr,
-                         int B, int k, int mode, int width, const LocalScratch& s, void* block,
-                         bool to_peers) {
+// K2 + K3 on this shard -> packed block -> K4.  world == 1: the block stays in the scratch
+// (s.block); world > 1: it is stored into every shard's exchange region, and K4 reads all the
+// shards' blocks from this rank's region.  Arguments are checked by the callers.
+static int enqueue_search(lrx_handle* h, const LocalScratch& s, const void* q, const int32_t* q_terms,
+                          const int32_t* q_ptr, const double* weights, int B, int k, int mode, int width,
+                          int64_t* ids, double* score, double* sem, double* kw, int32_t* status) {
     const int K = 2 * k;
     size_t o_max, o_flags, total;
     packed_layout(B, k, &o_max, &o_flags, &total);
+    const bool peers = h->world > 1;
     const int Kb = (mode == LRX_FUSE_RRF) ? K : 0;
     h->bm_list_k = Kb;
     // K2a's CTA shares the SM (profiles/r2_runs/ab_bm25_chain_ctas.txt; 5..8 queries on a small shard keep
@@ -707,20 +709,9 @@ static int enqueue_local(lrx_handle* h, const void* q, const int32_t* q_terms, c
     LRX_CUDA(h, cudaEventRecord(h->ev_join, h->aux));
     LRX_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join, 0));   // join
     LRX_CUDA(h, launch_pack_exchange(h, q_terms, q_ptr, B, K, mode, s.dense_exact, s.dense_I, s.bm_scores,
-                                     s.bm_ids, s.maxbm, s.flags, q, block, to_peers, o_max, o_flags));
-    return LRX_OK;
-}
-
-// K4 on [world] packed blocks `all` (stride bytes apart), or on this rank's exchange region.
-static int enqueue_fuse_packed(lrx_handle* h, const void* all, size_t stride, int world, bool from_peers,
-                               int B, int k, int mode, const double* weights, int64_t* ids,
-                               double* score, double* sem, double* kw, int32_t* status) {
-    size_t o_max, o_flags, total;
-    packed_layout(B, k, &o_max, &o_flags, &total);
-    const char* p = (const char*)all;
-    LRX_CUDA(h, launch_fuse(h, (const lrx_record*)p, (const double*)(p + o_max),
-                            (const int32_t*)(p + o_flags), (int64_t)stride, world, B, 2 * k, k, mode,
-                            weights, ids, score, sem, kw, status, from_peers));
+                                     s.bm_ids, s.maxbm, s.flags, q, s.block, peers, o_max, o_flags));
+    LRX_CUDA(h, launch_fuse(h, peers ? h->xchg : s.block, peers ? h->xchg_slot : total, o_max, o_flags, peers,
+                            h->world, B, K, k, mode, weights, ids, score, sem, kw, status));
     return LRX_OK;
 }
 
@@ -835,102 +826,6 @@ int lrx_set_exchange_timeout(lrx_handle* h, int32_t milliseconds) {
     return LRX_OK;
 }
 
-int lrx_search_local(lrx_handle* h, const void* dev_q_fp16, const int32_t* dev_q_terms,
-                     const int32_t* dev_q_ptr, int32_t B, int32_t k, int32_t mode, int32_t width,
-                     lrx_record* dev_records, double* dev_maxbm25, int32_t* dev_flags) {
-    if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_search_local: null handle");
-    std::lock_guard<std::mutex> g(h->mu);
-    if (dev_q_fp16 == nullptr || dev_q_ptr == nullptr || dev_records == nullptr ||
-        dev_maxbm25 == nullptr || dev_flags == nullptr)
-        return fail(h, LRX_E_ARG, "lrx_search_local: null pointer");
-    int rc = check_search_args(h, "lrx_search_local", B, k, mode, &width);
-    if (rc != LRX_OK) return rc;
-    LRX_CUDA(h, cudaSetDevice(h->device));
-    h->bm_rows = h->bm_rows_cfg;
-    LocalScratch s;
-    rc = carve_scratch(h, B, k, &s);
-    if (rc != LRX_OK) return rc;
-    rc = enqueue_local(h, dev_q_fp16, dev_q_terms, dev_q_ptr, B, k, mode, width, s, s.block, false);
-    if (rc != LRX_OK) return rc;
-    size_t o_max, o_flags, total;
-    packed_layout(B, k, &o_max, &o_flags, &total);
-    LRX_CUDA(h, cudaMemcpyAsync(dev_records, s.block, o_max, cudaMemcpyDeviceToDevice, h->stream));
-    LRX_CUDA(h, cudaMemcpyAsync(dev_maxbm25, s.block + o_max, (size_t)B * sizeof(double),
-                                cudaMemcpyDeviceToDevice, h->stream));
-    LRX_CUDA(h, cudaMemcpyAsync(dev_flags, s.block + o_flags, (size_t)B * sizeof(int32_t),
-                                cudaMemcpyDeviceToDevice, h->stream));
-    return LRX_OK;
-}
-
-int lrx_search_finish(lrx_handle* h, const lrx_record* dev_records_all, const double* dev_max_all,
-                      const int32_t* dev_flags_all, int32_t world, int32_t B, int32_t k,
-                      int32_t mode, const double* dev_weights, int64_t* dev_ids, double* dev_score,
-                      double* dev_sem, double* dev_kw, int32_t* dev_status) {
-    if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_search_finish: null handle");
-    std::lock_guard<std::mutex> g(h->mu);
-    if (dev_records_all == nullptr || dev_max_all == nullptr || dev_ids == nullptr ||
-        dev_score == nullptr || dev_sem == nullptr || dev_kw == nullptr || dev_status == nullptr ||
-        (mode == LRX_FUSE_LINEAR && dev_weights == nullptr))
-        return fail(h, LRX_E_ARG, "lrx_search_finish: null pointer");
-    const int K = 2 * k;
-    if (world < 1 || world * K > 2048)
-        return fail(h, LRX_E_ARG, "lrx_search_finish: world*2k must be in [1,2048]");
-    if (B < 1 || B > LRX_MAX_BATCH || k < 1 || K > LRX_MAX_DEPTH)
-        return fail(h, LRX_E_ARG, "lrx_search_finish: bad B/k");
-    LRX_CUDA(h, cudaSetDevice(h->device));
-    LRX_CUDA(h, launch_fuse(h, dev_records_all, dev_max_all, dev_flags_all, 0, world, B, K, k, mode,
-                            dev_weights, dev_ids, dev_score, dev_sem, dev_kw, dev_status, false));
-    return LRX_OK;
-}
-
-int64_t lrx_packed_bytes(int32_t B, int32_t k) {
-    if (B < 1 || k < 1) return 0;
-    size_t a, b, t;
-    packed_layout(B, k, &a, &b, &t);
-    return (int64_t)t;
-}
-
-int lrx_search_local_packed(lrx_handle* h, const void* dev_q_fp16, const int32_t* dev_q_terms,
-                            const int32_t* dev_q_ptr, int32_t B, int32_t k, int32_t mode,
-                            int32_t width, void* dev_packed) {
-    if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_search_local_packed: null handle");
-    std::lock_guard<std::mutex> g(h->mu);
-    if (dev_q_fp16 == nullptr || dev_q_ptr == nullptr || dev_packed == nullptr)
-        return fail(h, LRX_E_ARG, "lrx_search_local_packed: null pointer");
-    int rc = check_search_args(h, "lrx_search_local_packed", B, k, mode, &width);
-    if (rc != LRX_OK) return rc;
-    LRX_CUDA(h, cudaSetDevice(h->device));
-    h->bm_rows = h->bm_rows_cfg;
-    LocalScratch s;
-    rc = carve_scratch(h, B, k, &s);
-    if (rc != LRX_OK) return rc;
-    return run_planned(h, {1u, pk(dev_q_fp16), pk(dev_q_terms), pk(dev_q_ptr), pk(dev_packed), (uint64_t)B,
-                           (uint64_t)k, (uint64_t)mode, (uint64_t)width, (uint64_t)h->bm_rows},
-                       [&]() -> int { return enqueue_local(h, dev_q_fp16, dev_q_terms, dev_q_ptr, B, k, mode,
-                                                    width, s, dev_packed, false); });
-}
-
-int lrx_search_finish_packed(lrx_handle* h, const void* dev_packed_all, int32_t world, int32_t B,
-                             int32_t k, int32_t mode, const double* dev_weights, int64_t* dev_ids,
-                             double* dev_score, double* dev_sem, double* dev_kw,
-                             int32_t* dev_status) {
-    if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_search_finish_packed: null handle");
-    std::lock_guard<std::mutex> g(h->mu);
-    if (dev_packed_all == nullptr || dev_ids == nullptr || dev_score == nullptr ||
-        dev_sem == nullptr || dev_kw == nullptr || dev_status == nullptr ||
-        (mode == LRX_FUSE_LINEAR && dev_weights == nullptr))
-        return fail(h, LRX_E_ARG, "lrx_search_finish_packed: null pointer");
-    if (B < 1 || B > LRX_MAX_BATCH || k < 1 || 2 * k > LRX_MAX_DEPTH)
-        return fail(h, LRX_E_ARG, "lrx_search_finish_packed: bad B/k");
-    if (world < 1 || world * 2 * k > 2048)
-        return fail(h, LRX_E_ARG, "lrx_search_finish_packed: world*2k must be in [1,2048]");
-    size_t o_max, o_flags, total;
-    packed_layout(B, k, &o_max, &o_flags, &total);
-    LRX_CUDA(h, cudaSetDevice(h->device));
-    return enqueue_fuse_packed(h, dev_packed_all, total, world, false, B, k, mode, dev_weights, dev_ids,
-                               dev_score, dev_sem, dev_kw, dev_status);
-}
-
 // ---- peer exchange: region = data [2 parities][world][slot] | flags u64 [2][world] | ctr u64
 static_assert(sizeof(cudaIpcMemHandle_t) == LRX_IPC_HANDLE_BYTES, "IPC handle size");
 
@@ -1001,12 +896,8 @@ static int search_device_locked(lrx_handle* h, const char* fn, const void* q, co
         h, {2u, pk(q), pk(q_terms), pk(q_ptr), pk(weights), pk(ids), pk(score), pk(sem), pk(kw), pk(status),
             (uint64_t)B, (uint64_t)k, (uint64_t)mode, (uint64_t)width, (uint64_t)h->bm_rows},
         [&]() -> int {
-            int r = enqueue_local(h, q, q_terms, q_ptr, B, k, mode, width, s, s.block, peers);
-            if (r != LRX_OK) return r;
-            return peers ? enqueue_fuse_packed(h, h->xchg, h->xchg_slot, h->world, true, B, k, mode, weights,
-                                               ids, score, sem, kw, status)
-                         : enqueue_fuse_packed(h, s.block, total, 1, false, B, k, mode, weights, ids, score,
-                                               sem, kw, status);
+            return enqueue_search(h, s, q, q_terms, q_ptr, weights, B, k, mode, width, ids, score, sem, kw,
+                                  status);
         });
 }
 
@@ -1073,20 +964,10 @@ static int enqueue_host_chain(lrx_handle* h, const lrx_pending& p) {
             LocalScratch s;
             int rc = carve_scratch(h, p.B, p.k, &s);
             if (rc != LRX_OK) return rc;
-            size_t o_max, o_flags, total;
-            packed_layout(p.B, p.k, &o_max, &o_flags, &total);
-            const bool peers = h->world > 1;
-            rc = enqueue_local(h, dp + L.o_q, (const int32_t*)(dp + L.o_terms), (const int32_t*)(dp + L.o_ptr),
-                               p.B, p.k, p.mode, p.width, s, s.block, peers);
-            if (rc != LRX_OK) return rc;
-            rc = peers ? enqueue_fuse_packed(h, h->xchg, h->xchg_slot, h->world, true, p.B, p.k, p.mode,
-                                             (const double*)(dp + L.o_w), (int64_t*)(dp + L.o_ids),
-                                             (double*)(dp + L.o_score), (double*)(dp + L.o_sem),
-                                             (double*)(dp + L.o_kw), (int32_t*)(dp + L.o_status))
-                       : enqueue_fuse_packed(h, s.block, total, 1, false, p.B, p.k, p.mode,
-                                             (const double*)(dp + L.o_w), (int64_t*)(dp + L.o_ids),
-                                             (double*)(dp + L.o_score), (double*)(dp + L.o_sem),
-                                             (double*)(dp + L.o_kw), (int32_t*)(dp + L.o_status));
+            rc = enqueue_search(h, s, dp + L.o_q, (const int32_t*)(dp + L.o_terms), (const int32_t*)(dp + L.o_ptr),
+                                (const double*)(dp + L.o_w), p.B, p.k, p.mode, p.width, (int64_t*)(dp + L.o_ids),
+                                (double*)(dp + L.o_score), (double*)(dp + L.o_sem), (double*)(dp + L.o_kw),
+                                (int32_t*)(dp + L.o_status));
             if (rc != LRX_OK) return rc;
             LRX_CUDA(h, cudaMemcpyAsync(hp + L.in_bytes, dp + L.in_bytes, L.out_bytes, cudaMemcpyDeviceToHost,
                                         h->stream));
@@ -1236,14 +1117,6 @@ int lrx_search_batch_host(lrx_handle* h, const void* host_q_fp16, const int32_t*
                                host_q_ptr, host_weights, B, k, mode);
     if (rc != LRX_OK) return rc;
     return host_end_locked(h, "lrx_search_batch_host", host_ids, host_score, host_sem, host_kw);
-}
-
-int lrx_search_sharded_host(lrx_handle* h, const void* host_q_fp16, const int32_t* host_q_terms,
-                            const int32_t* host_q_ptr, const double* host_weights, int32_t B,
-                            int32_t k, int32_t mode, int64_t* host_ids, double* host_score,
-                            double* host_sem, double* host_kw) {
-    return lrx_search_batch_host(h, host_q_fp16, host_q_terms, host_q_ptr, host_weights, B, k, mode,
-                                 host_ids, host_score, host_sem, host_kw);
 }
 
 int lrx_search_text_host(lrx_handle* h, const int32_t* host_tok_ids, const int32_t* host_tok_lens,

@@ -8,7 +8,7 @@
 //          and BM25 lists, order (rrf desc, id asc).  See oracle/fusion.py.
 //
 // One CTA per sub-query; every shard runs the same deterministic merge on the
-// all-gathered records, so the result is replicated bit for bit.  The shards' lists arrive
+// exchanged records, so the result is replicated bit for bit.  The shards' lists arrive
 // sorted, so merging is rank arithmetic (binary searches), not sorting.
 #include "common.cuh"
 #include "handle.h"
@@ -21,8 +21,8 @@ constexpr int kFuseMaxIn = 2048;   // world * K records per list
 constexpr int kFuseMaxK = LRX_MAX_DEPTH;
 
 // Where a shard's packed block `[B][2][K] records | [B] max | [B] flags` goes.
-//   world == 1 / NCCL exchange : `local` (handle workspace or the caller's all-gather buffer).
-//   peer exchange              : slot `rank` of parity `seq & 1` in EVERY shard's exchange region
+//   world == 1    : `local` (handle workspace).
+//   peer exchange : slot `rank` of parity `seq & 1` in EVERY shard's exchange region
 //     (region = data [2][world][slot] | flags u64 [2][world] | ctr u64 | done u32), stored over
 //     NVLink, then a release store of the call's sequence number into the flag word.  The
 //     sequence number lives ON THE DEVICE (`ctr` in this rank's own region, advanced by the last
@@ -166,14 +166,15 @@ __device__ __forceinline__ int count_greater_sorted(const u128* run, int n, u128
 // K3's merge emit (score desc, id asc)), so the rank of a record in the merged order is a sum of
 // binary searches, and the final order of the <= 2K fused scores is a rank by counting.  Keys are
 // unique (they end in the source slot), so ranks are a permutation.
+//
+// Input: `world` packed blocks `stride` bytes apart -- with `exchange`, one parity of this rank's
+// exchange region (data [2][world][stride] | flags u64 [2][world] | ctr u64), else the local block.
 __global__ void __launch_bounds__(kFuseThreads)
-fuse_kernel(const lrx_record* __restrict__ rec_all, const double* __restrict__ max_all,
-            const int32_t* __restrict__ flags_all, int64_t shard_stride /* bytes; 0 = dense */,
-            int world, int B, int K, int k, int mode,
+fuse_kernel(const unsigned char* __restrict__ blocks, size_t stride, size_t o_max, size_t o_flags,
+            bool exchange, int world, int B, int K, int k, int mode,
             const double* __restrict__ weights, int64_t* __restrict__ out_ids,
             double* __restrict__ out_score, double* __restrict__ out_sem,
             double* __restrict__ out_kw, int32_t* __restrict__ out_status,
-            const void* xchg /* this rank's exchange region, or NULL */, size_t xchg_slot,
             long long timeout_ns, int self) {
     pdl_wait();                                  // the packing / exchange kernel has finished
     extern __shared__ __align__(16) unsigned char fuse_dyn[];
@@ -194,15 +195,11 @@ fuse_kernel(const lrx_record* __restrict__ rec_all, const double* __restrict__ m
     __shared__ int wait_failed;
     if (tid == 0) wait_failed = 0;
     __syncthreads();
-    if (xchg != nullptr) {
-        const unsigned char* base = reinterpret_cast<const unsigned char*>(xchg);
-        const size_t data_bytes = 2 * (size_t)world * xchg_slot;
-        const unsigned long long* fl = reinterpret_cast<const unsigned long long*>(base + data_bytes);
+    if (exchange) {
+        const size_t data_bytes = 2 * (size_t)world * stride;
+        const unsigned long long* fl = reinterpret_cast<const unsigned long long*>(blocks + data_bytes);
         const unsigned long long seq = __ldcg(fl + 2 * world);           // ctr
-        const size_t par_off = (size_t)(seq & 1ull) * world * xchg_slot;
-        rec_all = reinterpret_cast<const lrx_record*>(reinterpret_cast<const unsigned char*>(rec_all) + par_off);
-        max_all = reinterpret_cast<const double*>(reinterpret_cast<const unsigned char*>(max_all) + par_off);
-        flags_all = reinterpret_cast<const int32_t*>(reinterpret_cast<const unsigned char*>(flags_all) + par_off);
+        blocks += (size_t)(seq & 1ull) * world * stride;
         if (tid < world && tid != self) {
             const unsigned long long* wf = fl + (size_t)(seq & 1ull) * world + tid;
             long long t0;
@@ -223,29 +220,21 @@ fuse_kernel(const lrx_record* __restrict__ rec_all, const double* __restrict__ m
     // max_bm25 = max(scores) if max(scores) > 0 else 1.0   (retrieval_engine.py:74)
     double maxbm = 0.0;
     int status = 0;
+#pragma unroll 1                                 // unrolled, its loads in flight set the kernel's register count
     for (int w = 0; w < world; ++w) {
-        const double* mw = shard_stride
-            ? reinterpret_cast<const double*>(reinterpret_cast<const char*>(max_all) + w * shard_stride)
-            : max_all + (size_t)w * B;
-        const double mv = __ldcg(mw + b);
+        const unsigned char* bw = blocks + w * stride;
+        const double mv = __ldcg(reinterpret_cast<const double*>(bw + o_max) + b);
         if (mv != mv) status |= 2;               // NaN: a shard saw more query tokens than its capacity
         maxbm = fmax(maxbm, mv);
-        if (flags_all != nullptr) {
-            const int32_t* fw = shard_stride
-                ? reinterpret_cast<const int32_t*>(reinterpret_cast<const char*>(flags_all) + w * shard_stride)
-                : flags_all + (size_t)w * B;
-            status |= __ldcg(fw + b);
-        }
+        status |= __ldcg(reinterpret_cast<const int32_t*>(bw + o_flags) + b);
     }
     if (!(maxbm > 0.0)) maxbm = 1.0;
 
     // by value, through L2 (ld.cg): the records may have been written by another GPU
     auto rec_at = [&](int list, int src) -> lrx_record {
         const int w = src / K, j = src - w * K;
-        const lrx_record* rw = shard_stride
-            ? reinterpret_cast<const lrx_record*>(reinterpret_cast<const char*>(rec_all) + w * shard_stride)
-            : rec_all + (size_t)w * B * 2 * K;
-        const lrx_record* r = rw + ((size_t)b * 2 + list) * K + j;
+        const lrx_record* r =
+            reinterpret_cast<const lrx_record*>(blocks + w * stride) + ((size_t)b * 2 + list) * K + j;
         lrx_record out;
         out.id = __ldcg(&r->id);
         out.dense = __ldcg(&r->dense);
@@ -389,10 +378,9 @@ cudaError_t launch_pack_exchange(lrx_handle* h, const int32_t* q_terms, const in
     return cudaGetLastError();
 }
 
-cudaError_t launch_fuse(lrx_handle* h, const lrx_record* records_all, const double* max_all,
-                        const int32_t* flags_all, int64_t shard_stride, int world, int B, int K,
-                        int k, int mode, const double* weights, int64_t* ids, double* score,
-                        double* sem, double* kw, int32_t* status, bool from_peers) {
+cudaError_t launch_fuse(lrx_handle* h, const void* blocks, size_t stride, size_t o_max, size_t o_flags,
+                        bool exchange, int world, int B, int K, int k, int mode, const double* weights,
+                        int64_t* ids, double* score, double* sem, double* kw, int32_t* status) {
     {
         std::lock_guard<std::recursive_mutex> attr_guard(attr_mutex());   // the flags below are process-wide
         static bool attr_dev[64] = {false};   // function attributes are per device
@@ -406,9 +394,9 @@ cudaError_t launch_fuse(lrx_handle* h, const lrx_record* records_all, const doub
     }
     if (world * K > kFuseMaxIn || K > kFuseMaxK) return cudaErrorInvalidValue;
     cudaError_t e = launch_pdl(fuse_kernel, dim3(B), dim3(kFuseThreads), kFuseMaxIn * sizeof(u128), h->stream,
-                               records_all, max_all, flags_all, shard_stride, world, B, K, k, mode, weights,
-                               ids, score, sem, kw, status, from_peers ? (const void*)h->xchg : (const void*)nullptr,
-                               h->xchg_slot, (long long)h->xchg_timeout_ms * 1000000ll, h->rank);
+                               (const unsigned char*)blocks, stride, o_max, o_flags, exchange, world, B, K, k,
+                               mode, weights, ids, score, sem, kw, status,
+                               (long long)h->xchg_timeout_ms * 1000000ll, h->rank);
     h->launches++;
     return e;
 }

@@ -10,6 +10,14 @@
 
 #include "../../include/lrx.h"
 
+// One candidate of one sub-query on one shard: the unit of the packed block the shards exchange
+// (SURVEY.md section 8e).  24 bytes.
+struct lrx_record {
+    int64_t id;            // global chunk id, -1 = empty slot
+    double dense;          // exact inner product (see oracle/flat_ip.py)
+    double bm25;           // exact BM25Okapi score of that chunk
+};
+
 // One captured launch chain (CUDA graph) of a search entry point, keyed on everything the
 // launches depend on (shapes, mode, pointers); replayed with one cudaGraphLaunch.
 struct lrx_plan {
@@ -74,7 +82,7 @@ struct lrx_handle {
     void* ws_dense_part = nullptr;   size_t ws_dense_part_bytes = 0;    // per-CTA key lists
     void* ws_bm_part = nullptr;      size_t ws_bm_part_bytes = 0;       // per-chunk key lists
     void* ws_bm_max = nullptr;       size_t ws_bm_max_bytes = 0;        // per-CTA max
-    void* ws_misc = nullptr;         size_t ws_misc_bytes = 0;          // search_local scratch
+    void* ws_misc = nullptr;         size_t ws_misc_bytes = 0;          // search chain scratch
     void* ws_host = nullptr;         size_t ws_host_bytes = 0;          // pinned staging
     void* ws_io = nullptr;           size_t ws_io_bytes = 0;            // device staging
     void* ws_rm = nullptr;           size_t ws_rm_bytes = 0;            // index removal: doc map, tile table
@@ -169,10 +177,11 @@ cudaError_t launch_pack_exchange(lrx_handle* h, const int32_t* q_terms, const in
                                  const double* bm_scores, const int64_t* bm_ids, const double* maxbm,
                                  const int32_t* flags, const void* q, void* local_block, bool to_peers,
                                  size_t o_max, size_t o_flags);
-cudaError_t launch_fuse(lrx_handle* h, const lrx_record* records_all, const double* max_all,
-                        const int32_t* flags_all, int64_t shard_stride, int world, int B, int K,
-                        int k, int mode, const double* weights, int64_t* ids, double* score,
-                        double* sem, double* kw, int32_t* status, bool from_peers);
+// blocks: `world` packed blocks `stride` bytes apart -- this rank's exchange region (exchange) or the
+// local block (world == 1)
+cudaError_t launch_fuse(lrx_handle* h, const void* blocks, size_t stride, size_t o_max, size_t o_flags,
+                        bool exchange, int world, int B, int K, int k, int mode, const double* weights,
+                        int64_t* ids, double* score, double* sem, double* kw, int32_t* status);
 
 // encoder.cu
 cudaError_t encoder_set_weights(lrx_handle* h, const lrx_bert_weights* w);

@@ -10,7 +10,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import LRX_DIM, LRX_FUSE_LINEAR, LRX_FUSE_RRF, RECORD_BYTES
+from ._lib import LRX_DIM, LRX_FUSE_LINEAR, LRX_FUSE_RRF
 
 FUSION = {"linear": LRX_FUSE_LINEAR, "rrf": LRX_FUSE_RRF}
 
@@ -342,60 +342,13 @@ class DeviceIndex:
                                    K, _ptr(ts), _ptr(ti)))
         return cs, mx, ts[:, :K], ti[:, :K]
 
-    def search_local(self, q, q_terms, q_ptr, k: int, mode: int, width: int = 0):
-        """K2 + K3 on this shard -> (records uint8 [B,2,2k,24], maxbm25 [B], flags [B])."""
-        B = int(q.shape[0])
-        K = 2 * k
-        rec = torch.empty((B, 2, K, RECORD_BYTES), dtype=torch.uint8, device=self.device)
-        mx = torch.empty(B, dtype=torch.float64, device=self.device)
-        flags = torch.empty(B, dtype=torch.int32, device=self.device)
-        if q_terms.numel() == 0:
-            q_terms = torch.zeros(1, dtype=torch.int32, device=self.device)
-        self._cap(q_terms, B)
-        self._ck(self.lib.lrx_search_local(self.h, _ptr(q), _ptr(q_terms), _ptr(q_ptr), B, k, mode,
-                                           width, _ptr(rec), _ptr(mx), _ptr(flags)))
-        return rec, mx, flags
-
-    def search_finish(self, rec_all, max_all, flags_all, world: int, B: int, k: int, mode: int,
-                      weights: torch.Tensor):
-        ids = torch.empty((B, k), dtype=torch.int64, device=self.device)
-        score = torch.empty((B, k), dtype=torch.float64, device=self.device)
-        sem = torch.empty((B, k), dtype=torch.float64, device=self.device)
-        kw = torch.empty((B, k), dtype=torch.float64, device=self.device)
-        status = torch.empty(B, dtype=torch.int32, device=self.device)
-        self._ck(self.lib.lrx_search_finish(self.h, _ptr(rec_all), _ptr(max_all), _ptr(flags_all),
-                                            world, B, k, mode, _ptr(weights), _ptr(ids), _ptr(score),
-                                            _ptr(sem), _ptr(kw), _ptr(status)))
-        return ids, score, sem, kw, status
-
-    # ------------------------------------------------ packed form (one all-gather)
-    def packed_bytes(self, B: int, k: int) -> int:
-        return int(self.lib.lrx_packed_bytes(B, k))
-
-    def search_local_packed(self, q, q_terms, q_ptr, k: int, mode: int, out: torch.Tensor,
-                            width: int = 0):
-        """K2 + K3 on this shard into `out` (uint8 [packed_bytes]) -- the all-gather unit."""
-        B = int(q.shape[0])
-        self._cap(q_terms, B)
-        self._ck(self.lib.lrx_search_local_packed(self.h, _ptr(q), _ptr(q_terms), _ptr(q_ptr), B, k,
-                                                  mode, width, _ptr(out)))
-        return out
-
-    def search_finish_packed(self, packed_all, world: int, B: int, k: int, mode: int, weights, outs):
-        """K4 on the gathered [world][packed] buffer; outs = (ids, score, sem, kw, status)."""
-        ids, score, sem, kw, status = outs
-        self._ck(self.lib.lrx_search_finish_packed(self.h, _ptr(packed_all), world, B, k, mode,
-                                                   _ptr(weights), _ptr(ids), _ptr(score), _ptr(sem),
-                                                   _ptr(kw), _ptr(status)))
-        return outs
-
     # ------------------------------------ peer-memory exchange (world > 1, one box)
     def exchange_setup(self, B_max: int, k_max: int, group=None) -> bool:
         """Allocate this rank's exchange region, swap IPC handles with the other ranks (one
         all-gather of 64 bytes at start-up) and open theirs: afterwards `search_sharded` needs no
         collective call per query batch.  Returns False -- on EVERY rank, the outcome is agreed by
         an all-reduce -- when some rank could not export or map a region (e.g. no peer access
-        between the GPUs); the caller then keeps the NCCL exchange."""
+        between the GPUs): a sharded search cannot run on that box."""
         import torch.distributed as dist
         from ._lib import LRX_IPC_HANDLE_BYTES, LrxError
         ok = 1

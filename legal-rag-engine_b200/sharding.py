@@ -1,5 +1,5 @@
 """Multi-GPU layout of the hybrid index: one process per GPU (torchrun), aligned row shards,
-one all-gather of candidate records per query batch (SURVEY.md 8e).
+one exchange of candidate records per query batch (SURVEY.md 8e).
 
 GPU g owns the contiguous global id range ``shard_range(N, g, G)`` of BOTH the fp16 chunk
 matrix and the BM25 postings (doc ids local, ``id_base`` added on the way out).  idf / avgdl
@@ -7,19 +7,13 @@ are whole-corpus statistics (``global_bm25_stats``: two all-reduces at build tim
 shard's BM25 scores equal the unsharded ones bit for bit.  Per query batch each rank runs
 K2 + K3 on its shard, the packed blocks ``[B][2][2k] records | [B] max | [B] flags`` (~1 KB per
 sub-query per rank -- latency-bound) are exchanged, and every rank runs the same deterministic
-merge + fusion.  Two exchanges:
-
-* ``exchange="peer"`` (default on CUDA): ``lrx_search_sharded`` -- the block is stored straight
-  into every peer's memory over NVLink by a kernel of the chain and the fusion kernel acquires the
-  peers' sequence flags; no collective call per batch (the IPC handles are swapped once).
-* ``exchange="nccl"``: ``lrx_search_local_packed`` -> ONE ``all_gather_into_tensor`` ->
-  ``lrx_search_finish_packed`` (also what the gloo CPU test of the host logic mirrors).
+merge + fusion.  The exchange is ``lrx_search_sharded``: a kernel of the chain stores the block
+straight into every peer's memory over NVLink and the fusion kernel acquires the peers' sequence
+flags; no collective call per batch (the IPC handles are swapped once).
 """
 from __future__ import annotations
 
-from typing import Optional, Tuple
-
-import os
+from typing import Tuple
 
 import numpy as np
 import torch
@@ -45,7 +39,7 @@ def global_bm25_stats(df_local: torch.Tensor, total_len_local: int, group=None):
 
 
 def packed_layout(B: int, k: int):
-    """Byte offsets of the packed per-shard block (must equal lrx_packed_bytes / api.cu)."""
+    """Byte offsets of the packed per-shard block (must equal packed_layout in csrc/api.cu)."""
     rec = B * 2 * (2 * k) * RECORD.itemsize
     o_max = rec
     o_flags = rec + B * 8
@@ -62,33 +56,25 @@ def unpack(block: np.ndarray, B: int, k: int):
 
 
 class ShardedSearcher:
-    """K2+K3 local -> all-gather -> K4, for device-resident query batches."""
+    """K2+K3 local -> peer exchange -> K4, for device-resident query batches."""
 
-    def __init__(self, dev, group=None, exchange: Optional[str] = None, B_max: int = 64,
-                 k_max: int = 128):
+    exchange = "peer"          # the only cross-shard path; bench.py reports it
+
+    def __init__(self, dev, group=None, B_max: int = 64, k_max: int = 128):
         self.dev = dev
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         self._bufs = {}
-        self.exchange = exchange or os.environ.get("LRX_EXCHANGE", "peer")
-        if self.exchange not in ("peer", "nccl"):
-            raise ValueError("exchange must be 'peer' or 'nccl'")
-        if self.world > 1 and self.exchange == "peer":
-            if not dev.exchange_setup(B_max, k_max, group):
-                import warnings
-                warnings.warn("peer-memory exchange unavailable on this box (no CUDA IPC / peer access "
-                              "between the GPUs): using the NCCL all-gather exchange")
-                self.exchange = "nccl"
+        if self.world > 1 and not dev.exchange_setup(B_max, k_max, group):
+            raise RuntimeError("the GPUs of this box cannot map each other's memory (CUDA IPC / peer "
+                               "access): the sharded engine needs it")
 
     def buffers(self, B: int, k: int):
+        # a 3-tuple whose third item is the output tuple: the layout bench.py reads
         key = (B, k)
         if key not in self._bufs:
-            pb = self.dev.packed_bytes(B, k)
-            mine = torch.empty(pb, dtype=torch.uint8, device=self.dev.device)
-            every = torch.empty(pb * self.world, dtype=torch.uint8, device=self.dev.device) \
-                if self.world > 1 else mine
-            self._bufs[key] = (mine, every, self.dev.alloc_outputs(B, k))
+            self._bufs[key] = (None, None, self.dev.alloc_outputs(B, k))
         return self._bufs[key]
 
     def search(self, q_fp16: torch.Tensor, q_terms: torch.Tensor, q_ptr: torch.Tensor, k: int, mode: int,
@@ -97,13 +83,8 @@ class ShardedSearcher:
         rank).  Asynchronous on torch's current stream; `status` must be looked at by the caller
         (`search_checked` does) -- 0 ok, 1 = exactness guard (rerun wider), 2 = token capacity,
         -1 = a peer's block did not arrive in time."""
-        B = int(q_fp16.shape[0])
-        mine, every, outs = self.buffers(B, k)
-        if self.world == 1 or self.exchange == "peer":
-            return self.dev.search_sharded(q_fp16, q_terms, q_ptr, k, mode, weights, outs, width)
-        self.dev.search_local_packed(q_fp16, q_terms, q_ptr, k, mode, mine, width)
-        dist.all_gather_into_tensor(every, mine, group=self.group)
-        return self.dev.search_finish_packed(every, self.world, B, k, mode, weights, outs)
+        outs = self.buffers(int(q_fp16.shape[0]), k)[2]
+        return self.dev.search_sharded(q_fp16, q_terms, q_ptr, k, mode, weights, outs, width)
 
     def search_checked(self, q_fp16, q_terms, q_ptr, k: int, mode: int, weights):
         """`search` + a synchronising look at the status words: widens the dense candidate lists

@@ -329,43 +329,6 @@ def test_real_corpus_hybrid_search(dev, legal_texts, reference_queries):
         _assert_results(got, want, 10)
 
 
-# ------------------------------------------------------ shards on one GPU
-@pytest.mark.parametrize("fusion", ["linear", "rrf"])
-def test_two_shards_merge_equals_unsharded(fusion):
-    """Emulates the all-gather on one GPU: two shard handles, records concatenated,
-    lrx_search_finish on the union == the unsharded oracle."""
-    from legal_rag_engine_b200.device_index import DeviceIndex, FUSION
-    n, cut = 50000, 21000
-    x = synth.host_vectors(n, seed=31, dup_frac=0.01)
-    idx = synth.host_bm25(n, seed=32, vocab=3000)
-    csr = _csr_of(idx)
-    B, k = 4, 10
-    q = synth.host_queries(B, seed=33)
-    terms, ptr = synth.host_query_terms(B, 8, seed=34, vocab=3000)
-    lists = [terms[ptr[b]:ptr[b + 1]].tolist() for b in range(B)]
-    weights = [0.5, 0.6, 0.5, 0.6]
-    shards = []
-    for r, (lo, hi) in enumerate([(0, cut), (cut, n)]):
-        d = DeviceIndex(0, rank=r, world=2)
-        d.set_corpus(_cuda(x[lo:hi]), lo)
-        sh = idx.shard(lo, hi)
-        d.set_postings(sh.term_ptr, sh.postings, sh.doc_len, sh.idf, sh.avgdl)
-        shards.append(d)
-    recs, maxes, flags = [], [], []
-    for d in shards:
-        r, m, f = d.search_local(_cuda(q), _cuda(terms), _cuda(ptr), k, FUSION[fusion])
-        recs.append(r); maxes.append(m); flags.append(f)
-    rec_all, max_all, flags_all = torch.stack(recs), torch.stack(maxes), torch.stack(flags)
-    out = shards[0].search_finish(rec_all, max_all, flags_all, 2, B, k, FUSION[fusion],
-                                  _cuda(np.array(weights)))
-    ids, score, sem, kw, status = [t.cpu().numpy() for t in out]
-    assert status.sum() == 0
-    want = _oracle_search(x, csr, q, lists, k, weights, fusion)
-    _assert_results((ids, score, sem, kw), want, k)
-    for d in shards:
-        d.close()
-
-
 def test_one_million_rows(dev):
     """Config C3 size: 1 M x 384, batch 1 and 4, top-20 -- still bit-exact."""
     n = 1_000_000

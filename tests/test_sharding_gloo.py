@@ -1,7 +1,7 @@
 """world_size-2 gloo test (CPU) of the multi-GPU host logic: aligned shard ranges, global BM25
-statistics by all-reduce, the packed record block and its single all-gather, and the merge rule
--- with the CPU oracle standing in for the per-shard kernels.  The result on every rank must
-equal the unsharded oracle search."""
+statistics by all-reduce, the per-shard packed record block exchanged between the ranks, and the
+merge rule -- with the CPU oracle standing in for the per-shard kernels.  The result on every rank
+must equal the unsharded oracle search."""
 import os
 import socket
 
@@ -11,7 +11,7 @@ import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
-from legal_rag_engine_b200 import _lib, sharding, synth
+from legal_rag_engine_b200 import sharding, synth
 from legal_rag_engine_b200.bm25_index import okapi_idf
 from oracle import bm25 as obm25
 from oracle import flat_ip, fusion
@@ -36,7 +36,7 @@ def _inputs():
 
 
 def _oracle_local_block(x_sh, csr_sh, lo, q, lists, k, mode):
-    """What lrx_search_local_packed emits for one shard, computed by the oracle."""
+    """The packed block one shard's K2 + K3 emit, computed by the oracle."""
     o_max, o_flags, total = sharding.packed_layout(B, k)
     block = np.zeros(total, dtype=np.uint8)
     rec, mx, flags = sharding.unpack(block, B, k)
@@ -61,7 +61,7 @@ def _oracle_local_block(x_sh, csr_sh, lo, q, lists, k, mode):
 
 
 def _oracle_finish(blocks, world, k, mode, weights):
-    """The merge rule of lrx_search_finish_packed: (score desc, id asc) over the union."""
+    """The merge rule of K4 (fuse_kernel): (score desc, id asc) over the union."""
     K = 2 * k
     out = []
     parts = [sharding.unpack(blocks[r], B, k) for r in range(world)]
@@ -123,13 +123,6 @@ def test_two_rank_exchange_equals_unsharded(mode):
         mp.spawn(_worker, args=(2, port, mode, ret), nprocs=2, join=True)
         got0, got1 = ret[0], ret[1]
     assert got0 == got1 == want
-
-
-def test_packed_layout_matches_c_abi():
-    lib = _lib.load()
-    for B_, k_ in ((1, 1), (4, 10), (3, 7), (64, 128), (5, 50)):
-        assert sharding.packed_layout(B_, k_)[2] == lib.lrx_packed_bytes(B_, k_)
-    assert sharding.RECORD.itemsize == _lib.RECORD_BYTES
 
 
 def test_shard_ranges_tile_the_corpus():
