@@ -202,8 +202,11 @@ int lrx_dense_topk_ex(lrx_handle* h, const void* dev_q_fp16, int32_t B, int32_t 
 /* K2b: the same search for LARGE batches (B up to 4096; FAISS's BLAS regime, nq >= 20) on the
  * tensor cores: two tcgen05 GEMM passes (tile maxima -> per-query threshold; candidates above
  * it) + exact float64 re-score.  Same outputs and ordering as lrx_dense_topk.  stride: pass 1
- * samples every stride-th 256-row tile (0 = automatic).  dev_flags[b] = 1: more than 1024
- * candidates survived for query b -- rerun with stride 1. */
+ * samples every stride-th 256-row tile (0 = automatic; above 524 288 rows the stride is raised so
+ * that at most 16 384 chunks are sampled).  When fewer than 2K sampled 32-row chunks hold rows the
+ * batch runs the lrx_dense_topk scan instead.  dev_flags[b] = 1: more than 1024 rows scored within
+ * the band of query b's K-th score (many near-identical rows: a stride-1 rerun is flagged too) --
+ * answer query b with lrx_dense_topk_ex and a larger width. */
 int lrx_dense_topk_batched(lrx_handle* h, const void* dev_q_fp16, int32_t B, int32_t K, int32_t stride,
                            double* dev_exact, float* dev_D, int64_t* dev_I, int32_t* dev_flags);
 /* Exact inner products at given global ids (ids outside the shard or -1 -> -inf). */

@@ -505,8 +505,10 @@ int lrx_gemm_f16(lrx_handle* h, const void* dev_a, const void* dev_w, int32_t M,
 // of the matrix (K2a, HBM-bound: the 8 columns of its MMA tile are all queries then); from 9 queries
 // on the tensor-core kernel scores the whole batch in one pass (K2b) where K2a would need
 // ceil(B / 8) -- measured at 10 M rows: B = 64 1.32 ms against 18.1 ms (tools/k2_crossover.py); both
-// emit the same exact lists.  A widened retry (exactness guard / candidate overflow) makes K2b sample
-// every tile.  LRX_K2B_MIN_B overrides the crossover (A/B runs).
+// emit the same exact lists.  A widened retry (exactness guard / candidate overflow) runs K2a at
+// that width: width is K2a's parameter, and K2b flags only a query with more than 1024 rows near its
+// K-th score, which K2b at any stride would flag again.  LRX_K2B_MIN_B overrides the crossover (A/B
+// runs).
 static int k2b_min_b() {
     static int v = -1;
     if (v < 0) {
@@ -526,10 +528,8 @@ static int bm_chain_ctas() {
 }
 static cudaError_t launch_dense_auto(lrx_handle* h, const void* q, int B, int K, int width, double* exact,
                                      float* D, int64_t* I, int32_t* flags) {
-    if (B >= k2b_min_b() && h->n_local > 0 && ((uintptr_t)q & 15) == 0) {
-        const int stride = (width > dense_default_width(K)) ? 1 : 0;
-        return launch_dense_topk_batched(h, q, B, K, stride, exact, D, I, flags);
-    }
+    if (B >= k2b_min_b() && h->n_local > 0 && ((uintptr_t)q & 15) == 0 && width <= dense_default_width(K))
+        return launch_dense_topk_batched(h, q, B, K, 0, exact, D, I, flags);
     return launch_dense_topk(h, q, B, K, width, exact, D, I, flags);
 }
 

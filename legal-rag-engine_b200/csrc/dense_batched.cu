@@ -10,11 +10,16 @@
 //           The K-th largest chunk maximum T[q] (tilemax_kth_kernel) is a lower bound of the
 //           K-th best score: K distinct rows reach it.
 //   pass 2  over all tiles: every (query, row) with score >= T[q] - slack is appended to the
-//           query's candidate list (global atomics; a few hundred per query).
+//           query's candidate list (a few hundred per query): a private region per (query, CTA,
+//           column half), and once that region is full a per-query overflow list of kDbCap slots.
 // dense_rescore_list_kernel then re-scores the candidates EXACTLY in float64 (oracle/flat_ip.py),
 // orders them by (score desc, id asc) and emits the best K.  With slack = 2 * kTcEps a row that
 // was not appended is strictly below the K-th best exact score, so the result is bit-exact; the
-// only failure mode is a candidate list overflow (flag -> caller reruns with stride 1).
+// only failure mode is more than kDbCap candidates for a query (flag).  Where fewer than 2K
+// sampled chunks hold rows, T would be loose (or -FLT_MAX: chunks past the corpus end rank too),
+// so such a batch goes to the streaming scan (K2a) instead.  Chunk stores keep similar chunks next
+// to one another, so a query's candidates can crowd into a few regions: the overflow list keeps
+// that from flagging it.
 //
 // Kernel shape (one CTA per SM, 320 threads, warp-specialised like tc_gemm.cu):
 //   A operand = 128 queries x 384, loaded once by TMA and RESIDENT in shared memory (96 KB);
@@ -70,8 +75,16 @@ struct DbParams {
     int n_regions;         // 2 * CTAs per query tile
     int region_cap;        // slots per region
     int* cnt;              // [n_mt*128][n_regions] candidates found (may exceed region_cap: overflow)
-    uint32_t* cand;        // [n_mt*128][n_regions][region_cap] local row ids
+    // [n_mt*128][n_regions * region_cap + kDbCap] local row ids: the query's regions, then its
+    // overflow list, where a full region's further candidates go behind one atomicAdd (rare: a
+    // region fills only where similar rows cluster)
+    uint32_t* cand;
+    int* ov_cnt;           // [n_mt*128] candidates spilled (may exceed kDbCap); tilemax_kth_kernel zeroes it
 };
+
+__host__ __device__ inline size_t db_cand_per_query(int n_regions, int region_cap) {
+    return (size_t)n_regions * region_cap + kDbCap;
+}
 
 // CS: cluster size.  The CS CTAs of a cluster serve CS different query tiles and walk the SAME chunk
 // tiles: each loads 1/CS of a tile's rows and multicasts them to all (one L2 read per cluster).
@@ -192,7 +205,8 @@ dense_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant
         uint32_t rb[2][32];
         const int region = group * 2 + half;
         int my_cnt = 0;                                      // candidates of (q, region) so far
-        uint32_t* my_cand = P.cand + ((size_t)q * P.n_regions + region) * P.region_cap;
+        uint32_t* q_cand = P.cand + (size_t)q * db_cand_per_query(P.n_regions, P.region_cap);
+        uint32_t* my_cand = q_cand + (size_t)region * P.region_cap;
         for (int u = 0; u < my_units; ++u) {
             const int buf = u & 1;
             const uint32_t use = (uint32_t)(u >> 1);
@@ -239,7 +253,13 @@ dense_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant
                         while (mask != 0u) {
                             const int j = __ffs((int)mask) - 1;
                             mask &= mask - 1u;
-                            if (my_cnt < P.region_cap) my_cand[my_cnt] = (uint32_t)(row0 + c + j);
+                            const uint32_t row = (uint32_t)(row0 + c + j);
+                            if (my_cnt < P.region_cap) {
+                                my_cand[my_cnt] = row;
+                            } else {
+                                const int o = atomicAdd(&P.ov_cnt[q], 1);
+                                if (o < kDbCap) q_cand[(size_t)P.n_regions * P.region_cap + o] = row;
+                            }
                             ++my_cnt;
                         }
                     }
@@ -264,10 +284,11 @@ dense_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant
 // T[q] = (K-th largest tile maximum) - slack; -FLT_MAX when fewer than K tiles were sampled.
 // One CTA per query.  Only the K-th largest of up to 16 384 values is needed, so this is a radix
 // SELECT over the order images (four 8-bit passes: shared-memory histogram of the keys that match
-// the prefix found so far, then warp 0 walks the 256 bins from the top), not a sort.
+// the prefix found so far, then warp 0 walks the 256 bins from the top), not a sort.  Also resets
+// the query's overflow counter for pass 2.
 __global__ void __launch_bounds__(256)
 tilemax_kth_kernel(const float* __restrict__ tilemax, int n_samp, int K, float slack,
-                   float* __restrict__ thr) {
+                   float* __restrict__ thr, int* __restrict__ ov_cnt) {
     extern __shared__ uint32_t tm_keys[];
     __shared__ uint32_t hist[256];
     __shared__ uint32_t s_prefix, s_rank;
@@ -315,7 +336,10 @@ tilemax_kth_kernel(const float* __restrict__ tilemax, int n_samp, int K, float s
             __syncthreads();
         }
     }
-    if (tid == 0) thr[q] = (K <= n_samp) ? ord_f32(s_prefix) - slack : -FLT_MAX;
+    if (tid == 0) {
+        thr[q] = (K <= n_samp) ? ord_f32(s_prefix) - slack : -FLT_MAX;
+        ov_cnt[q] = 0;
+    }
 }
 
 // Exact float64 re-score of a query's (unsorted) candidate list, best K out.  Each warp takes four
@@ -325,34 +349,32 @@ constexpr int kRlThreads = 256;
 __global__ void __launch_bounds__(kRlThreads)
 dense_rescore_list_kernel(const unsigned char* __restrict__ x, int64_t id_base,
                           const __half* __restrict__ q, const uint32_t* __restrict__ cand,
-                          const int* __restrict__ cnt, int n_regions, int region_cap, int K,
-                          double* __restrict__ out_exact,
+                          const int* __restrict__ cnt, const int* __restrict__ ov_cnt, int n_regions,
+                          int region_cap, int K, double* __restrict__ out_exact,
                           float* __restrict__ out_D, int64_t* __restrict__ out_I,
                           int32_t* __restrict__ out_flag) {
     __shared__ u128 keys[kDbCap];
     __shared__ u128 best[LRX_MAX_DEPTH];
-    __shared__ int pre[kDbMaxRegions + 1];                   // candidates before region r
-    __shared__ int s_over;
+    __shared__ int pre[kDbMaxRegions + 2];                   // candidates before region r
     const int qi = blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    // the query's regions, concatenated: candidate i lives in the region r with pre[r] <= i < pre[r+1]
+    // the query's regions, concatenated, then its overflow list as region n_regions (it follows the
+    // regions in memory): candidate i lives in the region r with pre[r] <= i < pre[r+1]
     if (tid == 0) {
-        int acc = 0, over = 0;
+        int acc = 0;
         for (int r = 0; r < n_regions; ++r) {
-            const int c = cnt[(size_t)qi * n_regions + r];
-            over |= (c > region_cap) ? 1 : 0;
             pre[r] = acc;
-            acc += min(c, region_cap);
+            acc += min(cnt[(size_t)qi * n_regions + r], region_cap);
         }
         pre[n_regions] = acc;
-        s_over = over;
+        pre[n_regions + 1] = acc + ov_cnt[qi];
     }
     __syncthreads();
-    const int total = pre[n_regions];
+    const int total = pre[n_regions + 1];
     const int n = min(total, kDbCap);
-    const uint32_t* qcand = cand + (size_t)qi * n_regions * region_cap;
+    const uint32_t* qcand = cand + (size_t)qi * db_cand_per_query(n_regions, region_cap);
     auto cand_at = [&](int i) -> uint32_t {
-        int lo = 0, hi = n_regions;                          // last r with pre[r] <= i
+        int lo = 0, hi = n_regions + 1;                      // last r with pre[r] <= i
         while (hi - lo > 1) {
             const int mid = (lo + hi) >> 1;
             if (pre[mid] <= i) lo = mid; else hi = mid;
@@ -419,7 +441,7 @@ dense_rescore_list_kernel(const unsigned char* __restrict__ x, int64_t id_base,
             out_I[o] = -1;
         }
     }
-    if (tid == 0) out_flag[qi] = (total > kDbCap || s_over) ? 1 : 0;
+    if (tid == 0) out_flag[qi] = (total > kDbCap) ? 1 : 0;
 }
 
 int dense_batched_max_stride(int64_t n_rows, int K) {
@@ -463,8 +485,13 @@ cudaError_t launch_dense_topk_batched(lrx_handle* h, const void* q, int B, int K
         stride = (n_tiles * kChunks + 16383) / 16384;
         n_samp = (n_tiles + stride - 1) / stride * kChunks;
     }
-    if (n_samp < K) {
-        // tiny corpus for this K: no useful threshold -- the streaming kernel, 64 queries a time
+    // sampled chunks that hold rows: 8 per sampled tile, fewer when the last tile is sampled.  The
+    // others have maximum -FLT_MAX; with fewer than 2K valid ones T is loose (the lists overflow) or
+    // -FLT_MAX (every row a candidate)
+    int64_t valid = (int64_t)((n_tiles + stride - 1) / stride) * kChunks;
+    if ((n_tiles - 1) % stride == 0) valid -= kChunks - (n - (int64_t)(n_tiles - 1) * kDbN + 31) / 32;
+    if (valid < 2 * (int64_t)K) {
+        // small corpus for this K: no useful threshold -- the streaming kernel, 64 queries a time
         for (int b0 = 0; b0 < B; b0 += LRX_MAX_BATCH) {
             const int nb = (B - b0 < LRX_MAX_BATCH) ? (B - b0) : LRX_MAX_BATCH;
             e = launch_dense_topk(h, (const __half*)q + (size_t)b0 * kDim, nb, K, dense_default_width(K),
@@ -485,7 +512,8 @@ cudaError_t launch_dense_topk_batched(lrx_handle* h, const void* q, int B, int K
     int region_cap = 16;                       // >= 2048 slots per query over its regions: an even
     while (region_cap * n_regions < 2048) region_cap <<= 1;   // spread fills a few percent of a region
     const size_t o_cnt = take((size_t)Bp * n_regions * sizeof(int));
-    const size_t o_cand = take((size_t)Bp * n_regions * region_cap * sizeof(uint32_t));
+    const size_t o_cand = take((size_t)Bp * db_cand_per_query(n_regions, region_cap) * sizeof(uint32_t));
+    const size_t o_ov_cnt = take((size_t)Bp * sizeof(int));
     e = ensure_ws(h, &h->ws_dense_part, &h->ws_dense_part_bytes, off);
     if (e != cudaSuccess) return e;
     char* W = (char*)h->ws_dense_part;
@@ -499,6 +527,7 @@ cudaError_t launch_dense_topk_batched(lrx_handle* h, const void* q, int B, int K
     P.tilemax = (float*)(W + o_tm); P.n_samp = n_samp; P.thr = (const float*)(W + o_thr);
     P.cnt = (int*)(W + o_cnt); P.cand = (uint32_t*)(W + o_cand);
     P.n_regions = n_regions; P.region_cap = region_cap;
+    P.ov_cnt = (int*)(W + o_ov_cnt);
     auto launch = [&](int pass) -> cudaError_t {
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(grid);
@@ -525,7 +554,7 @@ cudaError_t launch_dense_topk_batched(lrx_handle* h, const void* q, int B, int K
     h->launches++;
     if (e != cudaSuccess) return e;
     tilemax_kth_kernel<<<Bp, 256, (size_t)next_pow2(n_samp > 2 ? n_samp : 2) * sizeof(uint32_t), h->stream>>>(
-        P.tilemax, n_samp, K, 2.0f * kTcEps, (float*)(W + o_thr));
+        P.tilemax, n_samp, K, 2.0f * kTcEps, (float*)(W + o_thr), P.ov_cnt);
     h->launches++;
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
@@ -535,8 +564,8 @@ cudaError_t launch_dense_topk_batched(lrx_handle* h, const void* q, int B, int K
     h->launches++;
     if (e != cudaSuccess) return e;
     dense_rescore_list_kernel<<<B, kRlThreads, 0, h->stream>>>(
-        (const unsigned char*)h->x, h->id_base, (const __half*)q, P.cand, P.cnt, n_regions, region_cap, K, exact,
-        D, I, flags);
+        (const unsigned char*)h->x, h->id_base, (const __half*)q, P.cand, P.cnt, P.ov_cnt, n_regions,
+        region_cap, K, exact, D, I, flags);
     h->launches++;
     return cudaGetLastError();
 }

@@ -21,10 +21,8 @@ def _strip(res):
 
 def _answers(eng, queries):
     """search_batch over every (pre-filter, k, fusion) combination, in batches of the orchestrator's
-    fan-out size (4).  From 9 queries a batch takes the tensor-core dense path, whose fp32 band is
-    too wide to separate the candidates of some reference queries against this seeded encoder's
-    2 000-row corpus (LRX_E_AMBIGUOUS with or without an append); that path is not what an append
-    changes."""
+    fan-out size (4).  Larger coalesced batches, which take the tensor-core dense path, are checked
+    on the whole corpus by test_gpu_dense_batched.py."""
     out = {}
     for pf in (True, False):
         eng.dev.set_prefilter(pf)
