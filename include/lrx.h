@@ -306,6 +306,14 @@ int lrx_debug_set_trace(lrx_handle* h, void* dev_int64_128);
 int lrx_debug_bm25_divcheck(lrx_handle* h, double avgdl, double k1, double b, int32_t n_tf,
                             int32_t n_len, uint64_t* host_mismatches);
 
+/* Test hook for K1: the encoder's attention kernel alone, launched as the GEMM chain launches it
+ * (per activation chunk, same grid, block and shared memory).  dev_qkv_fp16 [B*S, 1152] = Q | K | V
+ * per token, head h at columns 32h .. 32h + 31 of each 384-wide block; dev_lens [B] (clamped to
+ * [0, S]); dev_ctx_fp16 [B*S, 384] = softmax(Q K^T / sqrt(32), keys < len) V per head, rows >= len
+ * zero.  1 <= B <= 2^20, 1 <= S <= 512.  Synchronises the handle's stream. */
+int lrx_debug_attention(lrx_handle* h, const void* dev_qkv_fp16, const int32_t* dev_lens, int32_t B,
+                        int32_t S, void* dev_ctx_fp16);
+
 /* Number of kernels launched by this handle since lrx_open (bench.py's gpu_launches). */
 int64_t lrx_launch_count(const lrx_handle* h);
 

@@ -209,6 +209,21 @@ int lrx_debug_bm25_divcheck(lrx_handle* h, double avgdl, double k1, double b, in
     return LRX_OK;
 }
 
+int lrx_debug_attention(lrx_handle* h, const void* dev_qkv_fp16, const int32_t* dev_lens, int32_t B,
+                        int32_t S, void* dev_ctx_fp16) {
+    if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_debug_attention: null handle");
+    if (B < 1 || B > (1 << 20)) return fail(h, LRX_E_ARG, "lrx_debug_attention: B must be in [1, 2^20]");
+    if (S < 1 || S > 512) return fail(h, LRX_E_ARG, "lrx_debug_attention: S must be in [1,512]");
+    if (dev_qkv_fp16 == nullptr || dev_lens == nullptr || dev_ctx_fp16 == nullptr)
+        return fail(h, LRX_E_ARG, "lrx_debug_attention: null pointer");
+    if ((((uintptr_t)dev_qkv_fp16 | (uintptr_t)dev_ctx_fp16) & 15) != 0 || ((uintptr_t)dev_lens & 3) != 0)
+        return fail(h, LRX_E_ARG, "lrx_debug_attention: misaligned pointer");
+    std::lock_guard<std::mutex> g(h->mu);
+    LRX_CUDA(h, cudaSetDevice(h->device));
+    LRX_CUDA(h, encoder_debug_attention(h, dev_qkv_fp16, dev_lens, B, S, dev_ctx_fp16));
+    return LRX_OK;
+}
+
 int64_t lrx_launch_count(const lrx_handle* h) { return h ? h->launches : 0; }
 
 int lrx_profile_enable(lrx_handle* h, int32_t on) {

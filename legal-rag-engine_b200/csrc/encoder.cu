@@ -1166,6 +1166,46 @@ static cudaError_t encoder_forward_small(lrx_handle* h, Encoder* e, const int32_
     return cudaSuccess;
 }
 
+// attention_kernel over nb sequences of S tokens, as the GEMM chain runs it (encoder_forward) and as
+// lrx_debug_attention tests it: one CTA per (head, sequence), K / V of all S padded keys reserved in
+// dynamic shared memory -- 80 KB at S = 512, past the 48 KB default, hence the one-time opt-in.
+static int chunk_sequences(int B, int S) {
+    int n = (int)(kChunkTokens / S);
+    if (n < 1) n = 1;
+    return n > B ? B : n;
+}
+
+static cudaError_t launch_attention(lrx_handle* h, const __half* qkv, const int32_t* lens, int nb, int S,
+                                    __half* ctx) {
+    {
+        std::lock_guard<std::recursive_mutex> attr_guard(attr_mutex());   // the flags below are process-wide
+        static bool attr_dev[64] = {false};   // function attributes are per device
+        bool& attr = attr_dev[h->device & 63];
+        if (!attr) {
+            ENC_CK(cudaFuncSetAttribute(attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        96 * 1024));
+            attr = true;
+        }
+    }
+    const int Sk = (S + 63) & ~63;
+    const size_t smem = (size_t)Sk * kKPad * 2 * 2;
+    ENC_CK(launch_pdl_if(kEncPdlSmall, attention_kernel, dim3(kHeads, nb), dim3(kAttnThreads), smem, h->stream,
+                         qkv, lens, S, ctx));
+    h->launches++;
+    return cudaSuccess;
+}
+
+cudaError_t encoder_debug_attention(lrx_handle* h, const void* qkv, const int32_t* lens, int B, int S, void* ctx) {
+    const int spc = chunk_sequences(B, S);
+    for (int b0 = 0; b0 < B; b0 += spc) {
+        const int nb = (B - b0 < spc) ? (B - b0) : spc;
+        const size_t row0 = (size_t)b0 * S;
+        ENC_CK(launch_attention(h, (const __half*)qkv + row0 * kQkv, lens + b0, nb, S,
+                                (__half*)ctx + row0 * kHidden));
+    }
+    return cudaStreamSynchronize(h->stream);
+}
+
 // Which path.  Sequences of at most 64 tokens in batches of at most 64 groups take the cluster
 // kernel -- its result for a sequence does not depend on the batch, the padded length or the tile
 // variant, so everything a serving front coalesces (serving.py: at most 64 queries per batch)
@@ -1191,23 +1231,13 @@ cudaError_t encoder_forward(lrx_handle* h, const int32_t* ids, const int32_t* le
     const int sp = small_path(B, S);
     if (sp == 2) return encoder_forward_small<2>(h, e, ids, lens, B, S, out_f32, out_f16);
     if (sp == 4) return encoder_forward_small<4>(h, e, ids, lens, B, S, out_f32, out_f16);
-    int seq_per_chunk = (int)(kChunkTokens / S);
-    if (seq_per_chunk < 1) seq_per_chunk = 1;
-    if (seq_per_chunk > B) seq_per_chunk = B;
+    const int seq_per_chunk = chunk_sequences(B, S);
     if ((int64_t)seq_per_chunk * S > e->cap) {
         // the activation workspace moves: not inside a capture, and captured chains are retired
         if (h->capturing) return cudaErrorStreamCaptureUnsupported;
         h->ws_epoch++;
     }
     ENC_CK(encoder_reserve(e, (int64_t)seq_per_chunk * S));
-    std::lock_guard<std::recursive_mutex> attr_guard(attr_mutex());   // the flags below are process-wide
-    static bool attr_dev[64] = {false};   // function attributes are per device
-    bool& attr = attr_dev[h->device & 63];
-    if (!attr) {
-        ENC_CK(cudaFuncSetAttribute(attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    96 * 1024));
-        attr = true;
-    }
     cudaStream_t st = h->stream;
     for (int b0 = 0; b0 < B; b0 += seq_per_chunk) {
         const int nb = (B - b0 < seq_per_chunk) ? (B - b0) : seq_per_chunk;
@@ -1218,17 +1248,13 @@ cudaError_t encoder_forward(lrx_handle* h, const int32_t* ids, const int32_t* le
                           e->max_pos, (const float*)e->word, (const float*)e->pos, (const float*)e->type0,
                           (const float*)e->eln_g, (const float*)e->eln_b, e->x));
         h->launches++;
-        const int Sk = (S + 63) & ~63;
-        const size_t attn_smem = (size_t)Sk * kKPad * 2 * 2;
         // which W tensor-map set matches the plan the GEMM launcher picks for this many rows
         const int pl = ((int)((T + 127) / 128) >= h->num_sms / 2) ? 1 : 0;
         for (int l = 0; l < kLayers; ++l) {
             EncLayer& L = e->L[l];
             ENC_CK(launch_tc_gemm(h, e->t_x, L.t_wqkv[pl], e->io_qkv, e->io_qkv, (int)T, kQkv, kHidden, 0,
                                   L.bqkv, nullptr, nullptr, 0.f, e->qkv, kQkv));
-            ENC_CK(launch_pdl_if(kEncPdlSmall, attention_kernel, dim3(kHeads, nb), dim3(kAttnThreads), attn_smem, st,
-                              (const __half*)e->qkv, clen, S, e->ctx));
-            h->launches++;
+            ENC_CK(launch_attention(h, e->qkv, clen, nb, S, e->ctx));
             ENC_CK(launch_tc_gemm(h, e->t_ctx, L.t_wo[pl], e->io_x1, e->io_x, (int)T, kHidden, kHidden, 2,
                                   L.bo, L.ln1_g, L.ln1_b, kLnEps, e->x1, kHidden));
             ENC_CK(launch_tc_gemm(h, e->t_x1, L.t_w1[pl], e->io_ff, e->io_ff, (int)T, kFfn, kHidden, 1,

@@ -190,6 +190,9 @@ cudaError_t encoder_forward(lrx_handle* h, const int32_t* ids, const int32_t* le
 cudaError_t encoder_forward_host(lrx_handle* h, const int32_t* host_ids, const int32_t* host_lens,
                                  int B, int S, float* host_out);
 void encoder_free(lrx_handle* h);
+// attention_kernel alone on qkv [B*S, 1152] -> ctx [B*S, 384], launched per chunk as encoder_forward
+// launches it (lrx_debug_attention); synchronises the handle's stream
+cudaError_t encoder_debug_attention(lrx_handle* h, const void* qkv, const int32_t* lens, int B, int S, void* ctx);
 // tc_gemm.cu
 cudaError_t gemm_f16_adhoc(lrx_handle* h, const void* a, const void* w, int M, int N, int K, int epi,
                            const float* bias, const void* residual, const float* gamma,

@@ -4,20 +4,22 @@
 // (reference: src/retrieval/retrieval_engine.py:61, create_vector_store.py:45): the six
 // BertLayer projections of all-MiniLM-L6-v2.  fp16 operands, fp32 accumulation in TMEM.
 //
-// One CTA = one 128 x BN output tile, 192 threads, warp-specialised:
-//   warp 4   TMA producer: 2-D tiled loads (SWIZZLE_128B) of the A tile (128 x 64 halves)
-//            and the W tile (BN x 64 halves) into a 3-stage shared-memory ring, completion
-//            counted on full[] mbarriers, slots recycled through empty[] mbarriers.
-//   warp 5   allocates TMEM and issues tcgen05.mma (UMMA 128 x N x 16, cta_group::1) from ONE
+// Persistent CTAs, each walking 128 x BN output tiles, 320 threads (kGemmThreads), warp-specialised:
+//   warp 8   TMA producer: 2-D tiled loads (SWIZZLE_128B) of the A tile (128 x 64 halves)
+//            and the W tile (BN x 64 halves) into a shared-memory ring (GemmCfg::kStages deep),
+//            completion counted on full[] mbarriers, slots recycled through empty[] mbarriers;
+//            for K = 384 on the big plans the CTA's A tile stays resident (ARES) and clusters
+//            of 2 multicast W (CS).
+//   warp 9   allocates TMEM and issues tcgen05.mma (UMMA 128 x N x 16, cta_group::1) from ONE
 //            lane: 4 k-steps per stage; tcgen05.commit releases the stage / publishes the
 //            accumulator.
-//   warps 0-3 epilogue: thread r owns output row r (= TMEM lane r): tcgen05.ld 32 columns at
-//            a time, then
+//   warps 0-7 epilogue (kEpiWarps): thread = output row (TMEM lane 32 (warp & 3) + lane) x column
+//            half (warp >> 2): tcgen05.ld 32 columns at a time, then
 //              EPI_BIAS        + bias                              -> fp16   (QKV projection)
-//              EPI_BIAS_GELU   + bias, exact-erf GELU              -> fp16   (FFN up)
+//              EPI_BIAS_GELU   + bias, GELU (fitted tanh form)     -> fp16   (FFN up)
 //              EPI_BIAS_RES_LN + bias + residual, LayerNorm(384)   -> fp16   (attention output /
-//                              FFN down; BN = 384 = the whole row, so mean/variance are
-//                              per-thread sums; the pre-norm row is parked in TMEM between
+//                              FFN down; BN = 384 = the whole row, each half's sums meet in
+//                              shared memory; the pre-norm row is parked in TMEM between
 //                              the three passes with tcgen05.st)
 //              EPI_F32         raw fp32 accumulators                         (tests / K2b)
 //

@@ -17,6 +17,11 @@ published modules:
   Normalize          F.normalize(p=2, dim=1)  = x / max(||x||, 1e-12)
   faiss.normalize_L2 x *= 1 / sqrt(sum x^2)   (rows with zero norm untouched)
 
+``dtype`` / ``device`` (keywords of the three entry points): the defaults, float32 on the CPU, are
+the restatement the golden file pins; ``dtype=torch.float64, device="cuda"`` runs the same
+arithmetic in double precision on a GPU -- the reference the kernel tests measure error against
+when thousands of rows are needed (the faiss step is then float64 as well).
+
 PINNED against HuggingFace ``transformers.BertModel`` (installed in the build
 container) by ``tests/golden/make_encoder_golden.py``: the golden file holds BertModel's
 own outputs for seeded weights; ``tests/test_oracle_encoder.py`` checks this restatement
@@ -34,10 +39,10 @@ HIDDEN, HEADS, HEAD_DIM, FFN, LAYERS = 384, 12, 32, 1536, 6
 LN_EPS = 1e-12
 
 
-def _t(a) -> torch.Tensor:
+def _t(a, dtype=torch.float32, device="cpu") -> torch.Tensor:
     if isinstance(a, torch.Tensor):
-        return a.detach().to(torch.float32).cpu()
-    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
+        return a.detach().to(device=device, dtype=dtype)
+    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)).to(device=device, dtype=dtype)
 
 
 def _layer_norm(x, g, b):
@@ -46,18 +51,19 @@ def _layer_norm(x, g, b):
     return (x - mean) / torch.sqrt(var + LN_EPS) * g + b
 
 
-def bert_hidden(sd: Dict[str, np.ndarray], ids: np.ndarray, mask: np.ndarray) -> torch.Tensor:
-    """Last hidden state [B,S,384] (float32) of the 6-layer BertModel without pooler.
-    ``sd``: HuggingFace state_dict names -> arrays; ``ids``/``mask``: int [B,S]."""
-    w = {k: _t(v) for k, v in sd.items()}
-    ids_t = torch.from_numpy(np.asarray(ids, dtype=np.int64))
-    mask_t = torch.from_numpy(np.asarray(mask, dtype=np.int64))
+def bert_hidden(sd: Dict[str, np.ndarray], ids: np.ndarray, mask: np.ndarray, *,
+                dtype=torch.float32, device="cpu") -> torch.Tensor:
+    """Last hidden state [B,S,384] (``dtype``, on ``device``) of the 6-layer BertModel without
+    pooler.  ``sd``: HuggingFace state_dict names -> arrays; ``ids``/``mask``: int [B,S]."""
+    w = {k: _t(v, dtype, device) for k, v in sd.items()}
+    ids_t = torch.from_numpy(np.asarray(ids, dtype=np.int64)).to(device)
+    mask_t = torch.from_numpy(np.asarray(mask, dtype=np.int64)).to(device)
     B, S = ids_t.shape
     x = (w["embeddings.word_embeddings.weight"][ids_t]
-         + w["embeddings.position_embeddings.weight"][torch.arange(S)][None]
+         + w["embeddings.position_embeddings.weight"][torch.arange(S, device=device)][None]
          + w["embeddings.token_type_embeddings.weight"][0][None, None])
     x = _layer_norm(x, w["embeddings.LayerNorm.weight"], w["embeddings.LayerNorm.bias"])
-    ext = (1.0 - mask_t[:, None, None, :].to(torch.float32)) * torch.finfo(torch.float32).min
+    ext = (1.0 - mask_t[:, None, None, :].to(dtype)) * torch.finfo(dtype).min
     for l in range(LAYERS):
         p = f"encoder.layer.{l}."
         lin = lambda t, name: t @ w[p + name + ".weight"].T + w[p + name + ".bias"]
@@ -78,20 +84,24 @@ def bert_hidden(sd: Dict[str, np.ndarray], ids: np.ndarray, mask: np.ndarray) ->
     return x
 
 
-def pool_normalize(hidden: torch.Tensor, mask: np.ndarray) -> np.ndarray:
-    """sentence-transformers Pooling(mean) + Normalize, then faiss.normalize_L2."""
-    m = torch.from_numpy(np.asarray(mask, dtype=np.int64)).to(torch.float32)[:, :, None]
+def pool_normalize(hidden: torch.Tensor, mask: np.ndarray, *, dtype=torch.float32) -> np.ndarray:
+    """sentence-transformers Pooling(mean) + Normalize, then faiss.normalize_L2; ``dtype`` [B,384]
+    numpy rows (faiss's own step is float32; with ``dtype=torch.float64`` it is float64 too)."""
+    m = torch.from_numpy(np.asarray(mask, dtype=np.int64)).to(device=hidden.device, dtype=dtype)[:, :, None]
+    hidden = hidden.to(dtype)
     emb = (hidden * m).sum(1) / torch.clamp(m.sum(1), min=1e-9)
     emb = emb / torch.clamp(emb.norm(dim=1, keepdim=True), min=1e-12)
-    out = emb.numpy().astype(np.float32)
-    n2 = (out.astype(np.float32) ** 2).sum(axis=1, dtype=np.float32)     # fvec_norm_L2sqr
+    npt = np.float64 if dtype == torch.float64 else np.float32
+    out = emb.cpu().numpy().astype(npt)
+    n2 = (out ** 2).sum(axis=1, dtype=npt)                                 # fvec_norm_L2sqr
     nz = n2 > 0
-    out[nz] *= (np.float32(1.0) / np.sqrt(n2[nz]))[:, None]
+    out[nz] *= (npt(1.0) / np.sqrt(n2[nz]))[:, None]
     return out
 
 
-def encode_ids(sd, ids: np.ndarray, lens: np.ndarray) -> np.ndarray:
-    """float32 [B,384] unit embeddings for 0-padded id rows with prefix masks of length ``lens``."""
+def encode_ids(sd, ids: np.ndarray, lens: np.ndarray, *, dtype=torch.float32, device="cpu") -> np.ndarray:
+    """[B,384] unit embeddings (float32, or float64 with ``dtype=torch.float64``) for 0-padded id
+    rows with prefix masks of length ``lens``."""
     ids = np.asarray(ids)
     mask = (np.arange(ids.shape[1])[None, :] < np.asarray(lens)[:, None]).astype(np.int64)
-    return pool_normalize(bert_hidden(sd, ids, mask), mask)
+    return pool_normalize(bert_hidden(sd, ids, mask, dtype=dtype, device=device), mask, dtype=dtype)

@@ -39,6 +39,31 @@ def test_pool_normalize_unit_and_masked():
     np.testing.assert_allclose(e[2], want / np.linalg.norm(want), atol=1e-6)
 
 
+@pytest.mark.parametrize("case", [0, 1])
+def test_float64_oracle_agrees_with_float32_on_golden_inputs(case):
+    """The float64 restatement (the reference of the encoder kernel tests) is the same function as
+    the float32 one the golden file pins: embeddings within float32 rounding of each other, unit
+    norm to double precision, and the len = 0 row stays the zero vector in both."""
+    import torch
+    g = np.load(GOLDEN / "encoder_golden.npz")
+    wseed, std, jit, b, s, tseed = g[f"case_{case}"]
+    sd = synth.bert_state_dict(int(wseed), float(std), ln_jitter=float(jit))
+    ids, lens = synth.token_batch(int(b), int(s), int(tseed))
+    ids = np.concatenate([ids, ids[:1]])
+    lens = np.concatenate([lens, [0]])                     # a fully masked row
+    e32 = oenc.encode_ids(sd, ids, lens)
+    e64 = oenc.encode_ids(sd, ids, lens, dtype=torch.float64)
+    assert e32.dtype == np.float32 and e64.dtype == np.float64
+    np.testing.assert_allclose(e64[:-1], e32[:-1].astype(np.float64), rtol=0, atol=1e-5)
+    np.testing.assert_allclose(np.linalg.norm(e64[:-1], axis=1), 1.0, rtol=0, atol=1e-12)
+    assert not e32[-1].any() and not e64[-1].any()
+    mask = (np.arange(int(s))[None] < lens[:, None]).astype(np.int64)
+    h64 = oenc.bert_hidden(sd, ids, mask, dtype=torch.float64)
+    assert h64.dtype == torch.float64
+    valid = mask.astype(bool)
+    np.testing.assert_allclose(h64.numpy()[valid], g[f"hidden_{case}"][valid[:-1]], rtol=0, atol=2e-5)
+
+
 def test_tokenizers():
     assert basic_tokenize("What is the procedure for Zero FIR?") == \
         ["what", "is", "the", "procedure", "for", "zero", "fir", "?"]
