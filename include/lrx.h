@@ -296,10 +296,6 @@ int lrx_search_text_host(lrx_handle* h, const int32_t* host_tok_ids, const int32
                          const double* host_weights, int32_t B, int32_t k, int32_t mode,
                          int64_t* host_ids, double* host_score, double* host_sem, double* host_kw);
 
-/* Kernel-tuning aid: when set (device int64[128], caller-owned; NULL to clear), CTA 0 of every
- * tensor-core GEMM launch writes clock64() stamps of its pipeline events there. */
-int lrx_debug_set_trace(lrx_handle* h, void* dev_int64_128);
-
 /* Test hook for K3: the scan divides with the branch-free fast path of the float64 division
  * (same FMA sequence as the compiler's, without the exponent-range test); this counts the
  * (tf, len) pairs in [0,n_tf) x [0,n_len) whose BM25 factor differs from the IEEE division. */

@@ -99,7 +99,6 @@ _SIGNATURES = {
                                         _vp]),
     "lrx_search_text_host": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp,
                                        _vp, _vp]),
-    "lrx_debug_set_trace": (C.c_int, [_vp, _vp]),
     "lrx_debug_bm25_divcheck": (C.c_int, [_vp, _f64, _f64, _f64, _i32, _i32, C.POINTER(C.c_uint64)]),
     "lrx_debug_attention": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _vp]),
     "lrx_launch_count": (_i64, [_vp]),

@@ -134,14 +134,10 @@ int lrx_open(const lrx_config* cfg, lrx_handle** out) {
     // The side stream carries the BM25 chain (bounds -> scan -> merge), the longer of the two chains of
     // a batch since the int8 dense scan: it gets the high stream priority, so that its CTAs are placed
     // first when SM slots free up (profiles/r2_runs/ab_aux_stream_priority.txt: two users per chain + 4 %,
-    // latency of one batch at 10 M rows 0.86 -> 0.80 ms).  LRX_AUX_PRIO=none / low: A/B switch.
+    // latency of one batch at 10 M rows 0.86 -> 0.80 ms).
     int prio_lo = 0, prio_hi = 0;
     cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
-    int aux_prio = prio_hi;
-    const char* ap = getenv("LRX_AUX_PRIO");
-    if (ap != nullptr && ap[0] == 'n') aux_prio = 0;
-    else if (ap != nullptr && ap[0] == 'l') aux_prio = prio_lo;
-    if (cudaStreamCreateWithPriority(&h->aux, cudaStreamNonBlocking, aux_prio) != cudaSuccess ||
+    if (cudaStreamCreateWithPriority(&h->aux, cudaStreamNonBlocking, prio_hi) != cudaSuccess ||
         cudaStreamCreateWithFlags(&h->cap, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming) != cudaSuccess ||
@@ -150,8 +146,6 @@ int lrx_open(const lrx_config* cfg, lrx_handle** out) {
         delete h;
         return fail(nullptr, LRX_E_CUDA, "lrx_open: cannot create side stream / events");
     }
-    const char* ng = getenv("LRX_NO_GRAPH");
-    h->graphs = !(ng != nullptr && ng[0] != '\0' && ng[0] != '0');
     *out = h;
     return LRX_OK;
 }
@@ -186,13 +180,6 @@ int lrx_set_stream(lrx_handle* h, void* cuda_stream) {
     if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_set_stream: null handle");
     std::lock_guard<std::mutex> g(h->mu);
     h->stream = (cudaStream_t)cuda_stream;
-    return LRX_OK;
-}
-
-int lrx_debug_set_trace(lrx_handle* h, void* dev_int64_128) {
-    if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_debug_set_trace: null handle");
-    std::lock_guard<std::mutex> g(h->mu);
-    h->debug_trace = dev_int64_128;
     return LRX_OK;
 }
 
@@ -522,28 +509,11 @@ int lrx_gemm_f16(lrx_handle* h, const void* dev_a, const void* dev_w, int32_t M,
 // ceil(B / 8) -- measured at 10 M rows: B = 64 1.32 ms against 18.1 ms (tools/k2_crossover.py); both
 // emit the same exact lists.  A widened retry (exactness guard / candidate overflow) runs K2a at
 // that width: width is K2a's parameter, and K2b flags only a query with more than 1024 rows near its
-// K-th score, which K2b at any stride would flag again.  LRX_K2B_MIN_B overrides the crossover (A/B
-// runs).
-static int k2b_min_b() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("LRX_K2B_MIN_B");
-        v = (e != nullptr && atoi(e) > 0) ? atoi(e) : 9;
-    }
-    return v;
-}
-// LRX_BM_CHAIN_CTAS: BM25 scan CTAs per SM inside the search chain (1 = what fits beside the dense scan; 2 = as alone)
-static int bm_chain_ctas() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("LRX_BM_CHAIN_CTAS");
-        v = (e != nullptr && atoi(e) == 2) ? 2 : 1;
-    }
-    return v;
-}
+// K-th score, which K2b at any stride would flag again.
+constexpr int kK2bMinB = 9;
 static cudaError_t launch_dense_auto(lrx_handle* h, const void* q, int B, int K, int width, double* exact,
                                      float* D, int64_t* I, int32_t* flags) {
-    if (B >= k2b_min_b() && h->n_local > 0 && ((uintptr_t)q & 15) == 0 && width <= dense_default_width(K))
+    if (B >= kK2bMinB && h->n_local > 0 && ((uintptr_t)q & 15) == 0 && width <= dense_default_width(K))
         return launch_dense_topk_batched(h, q, B, K, 0, exact, D, I, flags);
     return launch_dense_topk(h, q, B, K, width, exact, D, I, flags);
 }
@@ -714,8 +684,7 @@ static int enqueue_search(lrx_handle* h, const LocalScratch& s, const void* q, c
     h->bm_list_k = Kb;
     // K2a's CTA shares the SM (profiles/r2_runs/ab_bm25_chain_ctas.txt; 5..8 queries on a small shard keep
     // the second wave: there the BM25 scan outlasts the dense scan by far and the wave does real work)
-    h->bm_ctas_per_sm = (B < k2b_min_b() && h->n_local > 0 && (B <= 4 || h->n_local >= (4ll << 20)))
-                            ? bm_chain_ctas() : 0;
+    h->bm_ctas_per_sm = (B < kK2bMinB && h->n_local > 0 && (B <= 4 || h->n_local >= (4ll << 20))) ? 1 : 0;
     LRX_CUDA(h, cudaEventRecord(h->ev_fork, h->stream));
     LRX_CUDA(h, cudaStreamWaitEvent(h->aux, h->ev_fork, 0));
     LRX_CUDA(h, launch_dense_auto(h, q, B, K, width, s.dense_exact, s.dense_D, s.dense_I, s.flags));
@@ -744,7 +713,6 @@ static bool key_in(const std::vector<std::vector<uint64_t>>& set, const std::vec
 // captured stays on the direct path.
 template <typename F>
 static int run_planned(lrx_handle* h, std::vector<uint64_t> key, F&& enqueue) {
-    if (!h->graphs) return enqueue();
     key.push_back(h->prof ? 1u : 0u);
     for (size_t i = 0; i < h->plans.size(); ++i) {
         lrx_plan* pl = h->plans[i];

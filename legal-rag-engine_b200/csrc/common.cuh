@@ -51,16 +51,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
         if (++spins > (1u << 24)) __trap();   // each failed try_wait already sleeps in HW
     }
 }
-// 1-D bulk async copy global -> shared (TMA engine, no tensor map), completion
-// counted in bytes on an mbarrier.  dst/src 16-byte aligned, bytes % 16 == 0.
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes,
-                                         uint64_t* bar) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-        ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar))
-        : "memory");
-}
-
 // Programmatic dependent launch: a kernel launched with launch_pdl() (handle.h) may start while
 // its predecessor in the stream still runs; pdl_wait() blocks until the predecessor grid has
 // completed and its memory is visible (a no-op under a normal launch), pdl_trigger() lets the
@@ -68,8 +58,10 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-// Same with an L2 eviction-priority hint: a stream that is read once should not push the small
-// structures other kernels keep re-reading (tables, bounds, thresholds) out of L2.
+// 1-D bulk async copy global -> shared (TMA engine, no tensor map), completion counted in bytes on
+// an mbarrier, dst/src 16-byte aligned, bytes % 16 == 0; with an L2 eviction-priority hint: a stream
+// that is read once should not push the small structures other kernels keep re-reading (tables,
+// bounds, thresholds) out of L2.
 __device__ __forceinline__ uint64_t l2_policy_evict_first() {
     uint64_t p;
     asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));

@@ -36,11 +36,8 @@ namespace lrx {
 constexpr int kScanThreads = 256;                  // 8 warps: the SM is shared with a BM25 scan CTA
 constexpr int kTileRows = 64;                      // 4 rows per warp per tile
 constexpr int kTileBytes = kTileRows * kRowBytes;  // 49152
-#ifndef LRX_SCAN_STAGES
-#define LRX_SCAN_STAGES 2                          // 2, 3 and 4 measure the same (tools/scan_sweep.sh);
-                                                   // 2 leaves shared memory for a co-resident BM25 CTA
-#endif
-constexpr int kStages = LRX_SCAN_STAGES;
+constexpr int kStages = 2;                         // 2, 3 and 4 measure the same; 2 leaves shared
+                                                   // memory for a co-resident BM25 CTA
 constexpr int kCap = 1024;                         // candidate buffer entries per query
 constexpr int kSoftCap = 256;                      // prune once a buffer holds more than this minus a
                                                    // tile: sorting 256 keys costs ~3 us, 1024 keys ~40 us,
@@ -234,10 +231,7 @@ __global__ void __launch_bounds__(kScanThreads, 2)          // <= 128 registers:
 dense_scan_kernel(const unsigned char* __restrict__ x, int64_t n_rows,
                   const __half* __restrict__ q, int n_q, int width,
                   uint64_t* __restrict__ part /* [grid][NQ][width] */,
-                  unsigned int* __restrict__ tau_g /* [4] shared thresholds, zero at launch */,
-                  long long* __restrict__ trace /* optional clock64 stamps of CTA 0, or NULL */) {
-#define SCAN_TRACE(slot) do { if (trace != nullptr && blockIdx.x == 0 && threadIdx.x == 0) trace[(slot)] = clock64(); } while (0)
-    SCAN_TRACE(0);
+                  unsigned int* __restrict__ tau_g /* [4] shared thresholds, zero at launch */) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     ScanSmem& sm = *reinterpret_cast<ScanSmem*>(smem_raw);
     uint64_t* keys = sm.keys;
@@ -250,7 +244,7 @@ dense_scan_kernel(const unsigned char* __restrict__ x, int64_t n_rows,
     constexpr int cap = scan_cap(NQ);
     const int soft_cap = (2 * width <= kSoftCap) ? kSoftCap : cap;
     // Tiles are static, blockIdx + i * grid: at any moment the grid reads one contiguous ~7 MB
-    // window of the matrix.  (Measured, tools/scan_sweep.sh: claiming tiles from a grid-wide counter
+    // window of the matrix.  (Measured: claiming tiles from a grid-wide counter
     // costs 25 % -- one contended atomic per 48 KB -- and re-filling a stage BEFORE the tile's
     // per-row tests instead of after the closing barrier costs 30 %; 32-row tiles cost 50 %; a
     // variant without the k split -- 8 rows per warp over the whole k, half of each MMA redundant,
@@ -275,11 +269,7 @@ dense_scan_kernel(const unsigned char* __restrict__ x, int64_t n_rows,
         const int rows = (int)min((int64_t)kTileRows, n_rows - row0);
         const uint32_t bytes = (uint32_t)rows * kRowBytes;
         mbar_arrive_expect_tx(&sm.full[s], bytes);
-#ifdef LRX_SCAN_NO_HINT
-        bulk_g2s(sm.ring[s], x + row0 * kRowBytes, bytes, &sm.full[s]);
-#else
         bulk_g2s_hint(sm.ring[s], x + row0 * kRowBytes, bytes, &sm.full[s], l2_policy_evict_first());
-#endif
     };
     int next_tile = (int)blockIdx.x + kStages * (int)gridDim.x;   // thread 0: the next tile to load
     if (tid == 0) {
@@ -305,9 +295,7 @@ dense_scan_kernel(const unsigned char* __restrict__ x, int64_t n_rows,
     }
     const uint32_t a_off = (uint32_t)((mblk * 16 + g) * kRowBytes + (6 * kh) * 64 + 16 * t);
 
-    SCAN_TRACE(1);
     for (int it = 0;; ++it) {
-        if (it < 20 || (it & 15) == 0) SCAN_TRACE(8 + (it < 20 ? it : min(99, 20 + (it >> 4))));
         const int s = it % kStages;
         const uint32_t parity = (uint32_t)((it / kStages) & 1);
         const int tile = sm.tile_of[s];
@@ -384,7 +372,6 @@ dense_scan_kernel(const unsigned char* __restrict__ x, int64_t n_rows,
 
     // ---- final: sorted per-CTA lists out
     __syncthreads();
-    SCAN_TRACE(2);
     scan_prune<NQ>(keys, sm.count, sm.tau, width, tid, tau_g);
     for (int i = tid; i < NQ * width; i += kScanThreads) {
         const int qi = i / width;
@@ -392,8 +379,6 @@ dense_scan_kernel(const unsigned char* __restrict__ x, int64_t n_rows,
         const uint64_t k = (j < sm.count[qi]) ? keys[qi * cap + j] : 0ull;
         part[((size_t)blockIdx.x * NQ + qi) * width + j] = k;
     }
-    SCAN_TRACE(3);
-#undef SCAN_TRACE
 }
 
 // ---------------------------------------------------------------------------
@@ -920,7 +905,7 @@ static cudaError_t launch_scan(lrx_handle* h, const __half* q, int n_q, int widt
     if (e0 != cudaSuccess) return e0;
     prof_begin(h, 0);
     dense_scan_kernel<NQ><<<grid, kScanThreads, smem, h->stream>>>(
-        (const unsigned char*)h->x, h->n_local, q, n_q, width, part, tau_g, (long long*)h->debug_trace);
+        (const unsigned char*)h->x, h->n_local, q, n_q, width, part, tau_g);
     prof_end(h, 0);
     h->launches++;
     return cudaGetLastError();

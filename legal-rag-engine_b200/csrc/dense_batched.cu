@@ -199,9 +199,6 @@ dense_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant
         const uint32_t trow = tmem_base + ((uint32_t)(quarter * 32) << 16) + half * HB;
         float thr = 0.f;
         if (PASS == 2) thr = q_ok ? P.thr[q] : FLT_MAX;
-#ifdef LRX_DB_NOHIT
-        thr = FLT_MAX;                                       // timing experiment: no candidate ever
-#endif
         uint32_t rb[2][32];
         const int region = group * 2 + half;
         int my_cnt = 0;                                      // candidates of (q, region) so far

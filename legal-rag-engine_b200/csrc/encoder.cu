@@ -451,7 +451,6 @@ struct SmallParams {
     const float *word, *pos, *type0, *eln_g, *eln_b;
     SmallLayer L[kLayers];
     unsigned char* scratch;             // [groups][SmGeom::scratch]
-    long long* trace;                   // optional timeline of cluster 0 / CTA 0 (lrx_debug_set_trace), else NULL
     float* out_f32;
     __half* out_f16;
 };
@@ -700,11 +699,6 @@ encoder_small_kernel(const SmallParams P) {
     const int ng = c * 4 + (warp >> 1);                      // its column group in the cluster, 0..31
     SmB Bf;                                                  // B fragments in flight
     float acc[MW][kSmNu][4];
-    int tr_n = 0;
-    auto stamp = [&]() {
-        if (P.trace != nullptr && blockIdx.x == 0 && tid == 0 && tr_n < 128) P.trace[tr_n++] = clock64();
-    };
-    stamp();
     // column tiles (of 8) per phase: QKV 144 = 16 groups x 5 + 16 x 4; output projection 48 = 16 x 2 +
     // 16 x 1; FFN up 192 = 32 x 6; FFN down: CTA c owns k quarter c & 3 of tiles (c >> 2) * 24 .. + 24
     const int qkv_t0 = ng < 16 ? 5 * ng : 80 + 4 * (ng - 16), qkv_nu = ng < 16 ? 5 : 4;
@@ -744,7 +738,6 @@ encoder_small_kernel(const SmallParams P) {
         sm_ln_row(v, P.eln_g, P.eln_b, xrow, lane);
     }
     __syncthreads();
-    stamp();
 
     for (int l = 0; l < kLayers; ++l) {
         const SmallLayer& L = P.L[l];
@@ -768,9 +761,7 @@ encoder_small_kernel(const SmallParams P) {
         // the output projection's first weights travel under the attention (32-row groups; with 64
         // rows the attention needs the registers)
         if (MT == 2) sm_b_prefetch(Bf, w_lane(L.wo, out_t0, kHidden, 0), kHidden, out_nu);
-        stamp();
         cluster_sync_all();
-        stamp();
         // ---- (2) attention: (sequence, head) pairs over kSmAttnWarps warps per CTA
         if (warp < kSmAttnWarps) {
             __half* sK = as + (size_t)warp * (2 * 16 * MT * kKPad);
@@ -782,9 +773,7 @@ encoder_small_kernel(const SmallParams P) {
                 sm_attention_pair<MT>(s_qkv, sq * P.S, head, P.S, len, sK, sV, s_ctx, lane);
             }
         }
-        stamp();
         cluster_sync_all();
-        stamp();
         // ---- (3) output projection + residual -> scratch y (fp32); A = ctx staged from the scratch
         for (int i = tid; i < M * 48; i += kSmThreads) {
             const int r = i / 48, part = i - r * 48;
@@ -816,9 +805,7 @@ encoder_small_kernel(const SmallParams P) {
         }
         // FFN up's first weights travel under the barrier + LayerNorm
         sm_b_prefetch(Bf, w_lane(L.w1, up_t0, kHidden, 0), kHidden, 6);
-        stamp();
         cluster_sync_all();
-        stamp();
         // ---- (4) LayerNorm 1 (every CTA, all rows; the loads of four rows in flight together) -> X;
         //          FFN up + GELU -> scratch ff (fp16)
 #pragma unroll 1
@@ -853,9 +840,7 @@ encoder_small_kernel(const SmallParams P) {
             }
         }
         sm_b_prefetch(Bf, w_lane(L.w2, dn_t0, kFfn, kq * kHidden), kFfn, 6);
-        stamp();
         cluster_sync_all();
-        stamp();
         // ---- (5) FFN down: partial sums over this CTA's k quarter -> scratch ypart[kq] (fp32)
         for (int i = tid; i < M * 48; i += kSmThreads) {
             const int r = i / 48, part = i - r * 48;
@@ -881,9 +866,7 @@ encoder_small_kernel(const SmallParams P) {
                 }
             }
         }
-        stamp();
         cluster_sync_all();
-        stamp();
         // ---- (6) the four k quarters in order + bias + residual, LayerNorm 2 -> X (two rows' loads
         //          in flight together)
 #pragma unroll 1
@@ -916,7 +899,6 @@ encoder_small_kernel(const SmallParams P) {
         }
         if (l + 1 < kLayers) sm_b_prefetch(Bf, w_lane(P.L[l + 1].wqkv, qkv_t0, kHidden, 0), kHidden, qkv_nu);
         __syncthreads();
-        stamp();
     }
 
     // ---- pooling + Normalize + normalize_L2: sequence i of the group on CTA i % 8
@@ -1140,7 +1122,6 @@ static cudaError_t encoder_forward_small(lrx_handle* h, Encoder* e, const int32_
         d.ln1_g = s.ln1_g; d.ln1_b = s.ln1_b; d.ln2_g = s.ln2_g; d.ln2_b = s.ln2_b;
     }
     P.scratch = (unsigned char*)e->small_ws;
-    P.trace = (long long*)h->debug_trace;
     for (int g0 = 0; g0 < groups_all; g0 += groups_max) {
         const int ng = (groups_all - g0) < groups_max ? (groups_all - g0) : groups_max;
         const int b0 = g0 * spg;
@@ -1214,9 +1195,8 @@ cudaError_t encoder_debug_attention(lrx_handle* h, const void* qkv, const int32_
 // sequences are packed into 64-row groups (0.26 ms per wave; from about 30 groups on the chain
 // would be faster -- 0.4 ms for 64 x 32 tokens against 0.74 -- which is the price of the invariance).
 // 0: chain, 2 / 4: cluster kernel with 32- / 64-row groups.
-// LRX_NO_SMALL_ENCODER=1 forces the chain (A/B runs, tests).
 static int small_path(int B, int S) {
-    if (S > 64 || getenv("LRX_NO_SMALL_ENCODER") != nullptr) return 0;
+    if (S > 64) return 0;
     if (S <= 32) {
         const int spg = 32 / S;
         if ((B + spg - 1) / spg <= 14) return 2;

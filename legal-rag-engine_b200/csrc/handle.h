@@ -97,7 +97,6 @@ struct lrx_handle {
     unsigned int* pack_done = nullptr;   // device counter of pack_exchange_kernel (last CTA done)
 
     // captured launch chains (api.cu: run_planned)
-    bool graphs = true;                  // LRX_NO_GRAPH=1 -> every call enqueues its kernels one by one
     bool capturing = false;
     lrx_plan* cap_plan = nullptr;
     cudaStream_t cap = nullptr;          // capture origin (the user's stream may be the legacy default one)
@@ -109,7 +108,6 @@ struct lrx_handle {
 
     // K1 encoder state (packed weights, activation workspaces, tensor maps): encoder.cu
     void* encoder = nullptr;
-    void* debug_trace = nullptr;     // device int64[128]: GEMM timeline of CTA 0 (lrx_debug_set_trace)
 };
 
 namespace lrx {

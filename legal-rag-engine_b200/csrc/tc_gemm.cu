@@ -31,10 +31,8 @@
 
 namespace lrx {
 
-#ifndef LRX_GEMM_CLUSTER
-#define LRX_GEMM_CLUSTER 2
-#endif
 constexpr int kBM = 128;
+constexpr int kGemmCluster = 2;                   // cluster size along M when clusters apply (gemm_plan)
 constexpr int kBK = 64;
 constexpr int kEpiWarps = 8;                      // two per TMEM lane quarter: column halves
 constexpr int kGemmThreads = (kEpiWarps + 2) * 32;   // + TMA producer warp + MMA warp
@@ -49,7 +47,6 @@ struct GemmEpi {
     int ld_out, ld_res;
     int M;                    // valid rows
     float eps;
-    long long* trace;         // optional timeline of CTA 0 (lrx_debug_set_trace), else NULL
     int pdl_early;            // let the next kernel be scheduled at this kernel's start (else at its end)
 };
 
@@ -154,8 +151,6 @@ __device__ __forceinline__ void stage_acquire1(int lane) {
 // Persistent: CTA c owns output tiles c, c + grid, ... (n-block fastest, so CTAs running side by
 // side share the A rows in L2).  The shared-memory ring flows across tiles; with two TMEM
 // accumulators (BN <= 256) the epilogue of tile i overlaps the MMAs of tile i + 1.
-#define LRX_TRACE(slot) do { if (ep.trace != nullptr && blockIdx.x == 0) ep.trace[(slot)] = clock64(); } while (0)
-
 template <int BN, int EPI, bool ARES, int CS>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
@@ -192,7 +187,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
     const int total_tiles = m_tiles * n_tiles;
     constexpr int kProducerWarp = kEpiWarps, kMmaWarp = kEpiWarps + 1;
 
-    if (threadIdx.x == 0) LRX_TRACE(0);
     // Programmatic dependent launch: from the trigger on, CTAs of the next kernel of the stream may
     // take an SM as soon as one is free, run their prologue and wait.  A grid that leaves SMs idle
     // (fewer row blocks than SMs) triggers at once -- 0.566 -> 0.521 ms for 64 sequences of 128
@@ -226,7 +220,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     pdl_wait();                                // the previous kernel's outputs are complete and visible
-    if (threadIdx.x == 0) LRX_TRACE(1);
 
     if (warp == kProducerWarp) {
         // ===== TMA producer
@@ -298,17 +291,14 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                     mbar_wait(a_full, (uint32_t)(u / n_tiles) & 1u);
                     tc_fence_after();
                 }
-                if (u < 8) LRX_TRACE(16 + u * 4 + 0);
                 mbar_wait(&t_empty[buf], (use & 1u) ^ 1u);    // epilogue has drained this accumulator
                 tc_fence_after();
-                if (u < 8) LRX_TRACE(16 + u * 4 + 1);
                 const uint32_t tacc = tmem_base + buf * BN;
                 for (int kb = 0; kb < num_k_blocks; ++kb, ++it) {
                     const int s = (int)(it % kStages);
                     const uint32_t ph = (it / kStages) & 1u;
                     mbar_wait(&full[s], ph);
                     tc_fence_after();
-                    if (u < 8 && kb == 0) LRX_TRACE(16 + u * 4 + 2);
                     const uint32_t a_addr = smem_u32(sA + (ARES ? kb : s) * kABytes);
                     const uint32_t b_addr = smem_u32(sB + s * Cfg::kBBytes);
 #pragma unroll
@@ -326,7 +316,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                     else umma_commit(&empty[s]);              // smem slot free when the MMAs retire
                 }
                 umma_commit(&t_full[buf]);                    // accumulator complete
-                if (u < 8) LRX_TRACE(16 + u * 4 + 3);
                 if (ARES && (u % n_tiles) == n_tiles - 1) umma_commit(a_empty);   // A tile may be replaced
             }
         }
@@ -370,10 +359,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
             const uint32_t use = (uint32_t)(u / kAcc);
             const int n0 = n_blk * BN;
             const float* bias = s_bias + n0;
-            if (threadIdx.x == 0 && u < 8) LRX_TRACE(64 + u * 4 + 0);
             mbar_wait(&t_full[buf], use & 1u);
             tc_fence_after();
-            if (threadIdx.x == 0 && u < 8) LRX_TRACE(64 + u * 4 + 1);
             const int row = quarter * 32 + lane;
             const int64_t grow = (int64_t)m_blk * kBM + row;
             const bool ok = grow < ep.M;
@@ -528,7 +515,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
             }
             tc_fence_before();
             __syncwarp();
-            if (threadIdx.x == 0 && u < 8) LRX_TRACE(64 + u * 4 + 2);
             if (lane == 0) mbar_arrive(&t_empty[buf]);        // accumulator may be overwritten
         }
         stage_acquire(lane);                                  // shared memory outlives its last store
@@ -536,9 +522,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
     tc_fence_before();
     __syncthreads();
     if (!ep.pdl_early) pdl_trigger();          // this CTA's work is done
-    if (threadIdx.x == 0) LRX_TRACE(2);
     if (CS > 1) cluster_sync_all();            // nobody leaves while a peer may still multicast to it
-    if (threadIdx.x == 0) LRX_TRACE(3);
     if (warp == kMmaWarp) {
         tc_fence_after();
         tmem_dealloc(tmem_base, Cfg::kTmemCols);
@@ -648,7 +632,7 @@ GemmPlan gemm_plan(int num_sms, int M, int N, int K, int epi) {
     p.ares = (K == kAResKB * kBK) && (big || N / p.bn == 1);
     // clusters need every CTA of a cluster to walk the same n sequence: A-resident (n inner loop),
     // or a single n-block
-    p.cs = (big && (p.ares || N / p.bn == 1)) ? LRX_GEMM_CLUSTER : 1;
+    p.cs = (big && (p.ares || N / p.bn == 1)) ? kGemmCluster : 1;
     return p;
 }
 
@@ -658,8 +642,8 @@ static cudaError_t launch_one(lrx_handle* h, const CUtensorMap& ta, const CUtens
                               int N, int K, const GemmEpi& ep) {
     const GemmPlan p = gemm_plan(h->num_sms, M, N, K, EPI);
     if (p.cs > 1) {
-        if (p.ares) return launch_cfg<BN, EPI, true, LRX_GEMM_CLUSTER>(h, ta, tb, tout, tres, M, N, K, ep);
-        return launch_cfg<BN, EPI, false, LRX_GEMM_CLUSTER>(h, ta, tb, tout, tres, M, N, K, ep);
+        if (p.ares) return launch_cfg<BN, EPI, true, kGemmCluster>(h, ta, tb, tout, tres, M, N, K, ep);
+        return launch_cfg<BN, EPI, false, kGemmCluster>(h, ta, tb, tout, tres, M, N, K, ep);
     }
     if (p.ares) return launch_cfg<BN, EPI, true, 1>(h, ta, tb, tout, tres, M, N, K, ep);
     return launch_cfg<BN, EPI, false, 1>(h, ta, tb, tout, tres, M, N, K, ep);
@@ -685,7 +669,6 @@ cudaError_t launch_tc_gemm(lrx_handle* h, const CUtensorMap& ta, const CUtensorM
     GemmEpi ep;
     ep.bias = bias; ep.residual = nullptr; ep.gamma = gamma; ep.beta = beta;
     ep.out = out; ep.ld_out = ld_out; ep.ld_res = 0; ep.M = M; ep.eps = eps;
-    ep.trace = (long long*)h->debug_trace;
     const int bn = gemm_plan(h->num_sms, M, N, K, epi).bn;
     cudaError_t e = cudaErrorInvalidValue;
 #define LRX_GEMM_CASE(BN_, EPI_) \

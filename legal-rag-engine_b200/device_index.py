@@ -3,7 +3,6 @@
 from __future__ import annotations
 
 import ctypes as C
-import os
 from typing import Optional, Sequence
 
 import numpy as np
@@ -73,18 +72,16 @@ class DeviceIndex:
         self._ck(self.lib.lrx_set_stream(self.h, C.c_void_p(s)))
 
     # ------------------------------------------------------------- residency
-    def set_corpus(self, x: torch.Tensor, id_base: int = 0, prefilter: Optional[bool] = None):
-        """Make the fp16 chunk matrix resident.  `prefilter` (default: on, LRX_DENSE_PREFILTER=0
-        turns it off): also build the int8 shadow K2a scans for up to 4 queries at a time
-        (388 B/row instead of 768; results unchanged, see include/lrx.h)."""
+    def set_corpus(self, x: torch.Tensor, id_base: int = 0, prefilter: bool = True):
+        """Make the fp16 chunk matrix resident.  `prefilter`: also build the int8 shadow K2a scans
+        for up to 4 queries at a time (388 B/row instead of 768; results unchanged, see
+        include/lrx.h)."""
         assert x.dtype == torch.float16 and x.is_cuda and x.is_contiguous()
         assert x.dim() == 2 and x.shape[1] == LRX_DIM
         self.x, self.n_local, self.id_base = x, int(x.shape[0]), int(id_base)
         self._xbuf = x                                      # the rows append_rows can fill: x is its prefix
         self._ck(self.lib.lrx_set_corpus(self.h, _ptr(x), self.n_local, self.id_base, LRX_DIM))
         self._q8 = None
-        if prefilter is None:
-            prefilter = os.environ.get("LRX_DENSE_PREFILTER", "1") not in ("0", "", "off")
         self._prefilter_on = False
         if prefilter and self.n_local > 0:
             self.build_prefilter()

@@ -104,18 +104,19 @@ def test_encoder_padding_is_inert(dev):
     assert _cos(a.astype(np.float64), b.astype(np.float64)).min() > 0.999999
 
 
-def test_small_batch_kernel_agrees_with_the_gemm_chain(dev, monkeypatch):
-    """The same query batch through the one-launch cluster kernel and (LRX_NO_SMALL_ENCODER) through
-    the tcgen05 GEMM chain: same embeddings to fp16 rounding noise; padding inert on the small path."""
+def test_small_batch_kernel_agrees_with_the_gemm_chain(dev):
+    """The same query batch through the one-launch cluster kernel and, padded to 80 tokens (S > 64),
+    through the tcgen05 GEMM chain: same embeddings to fp16 rounding noise; padding inert on the
+    small path."""
     from legal_rag_engine_b200 import synth
     from legal_rag_engine_b200.encoder import SentenceEncoder
     sd = synth.bert_state_dict(54, 0.05, ln_jitter=0.1)
     enc = SentenceEncoder(dev, state_dict=sd)
     ids, lens = synth.token_batch(4, 30, seed=9)
     small = enc.encode_ids(ids, lens)
-    monkeypatch.setenv("LRX_NO_SMALL_ENCODER", "1")
-    chain = enc.encode_ids(ids, lens)
-    monkeypatch.delenv("LRX_NO_SMALL_ENCODER")
+    wide80 = np.zeros((4, 80), dtype=np.int32)
+    wide80[:, :30] = ids
+    chain = enc.encode_ids(wide80, lens)
     assert _cos(small.astype(np.float64), chain.astype(np.float64)).min() > 0.99999
     ids2 = ids.copy()
     for i, n in enumerate(lens):
