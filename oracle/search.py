@@ -24,10 +24,13 @@ class OracleIndex:
         self.bm25 = bm25
 
     def search_vec(self, qh: np.ndarray, term_ids: Sequence[int], k: int = 5,
-                   hybrid_weight: float = 0.5, fusion_mode: str = "linear"):
+                   hybrid_weight: float = 0.5, fusion_mode: str = "linear", dense_scores=None):
         """One (already encoded) query.  qh: fp16 [384]; term_ids: BM25 term ids
-        (-1 = out of vocabulary).  Returns [(id, score, semantic, keyword)]."""
-        scores = flat_ip.exact_scores(self.Xh, qh[None, :])
+        (-1 = out of vocabulary).  ``dense_scores``: this query's row of
+        ``flat_ip.exact_scores`` when the caller has it already (large corpora).
+        Returns [(id, score, semantic, keyword)]."""
+        scores = (flat_ip.exact_scores(self.Xh, qh[None, :]) if dense_scores is None
+                  else np.asarray(dense_scores, dtype=np.float64).reshape(1, -1))
         E, D, I = flat_ip.topk_from_scores(scores, 2 * k)          # :64  index.search(q, k*2)
         bm = self.bm25.get_scores_ids(term_ids)                    # :68
         max_bm25 = obm25.max_or_one(bm)                            # :74
@@ -41,8 +44,10 @@ class OracleIndex:
         raise ValueError(fusion_mode)
 
     def search_batch_vec(self, Qh: np.ndarray, term_id_lists: List[Sequence[int]], k: int,
-                         hybrid_weights: Sequence[float], fusion_mode: str = "linear"):
-        return [self.search_vec(Qh[i], term_id_lists[i], k, hybrid_weights[i], fusion_mode)
+                         hybrid_weights: Sequence[float], fusion_mode: str = "linear", dense_scores=None):
+        """``dense_scores``: ``flat_ip.exact_scores(Xh, Qh)`` computed once for several calls."""
+        return [self.search_vec(Qh[i], term_id_lists[i], k, hybrid_weights[i], fusion_mode,
+                                None if dense_scores is None else dense_scores[i])
                 for i in range(len(term_id_lists))]
 
 

@@ -186,9 +186,10 @@ def test_bm25_token_capacity_is_never_exceeded_silently(dev):
 
 def test_bm25_division_matches_ddiv_rn(dev):
     """The scan's branch-free float64 division (csrc/bm25.cu okapi_div) gives the bits of the IEEE
-    division for every (tf, len) a posting can hold, at several average lengths."""
+    division for every (tf, len) a posting can hold, at several average lengths.  An average below 1
+    (a corpus of mostly empty chunks) puts the divisor tf + k1*(1 - b + b*len/avgdl) far above 2^17."""
     import ctypes as C
-    for avgdl in (104.35572519083969, 80.0, 1.0, 517.3, 3.0e4):
+    for avgdl in (104.35572519083969, 80.0, 1.0, 517.3, 3.0e4, 0.05, 0.3337):
         bad = C.c_uint64(123)
         dev._ck(dev.lib.lrx_debug_bm25_divcheck(dev.h, avgdl, 1.5, 0.75, 4096, 65536, C.byref(bad)))
         assert bad.value == 0, (avgdl, bad.value)
