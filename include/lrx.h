@@ -145,6 +145,32 @@ int lrx_bm25_remove_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const 
                              const uint64_t* dev_rem_ptr, const uint32_t* dev_rem_doc,
                              const int32_t* dev_term_map, const uint64_t* dev_term_ptr_out,
                              int64_t n_terms_out, void* dev_postings_out);
+/* Index replacement (the reference has none: it rebuilds the store).  The text of some documents
+ * changes; document ids do not.  Current index: dev_term_ptr [n_terms+1] + dev_postings (nnz 8-byte
+ * entries) over local documents [0, n_docs).  Replaced: dev_replaced_docs [n_replaced], strictly
+ * ascending; per old term t its postings of replaced documents dev_rem_doc[dev_rem_ptr[t] ..
+ * dev_rem_ptr[t+1]), ascending (dropped; nnz_rem = rem_ptr[n_terms]); dev_term_map [n_terms]: t's new
+ * id, -1 for a word left without postings; per new term u its inserted entries dev_ins_doc_tf
+ * {u32 doc, u32 tf}[dev_ins_ptr[u] .. dev_ins_ptr[u+1]), doc ascending, every doc a replaced one
+ * (nnz_ins = ins_ptr[n_terms_out]); dev_doc_len [n_docs]: the lengths after the edit;
+ * dev_term_ptr_out [n_terms_out+1]: the new CSR's pointers.  Writes dev_postings_out (nnz - nnz_rem +
+ * nnz_ins entries, rounded up to an even count, 16-byte aligned, pad zeroed): under each new id, the
+ * kept postings of its old term (copied verbatim) merged by document with its inserted entries --
+ * byte for byte what lrx_bm25_build_postings makes of the rebuilt CSR.  The outputs must not overlap
+ * the inputs.  The handle's index is not touched: pass the outputs to lrx_set_postings with the new
+ * idf / avgdl.  Synchronous.  LRX_E_ARG, with nothing else changed, when the CSR ends do not match the
+ * counts, a dropped list is not strictly ascending or holds a document that is not a replaced posting
+ * of its term, a posting of a replaced document is missing from its term's list, an inserted list is
+ * not strictly ascending or holds a document that is not replaced, a tf is outside [1, 65535] or a
+ * length over 65535, term_map is not injective into [0, n_terms_out), or a new id's range is not its
+ * kept plus inserted count (or is empty). */
+int lrx_bm25_replace_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const void* dev_postings,
+                              int64_t n_terms, int64_t nnz, int64_t n_docs,
+                              const uint32_t* dev_replaced_docs, int64_t n_replaced,
+                              const uint64_t* dev_rem_ptr, const uint32_t* dev_rem_doc,
+                              const int32_t* dev_term_map, const uint64_t* dev_ins_ptr,
+                              const uint32_t* dev_ins_doc_tf, int64_t nnz_ins, const uint32_t* dev_doc_len,
+                              const uint64_t* dev_term_ptr_out, int64_t n_terms_out, void* dev_postings_out);
 
 /* ---- K1: encoder (replaces SentenceTransformer("all-MiniLM-L6-v2").encode followed by
  *      faiss.normalize_L2; retrieval_engine.py:28,61-62, create_vector_store.py:33-34,45,51) --

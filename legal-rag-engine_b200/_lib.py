@@ -76,6 +76,8 @@ _SIGNATURES = {
                                            _i64, _vp, _vp]),
     "lrx_bm25_remove_postings": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _vp,
                                            _i64, _vp]),
+    "lrx_bm25_replace_postings": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp,
+                                            _i64, _vp, _vp, _i64, _vp]),
     "lrx_set_encoder_weights": (C.c_int, [_vp, C.POINTER(lrx_bert_weights)]),
     "lrx_encode": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _vp, _vp]),
     "lrx_encode_host": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _vp]),

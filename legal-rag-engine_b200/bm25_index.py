@@ -298,6 +298,216 @@ def remove_csr(term_ptr: np.ndarray, postings: np.ndarray, rem: BM25Remove):
 
 
 @dataclass
+class BM25Replace:
+    """Documents whose text is replaced in place (document ids unchanged): per old term its postings
+    of replaced documents (dropped), the terms in the order a rebuild numbers them, per new term its
+    inserted entries, and the statistics after the edit."""
+    replaced: np.ndarray         # int64 [m] replaced document ids, ascending
+    doc_len: np.ndarray          # uint32 [m] their new lengths
+    rem_ptr: np.ndarray          # int64 [V+1] per old term, its postings of replaced documents ...
+    rem_doc: np.ndarray          # uint32 [nnz_rem] ... ascending (dropped)
+    term_map: np.ndarray         # int32 [V] old term id -> new id, -1 = vanished
+    new_words: List[str]         # words the old index lacks, in first-appearance order over the new texts ...
+    new_map: np.ndarray          # int32 [len(new_words)] ... and their new ids
+    ins_ptr: np.ndarray          # int64 [V_out+1] per new term, its inserted entries ...
+    ins_postings: np.ndarray     # uint32 [nnz_ins, 2] = (doc, tf), doc ascending per term, every doc replaced
+    term_ptr: np.ndarray         # int64 [V_out+1] the new CSR's pointers
+    stats: BM25Stats             # after the edit, new term ids
+
+    @property
+    def n_terms(self) -> int:
+        return len(self.term_ptr) - 1
+
+    @property
+    def nnz(self) -> int:
+        return int(self.term_ptr[-1])
+
+    @property
+    def nnz_rem(self) -> int:
+        return int(self.rem_ptr[-1])
+
+    @property
+    def nnz_ins(self) -> int:
+        return int(self.ins_ptr[-1])
+
+    def commit_vocab(self):
+        """Renumber ``stats.vocab`` in place: the old words that remain and the new words, in new id order."""
+        words = list(self.stats.vocab) + list(self.new_words)
+        ext = np.concatenate([self.term_map, self.new_map]).astype(np.int64)
+        live = np.flatnonzero(ext >= 0)
+        order = live[np.argsort(ext[live])]
+        self.stats.vocab.clear()
+        self.stats.vocab.update(zip(map(words.__getitem__, order.tolist()), range(len(order))))
+
+
+def csr_replace(stats: BM25Stats, ids: Sequence[int], new_token_lists: Sequence[Sequence[str]],
+                doc_tokens: Callable[[int], Sequence[str]],
+                first_postings: Callable[[np.ndarray, np.ndarray], np.ndarray]) -> BM25Replace:
+    """The plan of replacing the text of documents ``ids`` by ``new_token_lists`` (document ids do not
+    change), equal to what a rebuild over the edited documents computes.  ``stats`` is read, not
+    changed; ``doc_tokens(d)`` tokenises the current text of document d; ``first_postings(terms,
+    counts)`` returns the documents of the first ``counts[i]`` postings of each ``terms[i]``.
+
+    A rebuild numbers terms by the key (first document, position of the term's first occurrence
+    among that document's distinct tokens).  A term in neither the old nor the new text of a replaced
+    document keeps its postings, first document and key.  So does a touched term whose first document
+    is unchanged and not replaced.  Every other term that survives is re-keyed: its new first document
+    is the smaller of its first posting outside the replaced set (among its first ``r_t + 1`` postings
+    when its old first document is replaced) and the first replaced document whose new text holds it;
+    the position comes from tokenising that document (its new text if it is replaced).  New words are
+    keyed the same way; words left without postings vanish.  The re-keyed terms, sorted by key, are
+    merged into the kept ones, and okapi_idf in that order gives every idf bit of the rebuild.  Work:
+    O(old and new tokens of the replaced documents + tokens of the new first documents + V)."""
+    vocab, n_docs = stats.vocab, int(stats.n_docs)
+    V = len(vocab)
+    ids = np.asarray(ids, dtype=np.int64).reshape(-1)
+    if len(new_token_lists) != len(ids):
+        raise ValueError(f"{len(ids)} ids but {len(new_token_lists)} new documents")
+    order = np.argsort(ids, kind="stable")
+    replaced = ids[order]
+    if len(replaced) and (np.diff(replaced) == 0).any():
+        raise ValueError("duplicate ids")
+    if len(replaced) and (replaced[0] < 0 or replaced[-1] >= n_docs):
+        raise ValueError(f"ids must lie in [0, {n_docs})")
+    new_lists = [new_token_lists[i] for i in order.tolist()]
+    # the dropped entries: every (term, replaced document) of the old texts
+    t_l, d_l = [], []
+    len_old = 0
+    for d in replaced.tolist():
+        tokens = doc_tokens(d)
+        len_old += len(tokens)
+        for word in dict.fromkeys(tokens):
+            t = vocab.get(word)
+            if t is None:
+                raise ValueError(f"document {d}: token {word!r} is not in the index's vocabulary")
+            t_l.append(t); d_l.append(d)
+    t = np.asarray(t_l, dtype=np.int64)
+    d = np.asarray(d_l, dtype=np.int64)
+    o = np.lexsort((d, t))
+    t, d = t[o], d[o]
+    r = np.bincount(t, minlength=V).astype(np.int64)
+    rem_ptr = np.zeros(V + 1, dtype=np.int64)
+    np.cumsum(r, out=rem_ptr[1:])
+    df_kept = stats.df - r
+    if (df_kept < 0).any():
+        raise ValueError("the replaced documents' tokens do not match the index's postings")
+    # the inserted entries: every (term, replaced document, tf) of the new texts; new words get ids
+    # V, V + 1, ... in first-appearance order
+    new: Dict[str, int] = {}
+    it_l, id_l, if_l, lens = [], [], [], []
+    for dd, document in zip(replaced.tolist(), new_lists):
+        lens.append(len(document))
+        freqs: Dict[str, int] = {}
+        for word in document:
+            freqs[word] = freqs.get(word, 0) + 1
+        for word, f in freqs.items():
+            tt = vocab.get(word)
+            if tt is None:
+                tt = new.get(word)
+                if tt is None:
+                    tt = new[word] = V + len(new)
+            it_l.append(tt); id_l.append(dd); if_l.append(f)
+    W = V + len(new)
+    it = np.asarray(it_l, dtype=np.int64)
+    idd = np.asarray(id_l, dtype=np.int64)
+    iff = np.asarray(if_l, dtype=np.int64)
+    total = int(stats.total_len) - len_old + sum(lens)
+    if total <= 0:
+        raise ValueError("the edit leaves the corpus without BM25 tokens: avgdl would be 0")
+    ins_cnt = np.bincount(it, minlength=W).astype(np.int64)
+    df_ext = np.concatenate([df_kept, np.zeros(len(new), dtype=np.int64)]) + ins_cnt
+    alive = df_ext > 0
+    none = n_docs                                        # "no such document": larger than every id
+    is_rep = lambda a: replaced[np.minimum(np.searchsorted(replaced, a), len(replaced) - 1)] == a
+    # first replaced document whose new text holds each term (entries are in document order)
+    first_ins = np.full(W, none, dtype=np.int64)
+    np.minimum.at(first_ins, it, idd)
+    # first posting outside the replaced set
+    first_old = np.concatenate([stats.first_doc, np.full(len(new), none, dtype=np.int64)])
+    first_out = np.where(np.concatenate([df_kept, np.zeros(len(new), dtype=np.int64)]) > 0, first_old, none)
+    cand = np.nonzero(r)[0]
+    aff = cand[(df_kept[cand] > 0) & is_rep(stats.first_doc[cand])] if len(replaced) else cand[:0]
+    if len(aff):
+        counts = r[aff] + 1
+        docs = np.asarray(first_postings(aff, counts), dtype=np.int64)
+        idx = np.where(is_rep(docs), len(docs), np.arange(len(docs)))
+        pick = np.minimum.reduceat(idx, np.cumsum(counts) - counts)
+        if (pick >= len(docs)).any():
+            raise ValueError("the replaced documents' tokens do not match the index's postings")
+        first_out[aff] = docs[pick]
+    first_after = np.minimum(first_out, first_ins)
+    rekey = alive & ((first_after != first_old) | (is_rep(first_after) if len(replaced) else False))
+    rk = np.nonzero(rekey)[0]
+    # within-document positions of every term whose first document is one of the re-keyed terms'
+    pos = np.zeros(W, dtype=np.int64)
+    slot = {dd: i for i, dd in enumerate(replaced.tolist())}
+    for f in np.unique(first_after[rk]).tolist():
+        tokens = new_lists[slot[f]] if f in slot else doc_tokens(f)
+        for p, word in enumerate(dict.fromkeys(tokens)):
+            tt = vocab.get(word)
+            if tt is None:
+                tt = new.get(word)
+                if tt is None:
+                    raise ValueError(f"document {f}: token {word!r} is not in the index's vocabulary")
+            if first_after[tt] == f:
+                pos[tt] = p
+    key = (first_after << 17) + pos                      # a document has < 2^16 distinct tokens
+    keep = np.nonzero(alive & ~rekey)[0]                 # old terms with their old keys: in key order
+    a_sorted = rk[np.argsort(key[rk], kind="stable")]
+    new_order = np.insert(keep, np.searchsorted(key[keep], key[a_sorted]), a_sorted)
+    ext_map = np.full(W, -1, dtype=np.int32)
+    ext_map[new_order] = np.arange(len(new_order), dtype=np.int32)
+    df_out = df_ext[new_order]
+    term_ptr = np.zeros(len(new_order) + 1, dtype=np.int64)
+    np.cumsum(df_out, out=term_ptr[1:])
+    nt = ext_map[it].astype(np.int64)
+    o = np.lexsort((idd, nt))
+    ins_postings = np.empty((len(o), 2), dtype=np.uint32)
+    ins_postings[:, 0] = idd[o]
+    ins_postings[:, 1] = iff[o]
+    ins_ptr = np.zeros(len(new_order) + 1, dtype=np.int64)
+    np.cumsum(np.bincount(nt, minlength=len(new_order)), out=ins_ptr[1:])
+    idf, _ = okapi_idf(df_out, n_docs, stats.epsilon)
+    return BM25Replace(replaced, np.asarray(lens, dtype=np.uint32), rem_ptr, d.astype(np.uint32), ext_map[:V],
+                       list(new), ext_map[V:], ins_ptr, ins_postings, term_ptr,
+                       BM25Stats(vocab, df_out, first_after[new_order], n_docs, total, idf, total / n_docs,
+                                 stats.k1, stats.b, stats.epsilon))
+
+
+def replace_csr(term_ptr: np.ndarray, postings: np.ndarray, rep: BM25Replace):
+    """Host compaction (the device does the same in lrx_bm25_replace_postings), linear in the postings
+    but for one binary search per kept posting into the inserted entries: the postings of the replaced
+    documents dropped, the others moved verbatim to their term's new id, each new list merged by
+    document with its inserted entries.  Returns (term_ptr uint64 [V_out+1], postings uint32 [nnz_out, 2])."""
+    old_ptr = np.asarray(term_ptr, dtype=np.int64)
+    out_ptr = np.asarray(rep.term_ptr, dtype=np.int64)
+    V, V_out = len(old_ptr) - 1, rep.n_terms
+    mark = np.zeros(rep.stats.n_docs, dtype=bool)
+    mark[rep.replaced] = True
+    term_of = np.repeat(np.arange(V, dtype=np.int64), np.diff(old_ptr))
+    keep = ~mark[postings[:, 0]]
+    kt = term_of[keep]
+    m = rep.term_map[kt].astype(np.int64)
+    assert (m >= 0).all(), "the replacement plan does not describe these postings"
+    kcount = np.bincount(kt, minlength=V)
+    rank = np.arange(len(kt), dtype=np.int64) - np.repeat(np.cumsum(kcount) - kcount, kcount)
+    kept = postings[keep]
+    ins_ptr = np.asarray(rep.ins_ptr, dtype=np.int64)
+    ins_term = np.repeat(np.arange(V_out, dtype=np.int64), np.diff(ins_ptr))
+    key_i = (ins_term << 32) | rep.ins_postings[:, 0].astype(np.int64)
+    c = np.searchsorted(key_i, (m << 32) | kept[:, 0].astype(np.int64)) - ins_ptr[m]
+    dst = out_ptr[m] + rank + c
+    out = np.empty((int(out_ptr[-1]), 2), dtype=np.uint32)
+    assert len(kept) + rep.nnz_ins == len(out), "the replacement plan does not describe these postings"
+    taken = np.zeros(len(out), dtype=bool)
+    taken[dst] = True
+    assert int(taken.sum()) == len(kept), "the replacement plan does not describe these postings"
+    out[dst] = kept
+    out[~taken] = rep.ins_postings                       # free slots ascend with (new term, doc)
+    return out_ptr.astype(np.uint64), out
+
+
+@dataclass
 class BM25Index:
     n_docs: int
     doc_len: np.ndarray          # uint32 [n_docs]
@@ -417,6 +627,22 @@ class BM25Index:
         rem.commit_vocab()
         term_ptr, postings = remove_csr(self.term_ptr, self.postings, rem)
         return BM25Index.from_stats(rem.stats, term_ptr, postings, np.delete(self.doc_len, rem.removed))
+
+    # ------------------------------------------------------------------ replace
+    def replace(self, ids: Sequence[int], new_token_lists: Sequence[Sequence[str]],
+                doc_tokens: Callable[[int], Sequence[str]]) -> "BM25Index":
+        """This index with the text of documents ``ids`` replaced by ``new_token_lists`` (ids unchanged):
+        equal, field by field and bit for bit, to ``from_token_lists(edited documents)``, vocabulary
+        order included.  ``doc_tokens(d)`` tokenises the current document d; only the replaced
+        documents and the new first documents of re-keyed terms are read (``csr_replace``)."""
+        tp = self.term_ptr.astype(np.int64)
+        gather = lambda terms, counts: self.postings[_ranges(tp[terms], counts), 0]
+        rep = csr_replace(self.stats(), ids, new_token_lists, doc_tokens, gather)
+        rep.commit_vocab()
+        term_ptr, postings = replace_csr(self.term_ptr, self.postings, rep)
+        doc_len = self.doc_len.copy()
+        doc_len[rep.replaced] = rep.doc_len
+        return BM25Index.from_stats(rep.stats, term_ptr, postings, doc_len)
 
     # ------------------------------------------------------------------ query
     def term_ids(self, tokens: Sequence[str]) -> List[int]:

@@ -427,6 +427,48 @@ int lrx_bm25_remove_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const 
     return LRX_OK;
 }
 
+int lrx_bm25_replace_postings(lrx_handle* h, const uint64_t* dev_term_ptr, const void* dev_postings,
+                              int64_t n_terms, int64_t nnz, int64_t n_docs,
+                              const uint32_t* dev_replaced_docs, int64_t n_replaced,
+                              const uint64_t* dev_rem_ptr, const uint32_t* dev_rem_doc,
+                              const int32_t* dev_term_map, const uint64_t* dev_ins_ptr,
+                              const uint32_t* dev_ins_doc_tf, int64_t nnz_ins, const uint32_t* dev_doc_len,
+                              const uint64_t* dev_term_ptr_out, int64_t n_terms_out, void* dev_postings_out) {
+    if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_bm25_replace_postings: null handle");
+    std::lock_guard<std::mutex> g(h->mu);
+    if (n_terms < 0 || nnz < 0 || n_docs < 0 || n_docs >= (1ll << 32) || n_replaced < 0 || n_replaced > n_docs ||
+        nnz_ins < 0 || n_terms_out < 0 || n_terms_out > INT32_MAX)
+        return fail(h, LRX_E_ARG, "lrx_bm25_replace_postings: bad size");
+    if (dev_term_ptr == nullptr || dev_rem_ptr == nullptr || dev_ins_ptr == nullptr || dev_term_ptr_out == nullptr ||
+        (n_terms > 0 && dev_term_map == nullptr) || (n_replaced > 0 && dev_replaced_docs == nullptr) ||
+        (nnz_ins > 0 && (dev_ins_doc_tf == nullptr || dev_doc_len == nullptr)) ||
+        (nnz > 0 && dev_postings == nullptr) || (nnz + nnz_ins > 0 && dev_postings_out == nullptr))
+        return fail(h, LRX_E_ARG, "lrx_bm25_replace_postings: null pointer");
+    if ((((uintptr_t)dev_postings | (uintptr_t)dev_postings_out) & 15) != 0 ||
+        (((uintptr_t)dev_term_ptr | (uintptr_t)dev_rem_ptr | (uintptr_t)dev_ins_ptr | (uintptr_t)dev_ins_doc_tf |
+          (uintptr_t)dev_term_ptr_out) & 7) != 0 ||
+        (((uintptr_t)dev_replaced_docs | (uintptr_t)dev_rem_doc | (uintptr_t)dev_term_map |
+          (uintptr_t)dev_doc_len) & 3) != 0)
+        return fail(h, LRX_E_ARG, "lrx_bm25_replace_postings: postings must be 16-byte aligned, pointer "
+                                  "tables and (doc, tf) pairs 8-byte aligned, id arrays 4-byte aligned");
+    LRX_CUDA(h, cudaSetDevice(h->device));
+    int bad = 0;
+    LRX_CUDA(h, launch_bm25_replace(h, dev_term_ptr, dev_postings, n_terms, nnz, n_docs, dev_replaced_docs,
+                                    n_replaced, dev_rem_ptr, dev_rem_doc, dev_term_map, dev_ins_ptr, dev_ins_doc_tf,
+                                    nnz_ins, dev_doc_len, dev_term_ptr_out, n_terms_out, dev_postings_out, &bad));
+    if (bad == 2)
+        return fail(h, LRX_E_ARG, "lrx_bm25_replace_postings: term_ptr[n_terms] != nnz, ins_ptr[0] != 0, "
+                                  "ins_ptr[n_terms_out] != nnz_ins, term_ptr_out[0] != 0 or term_ptr_out[n_terms_out] "
+                                  "!= nnz - rem_ptr[n_terms] + nnz_ins");
+    if (bad)
+        return fail(h, LRX_E_ARG, "lrx_bm25_replace_postings: the replacement does not describe the index "
+                                  "(replaced ids unsorted or out of range, a dropped list unsorted or not the "
+                                  "term's postings of replaced documents, an inserted list unsorted or holding a "
+                                  "document that is not replaced, a tf or length over 65535, term_map not "
+                                  "injective, or an output range of the wrong length)");
+    return LRX_OK;
+}
+
 int lrx_set_encoder_weights(lrx_handle* h, const lrx_bert_weights* w) {
     if (h == nullptr) return fail(nullptr, LRX_E_ARG, "lrx_set_encoder_weights: null handle");
     std::lock_guard<std::mutex> g(h->mu);

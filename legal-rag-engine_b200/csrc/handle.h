@@ -85,7 +85,7 @@ struct lrx_handle {
     void* ws_misc = nullptr;         size_t ws_misc_bytes = 0;          // search chain scratch
     void* ws_host = nullptr;         size_t ws_host_bytes = 0;          // pinned staging
     void* ws_io = nullptr;           size_t ws_io_bytes = 0;            // device staging
-    void* ws_rm = nullptr;           size_t ws_rm_bytes = 0;            // index removal: doc map, tile table
+    void* ws_rm = nullptr;           size_t ws_rm_bytes = 0;            // index removal / replacement: doc map or bits, tile table
 
     // peer exchange (lrx_exchange_*): this rank's region, the peers' (IPC-mapped), a device copy of
     // the pointer table, the per-call sequence number
@@ -165,6 +165,14 @@ cudaError_t launch_bm25_remove(lrx_handle* h, const uint64_t* term_ptr, const vo
                                int64_t nnz, int64_t n_docs_old, const uint32_t* removed, int64_t n_removed,
                                const uint64_t* rem_ptr, const uint32_t* rem_doc, const int32_t* term_map,
                                const uint64_t* ptr_out, int64_t n_terms_out, void* post_out, int* host_bad);
+// host_bad: 1 = the replacement plan does not describe the postings (see lrx_bm25_replace_postings),
+// 2 = a CSR end does not match the counts (nothing launched)
+cudaError_t launch_bm25_replace(lrx_handle* h, const uint64_t* term_ptr, const void* post, int64_t n_terms,
+                                int64_t nnz, int64_t n_docs, const uint32_t* replaced, int64_t n_rep,
+                                const uint64_t* rem_ptr, const uint32_t* rem_doc, const int32_t* term_map,
+                                const uint64_t* ins_ptr, const uint32_t* ins_doc_tf, int64_t nnz_ins,
+                                const uint32_t* doc_len, const uint64_t* ptr_out, int64_t n_terms_out,
+                                void* post_out, int* host_bad);
 cudaError_t launch_bm25_lut(lrx_handle* h, double avgdl, double k1, double b, int max_len);
 cudaError_t launch_bm25_divcheck(lrx_handle* h, double avgdl, double k1, double b, int n_tf, int n_len,
                                  unsigned long long* host_mismatches);

@@ -245,8 +245,50 @@ class DeviceIndex:
         idf_t = _to(rem.stats.idf, torch.float64, self.device)
         return tp_out, p8_out, idf_t, dl, float(rem.stats.avgdl), int(dl.max().item())
 
+    def stage_replace(self, rep, doc_len_new):
+        """The resident postings with the text of a replacement plan's documents (bm25_index.BM25Replace)
+        replaced, merged on the device into new buffers (lrx_bm25_replace_postings): a staged index for
+        `commit_postings`.  `doc_len_new` [n_docs]: every document's length after the edit (torch or
+        numpy).  The handle is not changed; a plan that does not describe the postings raises LrxError
+        (LRX_E_ARG)."""
+        tp, p8, _ = self._post
+        nnz = self._post_args[0]
+        replaced = _to(np.asarray(rep.replaced).astype(np.uint32), torch.int32, self.device)
+        rem_ptr = _to(np.asarray(rep.rem_ptr, dtype=np.int64), torch.int64, self.device)
+        rem_doc = _to(np.asarray(rep.rem_doc, dtype=np.uint32), torch.int32, self.device)
+        term_map = _to(np.asarray(rep.term_map, dtype=np.int32), torch.int32, self.device)
+        ins_ptr = _to(np.asarray(rep.ins_ptr, dtype=np.int64), torch.int64, self.device)
+        ins = _to(np.asarray(rep.ins_postings, dtype=np.uint32).reshape(-1, 2), torch.int32, self.device)
+        dl = _to(np.asarray(doc_len_new, dtype=np.uint32) if not isinstance(doc_len_new, torch.Tensor)
+                 else doc_len_new, torch.int32, self.device)
+        assert dl.numel() == self.n_docs, (dl.numel(), self.n_docs)
+        tp_out = _to(np.asarray(rep.term_ptr, dtype=np.int64), torch.int64, self.device)
+        p8_out = torch.empty((rep.nnz + 2, 2), dtype=torch.int32, device=self.device)
+        self._ck(self.lib.lrx_bm25_replace_postings(
+            self.h, _ptr(tp), _ptr(p8), self.n_terms, nnz, self.n_docs, _ptr(replaced), len(rep.replaced),
+            _ptr(rem_ptr), _ptr(rem_doc), _ptr(term_map), _ptr(ins_ptr), _ptr(ins), rep.nnz_ins, _ptr(dl),
+            _ptr(tp_out), rep.n_terms, _ptr(p8_out)))
+        idf_t = _to(rep.stats.idf, torch.float64, self.device)
+        return tp_out, p8_out, idf_t, dl, float(rep.stats.avgdl), int(dl.max().item())
+
+    def replace_rows(self, ids, x_new: torch.Tensor, prefilter: Optional[bool] = None):
+        """Overwrite the fp16 rows `ids` (local ids, a sequence or a tensor) in place with `x_new`.  The int8 shadow of the old
+        rows is dropped from the handle first; `prefilter` (default: as before) rebuilds it."""
+        assert x_new.dtype == torch.float16 and x_new.is_cuda and x_new.dim() == 2
+        idx = (ids.to(self.device, torch.int64) if isinstance(ids, torch.Tensor)
+               else torch.as_tensor(np.asarray(ids, dtype=np.int64), device=self.device))
+        assert x_new.shape == (idx.numel(), LRX_DIM)
+        if prefilter is None:
+            prefilter = self._prefilter_on
+        if self._prefilter_on:
+            self.set_prefilter(False)
+        self._q8 = None                                     # the shadow of the old rows
+        self.x.index_copy_(0, idx, x_new)
+        if prefilter:
+            self.build_prefilter()
+
     def commit_postings(self, staged):
-        """Make a staged index of `stage_append` or `compact_postings` resident."""
+        """Make a staged index of `stage_append`, `compact_postings` or `stage_replace` resident."""
         tp_out, p8_out, idf_t, dl, avgdl, max_len = staged
         _, _, k1, b, _ = self._post_args
         self._install(tp_out, p8_out, idf_t, dl, avgdl, k1, b, max_len)

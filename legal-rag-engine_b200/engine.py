@@ -7,7 +7,8 @@ store directory; everything numeric runs in the CUDA library behind include/lrx.
 Additive surface only: ``search_batch`` (the orchestrator's concept-expansion fan-out in one
 launch chain, orchestrator.py:38-62), ``fusion="linear"|"rrf"`` (default "linear" = the
 reference's behaviour, retrieval_engine.py:71-96), ``encode``, ``add_chunks`` / ``remove_chunks`` /
-``save`` (grow or shrink a loaded index without a rebuild; results stay bit-identical to a rebuild).
+``replace_chunks`` / ``save`` (grow, shrink or edit a loaded index without a rebuild; results stay
+bit-identical to a rebuild).
 
 There is no CPU fallback: without a CUDA device or the built library the constructor raises.
 """
@@ -28,7 +29,7 @@ import torch
 
 from . import store as _store
 from ._lib import LRX_MAX_BATCH, LRX_MAX_DEPTH
-from .bm25_index import BM25Index, csr_append, csr_remove, tokenize
+from .bm25_index import BM25Index, csr_append, csr_remove, csr_replace, tokenize
 from .device_index import FUSION, DeviceIndex
 from .encoder import SentenceEncoder
 from .sharding import shard_range
@@ -50,6 +51,35 @@ def _resolve_model_dir(model_dir: Optional[str]) -> Optional[str]:
                 if "MiniLM-L6" in str(p):
                     return str(p.parent)
     return None
+
+
+def _chunk_tokens(chunks: Sequence[dict]) -> List[List[str]]:
+    """The BM25 tokens of each chunk, after checking it is a dict with a str ``"text"`` of at most
+    65 535 tokens (the 8-byte posting stores the document length in 16 bits)."""
+    tokens = []
+    for i, c in enumerate(chunks):
+        if not isinstance(c, dict) or not isinstance(c.get("text"), str):
+            raise ValueError(f"chunk {i}: expected a dict with a str 'text'")
+        tokens.append(tokenize(c["text"]))
+        if len(tokens[-1]) > 65535:
+            raise ValueError(f"chunk {i}: {len(tokens[-1])} tokens; a BM25 document holds at most 65535")
+    return tokens
+
+
+def _check_id_types(ids: Sequence) -> None:
+    for i in ids:
+        if isinstance(i, (bool, np.bool_)) or not isinstance(i, (int, np.integer)):
+            raise TypeError(f"chunk ids must be ints, got {i!r}")
+
+
+def _id_array(ids: Sequence[int], n: int) -> np.ndarray:
+    """Chunk ids as int64, after checking they lie in [0, n) and are unique."""
+    ids_arr = np.asarray(ids, dtype=np.int64).reshape(-1)
+    if len(ids_arr) and (ids_arr.min() < 0 or ids_arr.max() >= n):
+        raise ValueError(f"chunk ids must lie in [0, {n})")
+    if len(np.unique(ids_arr)) != len(ids_arr):
+        raise ValueError("duplicate chunk ids")
+    return ids_arr
 
 
 def _dist_state(group=None):
@@ -226,13 +256,7 @@ class RetrievalEngine:
         if self.world > 1:
             raise NotImplementedError("add_chunks on a sharded engine: rebuild the store instead")
         chunks = list(chunks)
-        tokens = []
-        for i, c in enumerate(chunks):
-            if not isinstance(c, dict) or not isinstance(c.get("text"), str):
-                raise ValueError(f"chunk {i}: expected a dict with a str 'text'")
-            tokens.append(tokenize(c["text"]))
-            if len(tokens[-1]) > 65535:
-                raise ValueError(f"chunk {i}: {len(tokens[-1])} tokens; a BM25 document holds at most 65535")
+        tokens = _chunk_tokens(chunks)
         with self._lock:
             n = self.n_total
             if n + len(chunks) >= 1 << 32:
@@ -261,21 +285,15 @@ class RetrievalEngine:
         numbered by rank.  Searches afterwards return exactly what an engine over a store rebuilt
         from the remaining chunks (with their current rows) returns.  Ids must be ints, in range and
         unique, and at least one chunk must remain; a rejected call raises and leaves the engine as
-        it was.  To replace a chunk, remove it and add the new version.  Not supported on a sharded
-        engine (world > 1)."""
+        it was.  To replace a chunk and keep its position, use ``replace_chunks``.  Not supported on a
+        sharded engine (world > 1)."""
         if self.world > 1:
             raise NotImplementedError("remove_chunks on a sharded engine: rebuild the store instead")
         ids = list(ids)
-        for i in ids:
-            if isinstance(i, (bool, np.bool_)) or not isinstance(i, (int, np.integer)):
-                raise TypeError(f"chunk ids must be ints, got {i!r}")
+        _check_id_types(ids)
         with self._lock:
             n = self.n_total
-            ids_arr = np.asarray(ids, dtype=np.int64).reshape(-1)
-            if len(ids_arr) and (ids_arr.min() < 0 or ids_arr.max() >= n):
-                raise ValueError(f"chunk ids must lie in [0, {n})")
-            if len(np.unique(ids_arr)) != len(ids_arr):
-                raise ValueError("duplicate chunk ids")
+            ids_arr = _id_array(ids, n)
             if len(ids_arr) >= n:
                 raise ValueError("removing every chunk: the BM25 statistics of an empty corpus are undefined")
             ids_map = np.arange(n, dtype=np.int64)
@@ -301,6 +319,45 @@ class RetrievalEngine:
             if prefilter:
                 self.dev.build_prefilter()
             return ids_map
+
+    def replace_chunks(self, ids: Sequence[int], chunks: Sequence[dict]) -> None:
+        """Replace chunks in place: chunk ``ids[i]`` (its position in ``self.chunks``) becomes
+        ``chunks[i]``, and every chunk keeps its position.  Searches afterwards return exactly what an
+        engine over a store rebuilt from the edited chunk list (with these rows) returns, BM25
+        vocabulary order and idf bits included.  Each new chunk is a dict with a str ``"text"``,
+        embedded and stored as ``add_chunks`` does.  Ids must be ints, in range and unique, one per
+        chunk, and the edit must leave the corpus some BM25 token; a rejected call raises and leaves
+        the engine as it was.  Not supported on a sharded engine (world > 1)."""
+        if self.world > 1:
+            raise NotImplementedError("replace_chunks on a sharded engine: rebuild the store instead")
+        ids, chunks = list(ids), list(chunks)
+        _check_id_types(ids)
+        if len(ids) != len(chunks):
+            raise ValueError(f"{len(ids)} ids but {len(chunks)} chunks")
+        tokens = _chunk_tokens(chunks)
+        with self._lock:
+            ids_arr = _id_array(ids, self.n_total)
+            if not len(ids_arr):
+                return
+            x16 = self.model.encode([c["text"] for c in chunks]).astype(np.float16)
+            rep = csr_replace(self._stats, ids_arr, tokens, lambda d: tokenize(self.chunks[d]["text"]),
+                              self.dev.posting_docs)
+            # the steps in the order remove_chunks gives them, for the same reason: the postings are
+            # staged into new buffers (the kernel validates the plan), the rows overwritten in place,
+            # then the handle takes the new postings; the int8 shadow is rebuilt last
+            doc_len = self.dev.doc_len[:self.n_total].clone()
+            doc_len[torch.from_numpy(rep.replaced).to(doc_len.device)] = torch.from_numpy(
+                rep.doc_len.astype(np.int32)).to(doc_len.device)
+            staged = self.dev.stage_replace(rep, doc_len)
+            prefilter = self.dev._prefilter_on
+            self.dev.replace_rows(ids_arr, torch.from_numpy(x16).to(self.dev.device), prefilter=False)
+            self.dev.commit_postings(staged)
+            rep.commit_vocab()
+            self._stats = rep.stats
+            for i, c in zip(ids_arr.tolist(), chunks):
+                self.chunks[i] = c
+            if prefilter:
+                self.dev.build_prefilter()
 
     def save(self, store_dir: Optional[str] = None) -> Path:
         """Write the current index (added chunks included) as a store that ``RetrievalEngine`` and
